@@ -1,6 +1,6 @@
 """bench.py -- steric grid-points/s on the OM4p25-shaped workload (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch: what ``momlevel.steric(dset)`` computes
@@ -43,10 +43,17 @@ WORKLOADS = {
 }
 
 
+def _positive(text):
+    n = int(text)
+    if n < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return n
+
+
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=_positive, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=os.environ.get("ML_BENCH_WORKLOAD", "om4p25"), choices=sorted(WORKLOADS))
@@ -58,7 +65,43 @@ def parse_args():
                     help="BASELINE configs timed beside the headline (extras.configs); '' or --no-configs for none")
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--no-selfcheck", action="store_true", help="skip the 200-step self-check (for ncu launch lists)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+DUMP_BYTES = 48 << 20  # the dumped sample stays well under 64 MB for every workload
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out_dir, eta, rho_ref, sums, v_ref):
+    """Write the arrays one timed step returned, so that two builds can be compared output for output.
+
+    ``sums.npy`` is {volo, masso}.  ``eta.npy`` ([nt][n]) holds ``n`` columns drawn with a fixed seed from those with
+    a surface reference volume (elsewhere eta is NaN by definition) and sorted, so the sample depends only on the
+    inputs.  When the call stored it, ``rho_ref.npy`` holds the reference density of the cells of these columns
+    that have a reference volume, level by level.
+    """
+    import torch
+
+    out_dir = pathlib.Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    nt, nz, ncol = eta.shape[0], v_ref.shape[0], eta[0].numel()
+    wet = np.flatnonzero(~torch.isnan(v_ref.reshape(nz, ncol)[0]).cpu().numpy())
+    n = min(wet.size, DUMP_BYTES // (8 * (nt + (nz if rho_ref is not None else 0))))
+    cols = np.sort(np.random.default_rng(DUMP_SEED).choice(wet, size=n, replace=False))
+    idx = torch.as_tensor(cols, device=eta.device)
+    arrays = {"eta": eta.reshape(nt, ncol)[:, idx], "sums": sums}
+    if rho_ref is not None:
+        present = ~torch.isnan(v_ref.reshape(nz, ncol)[:, idx])
+        arrays["rho_ref"] = rho_ref.reshape(nz, ncol)[:, idx][present]
+    for name, x in arrays.items():
+        np.save(out_dir / f"{name}.npy", x.double().cpu().numpy())
+    return {"dir": str(out_dir), "files": sorted(f"{k}.npy" for k in arrays),
+            "columns": f"{n} of the {wet.size} with a surface reference volume ({ncol} in all), seed {DUMP_SEED}"}
 
 
 def config_of(args):
@@ -542,6 +585,8 @@ def run_ours(args):
     }
     if world > 1:
         line["host_cpus_bound_per_rank"] = bound_cpus
+    if rank == 0 and args.dump_outputs:
+        line["dump_outputs"] = dump_outputs(args.dump_outputs, eta, rho_ref, sums, V)
     if rank == 0 and not args.no_cpu:
         # the headline's heights against the oracle on columns from every part of the grid (first / last / edge tiles
         # and a stride across the rest); the cpu_baseline leg below also compares the contiguous slab it times

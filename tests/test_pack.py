@@ -107,8 +107,16 @@ def test_scalar_bodies_give_the_same_rows():
 
 
 def test_packing_mode_argument(L):
-    assert L.ml_host_set_packing(5, 0) == -5 and b"packing mode" in L.ml_last_error()
-    assert L.ml_host_set_packing(-1, 0) == -5
-    for mode in (0, 2, 3, 4, 1):
-        assert L.ml_host_set_packing(mode, 0) == 0
-    assert L.ml_host_last_packed_fraction() == 0.0
+    # the packing settings and the accounting of the last host call belong to the calling host thread: a fresh
+    # thread starts from the defaults whatever host calls other tests made on theirs
+    from concurrent.futures import ThreadPoolExecutor
+
+    def body():
+        assert L.ml_host_set_packing(5, 0) == -5 and b"packing mode" in L.ml_last_error()
+        assert L.ml_host_set_packing(-1, 0) == -5
+        for mode in (0, 2, 3, 4, 1):
+            assert L.ml_host_set_packing(mode, 0) == 0
+        assert L.ml_host_last_packed_fraction() == 0.0
+
+    with ThreadPoolExecutor(max_workers=1) as ex:
+        ex.submit(body).result()
