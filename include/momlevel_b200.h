@@ -242,6 +242,31 @@ int ml_steric_global(int eos, int dtype, const void* T, const void* S, int t_bca
                      size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------
+ * ml_steric_global_variants -- the masses of the global steric, thermosteric and halosteric
+ * series in one call.  Replaces calc_masso(rho, reference["volcello"]) of the global branch
+ * (src/momlevel/steric.py:134-135, derived.py:435-438) for the three variants of steric.py:115-121:
+ *   sum rho(T,S) V,   sum rho(T,S_ref) V,   sum rho(T_ref,S) V        per step, V = reference volcello
+ * Fields that suit the TMA family (fp32, 16-byte aligned, ncol % 4 == 0, ncol >= 256) take ONE pass for
+ * all the masses asked for (csrc/ml_tma3.cu), each bit-identical to one ml_steric_global launch; anything
+ * else, a column pressure (ml_set_column_pressure) or a call that asks for one mass only runs one
+ * ml_steric_global per mass.  ml_set_force_direct(2) turns the one-pass kernel off.
+ *   T, S          [nt][nz][ncol] of `dtype`
+ *   T_ref, S_ref  [nz][ncol] of `dtype`: reference["thetao"], reference["so"]; when they are T, S themselves
+ *                 (the same pointers: the reference is step 0, steric.py:105-107) `sums` gets {volo, masso}
+ *                 of the reference state (reference.py:74-80), and must be NULL otherwise
+ *   v_ref         [nz][ncol] reference volcello of `vref_dtype`
+ *   masso_*       device fp64[nt] out each; a NULL pointer skips that variant; at least one is required
+ *   sums          device fp64[2] out (self-reference calls only)
+ *   workspace     ml_workspace_bytes(3 * nt, nz, ncol) bytes
+ * ------------------------------------------------------------------------------------- */
+int ml_steric_global_variants(int eos, int dtype, const void* T, const void* S, const void* T_ref,
+                              const void* S_ref, const void* v_ref, int vref_dtype,
+                              const double* p_level, int64_t nt, int64_t nz, int64_t ncol,
+                              double* masso_steric, double* masso_thermosteric,
+                              double* masso_halosteric, double* sums, void* workspace,
+                              size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------
  * ml_calc_masso -- skipna sums of a field that already exists: out[r] = sum_i rho[r][i] * volcello[i].
  * Replaces derived.calc_masso (src/momlevel/derived.py:414-444: `(rho * volcello).sum(...)` per time step, without
  * the rho * volcello temporary) and, with volcello == NULL, derived.calc_volo (derived.py:769-795:

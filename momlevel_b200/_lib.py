@@ -45,6 +45,8 @@ EXPORTS = {
                                       _vp, _vp, _vp, _vp, _sz, _vp]),
     "ml_calc_masso": (_i, [_i, _vp, _i, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),
     "ml_steric_global": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp, _sz, _vp]),
+    "ml_steric_global_variants": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp,
+                                       _sz, _vp]),
     "ml_host_stream_begin": (_i, [_i, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _d, _i64, _i64, _i64, _i,
                                   ctypes.POINTER(ctypes.c_void_p)]),
     "ml_host_stream_push": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _vp]),

@@ -24,6 +24,7 @@ __all__ = [
     "steric_local_selfref",
     "delta_rho",
     "steric_global",
+    "steric_global_variants",
     "steric_local_host",
     "host_packing",
     "host_last_transfer",
@@ -562,6 +563,44 @@ def steric_global(T, S, v_ref, p_level, eos="Wright", t_bcast=False, s_bcast=Fal
                                ws.data_ptr(), nbytes, _stream())
         )
     return masso
+
+
+GLOBAL_VARIANTS = ("steric", "thermosteric", "halosteric")
+
+
+def steric_global_variants(T, S, v_ref, p_level, T_ref=None, S_ref=None, eos="Wright", variants=GLOBAL_VARIANTS):
+    """The masses of the global steric, thermosteric and halosteric series in one call (steric.py:115-121, :135).
+
+    ``T_ref, S_ref`` default to step 0 of ``T, S`` (what ``steric()`` does without ``reference=``); the sums
+    ``{volo, masso}`` of that reference state are then produced on the way.  ``variants`` may name a subset.
+    Returns ``({variant: masso[nt]}, sums fp64[2] or None)`` on the device (``ml_steric_global_variants``).
+    """
+    L = _lib.lib()
+    p_level, _pcol = _pressure_parts(p_level)
+    T, S, nt, nz, ncol, _ = _steric_operands(T, S, False, False)
+    if (T_ref is None) != (S_ref is None):
+        raise ValueError("T_ref and S_ref are given together or not at all")
+    Tr = T if T_ref is None else to_device(T_ref).to(T.dtype).contiguous()
+    Sr = S if S_ref is None else to_device(S_ref).to(S.dtype).contiguous()
+    selfref = Tr.data_ptr() == T.data_ptr() and Sr.data_ptr() == S.data_ptr()  # step 0 of the fields themselves
+    assert selfref or (Tr.numel() == nz * ncol and Sr.numel() == nz * ncol)
+    v_ref = to_device(v_ref)
+    p = _f64(p_level)
+    assert v_ref.numel() == nz * ncol and p.numel() == nz
+    unknown = set(variants) - set(GLOBAL_VARIANTS)
+    if unknown or not variants:
+        raise ValueError(f"Unknown variants {sorted(unknown)}" if unknown else "at least one variant is required")
+    masso = torch.empty((3, nt), dtype=torch.float64, device=T.device)
+    sums = torch.empty(2, dtype=torch.float64, device=T.device) if selfref else None
+    ws, nbytes = _workspace(3 * nt, nz, ncol, T.device)
+    ptr = lambda i: masso[i].data_ptr() if GLOBAL_VARIANTS[i] in variants else None  # noqa: E731
+    with _pcol:
+        _lib.check(
+            L.ml_steric_global_variants(_eos_id(eos), _dt_id(T), T.data_ptr(), S.data_ptr(), Tr.data_ptr(), Sr.data_ptr(),
+                                        v_ref.data_ptr(), _dt_id(v_ref), p.data_ptr(), nt, nz, ncol, ptr(0), ptr(1), ptr(2),
+                                        sums.data_ptr() if sums is not None else None, ws.data_ptr(), nbytes, _stream())
+        )
+    return {v: masso[i] for i, v in enumerate(GLOBAL_VARIANTS) if v in variants}, sums
 
 
 def _host_tensor(x):

@@ -1022,6 +1022,73 @@ int ml_steric_global(int eos, int dtype, const void* T, const void* S, int t_bca
   return launch_global_direct<double, 1>(T, S, ts, ss, v_ref, v_f32, p_level, (int)nt, (int)nz, ncol, masso, partials, st);
 }
 
+int ml_steric_global_variants(int eos, int dtype, const void* T, const void* S, const void* T_ref, const void* S_ref,
+                              const void* v_ref, int vref_dtype, const double* p_level, int64_t nt, int64_t nz,
+                              int64_t ncol, double* masso_steric, double* masso_thermosteric,
+                              double* masso_halosteric, double* sums, void* workspace, size_t workspace_bytes,
+                              void* stream) {
+  int rc = check_common(eos, dtype);
+  if (rc) return rc;
+  if (vref_dtype != ML_F32 && vref_dtype != ML_F64) return fail(ML_ERR_DTYPE, "unknown vref dtype id %d", vref_dtype);
+  ML_REQUIRE_PTR(T);
+  ML_REQUIRE_PTR(S);
+  ML_REQUIRE_PTR(T_ref);
+  ML_REQUIRE_PTR(S_ref);
+  ML_REQUIRE_PTR(v_ref);
+  ML_REQUIRE_PTR(p_level);
+  const int wanted = (masso_steric != nullptr) + (masso_thermosteric != nullptr) + (masso_halosteric != nullptr);
+  if (wanted == 0) return fail(ML_ERR_NULL, "no output: at least one of the three masses is required");
+  // steric.py:105-107: without a supplied reference the reference state is step 0 of the fields (the same pointers)
+  const bool self_reference = T_ref == T && S_ref == S;
+  if (self_reference && sums == nullptr) return fail(ML_ERR_NULL, "sums is NULL: a self-reference call returns {volo, masso}");
+  if (!self_reference && sums != nullptr) return fail(ML_ERR_MODE, "sums is only produced when T_ref, S_ref are T, S");
+  if (nt <= 0 || nz <= 0 || ncol <= 0 || nt > INT32_MAX / 3 || nz > INT32_MAX)
+    return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ncol=%lld", (long long)nt, (long long)nz, (long long)ncol);
+  if (int rcp = check_column_pressure(ncol)) return rcp;
+  if (workspace == nullptr || workspace_bytes < ml_workspace_bytes(3 * nt, nz, ncol))
+    return fail(ML_ERR_WORKSPACE, "workspace needs %zu bytes, got %zu", ml_workspace_bytes(3 * nt, nz, ncol), workspace_bytes);
+  ML_REQUIRE_ALIGNED(workspace, 8);
+  ML_REQUIRE_ALIGNED(T, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(S, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(T_ref, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(S_ref, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(v_ref, elem_size(vref_dtype));
+  cudaStream_t st = (cudaStream_t)stream;
+  // One pass over T and S for all the masses asked for (csrc/ml_tma3.cu), bit-identical to the launches below.
+  if (tls().force_direct == 0 && !direct_only() && wanted >= 2 &&
+      tma::variants_eligible(dtype, T, S, T_ref, S_ref, vref_dtype, nt, nz, ncol) &&
+      tma::global_variants_partials(nt, ncol) <= workspace_bytes) {
+    tls().last_path = ML_PATH_TMA;
+    return tma::launch_global_variants(eos, T, S, T_ref, S_ref, v_ref, p_level, (int)nt, (int)nz, ncol, masso_steric,
+                                       masso_thermosteric, masso_halosteric, sums, static_cast<double*>(workspace), st);
+  }
+  if (self_reference) {
+    // the scalars of the reference state (reference.py:71-80); the density field itself is not an output here
+    double* rho = nullptr;
+    cudaError_t e = cudaMallocAsync(reinterpret_cast<void**>(&rho), (size_t)nz * (size_t)ncol * sizeof(double), st);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMallocAsync(reference density)");
+    rc = reference_state_impl(eos, dtype, T, S, v_ref, vref_dtype, p_level, nz, ncol, rho, sums, workspace,
+                              workspace_bytes, stream);
+    e = cudaFreeAsync(rho, st);
+    if (rc) return rc;
+    if (e != cudaSuccess) return cuda_fail(e, "cudaFreeAsync(reference density)");
+  }
+  // one single-height launch per wanted mass: thermosteric holds S at the reference slab, halosteric holds T
+  struct Variant {
+    double* masso;
+    const void *T, *S;
+    int t_bcast, s_bcast;
+  };
+  const Variant todo[3] = {{masso_steric, T, S, 0, 0}, {masso_thermosteric, T, S_ref, 0, 1}, {masso_halosteric, T_ref, S, 1, 0}};
+  for (const Variant& v : todo) {
+    if (v.masso == nullptr) continue;
+    if ((rc = ml_steric_global(eos, dtype, v.T, v.S, v.t_bcast, v.s_bcast, v_ref, vref_dtype, p_level, nt, nz, ncol,
+                               v.masso, workspace, workspace_bytes, stream)))
+      return rc;
+  }
+  return ML_OK;
+}
+
 }  // extern "C"
 
 int ml_calc_masso(int dtype, const void* rho, int w_dtype, const void* volcello, int64_t nrows, int64_t n, double* out,

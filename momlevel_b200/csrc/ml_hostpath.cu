@@ -907,7 +907,9 @@ extern "C" int ml_host_stream_begin(int domain, int eos, int dtype, int variants
   hs->nthreads = r.pack_threads > 0 ? std::min(r.pack_threads, 64) : default_threads();
   const size_t es = hs->es, lvl = (size_t)nz * (size_t)ncol, ves = (size_t)elem_size(vref_dtype);
   const size_t win_bytes = (size_t)max_block_steps * lvl * es;
-  hs->ws_bytes = ml_workspace_bytes(local ? 2 : std::max<int64_t>(2, max_block_steps), nz, ncol);
+  // a global stream that asks for two or more masses runs ml_steric_global_variants: three rows of partials per step
+  const int nwanted = (variants & 1) + ((variants >> 1) & 1) + ((variants >> 2) & 1);
+  hs->ws_bytes = ml_workspace_bytes(local ? 2 : std::max<int64_t>(2, (nwanted >= 2 ? 3 : 1) * max_block_steps), nz, ncol);
   auto bail = [&](int rc) {
     stream_fail(hs, rc);
     delete hs;
@@ -984,6 +986,12 @@ extern "C" int ml_host_stream_begin(int domain, int eos, int dtype, int variants
 }
 
 
+// Referenced weakly: this file is also built on its own against a simulated runtime with stand-ins for the
+// single-height entry points only (tests/sim), where the windows then take one ml_steric_global per mass.
+extern "C" int ml_steric_global_variants(int, int, const void*, const void*, const void*, const void*, const void*, int,
+                                         const double*, int64_t, int64_t, int64_t, double*, double*, double*, double*,
+                                         void*, size_t, void*) __attribute__((weak));
+
 extern "C" int ml_host_stream_push(void* stream, const void* T_block, const void* S_block, int64_t nt_block,
                                    double* out_steric, double* out_thermosteric, double* out_halosteric) {
   using namespace ml;
@@ -1040,7 +1048,14 @@ extern "C" int ml_host_stream_push(void* stream, const void* T_block, const void
     ML_HS_CUDA(cudaMemcpyAsync(hs->dTref, hs->dT[0], lvl * es, cudaMemcpyDeviceToDevice, r.comp));
     ML_HS_CUDA(cudaMemcpyAsync(hs->dSref, hs->dS[0], lvl * es, cudaMemcpyDeviceToDevice, r.comp));
   }
-  for (int v = 0; v < 3; ++v) {
+  // a global window that asks for two or more masses: all of them from one pass (the reference slabs are device
+  // copies, so this is never a self-reference call; the scalars came from ml_reference_state above)
+  const bool one_pass = !local && hs->want[0] + hs->want[1] + hs->want[2] >= 2 && ml_steric_global_variants != nullptr;
+  if (one_pass)
+    ML_HS_RC(ml_steric_global_variants(eos, dtype, hs->dT[b], hs->dS[b], hs->dTref, hs->dSref, hs->dV, vdt, dP, nt_block, nz,
+                                       ncol, hs->dOut[b][0], hs->dOut[b][1], hs->dOut[b][2], nullptr, hs->dWs, hs->ws_bytes,
+                                       r.comp));
+  for (int v = 0; v < 3 && !one_pass; ++v) {
     if (!hs->want[v]) continue;
     // thermosteric holds S at the reference slab, halosteric holds T
     const void* Tv = v == 2 ? hs->dTref : hs->dT[b];

@@ -35,6 +35,15 @@ int launch_variants(int eos, const void* T, const void* S, const void* T_ref, co
                     int nz, int64_t ncol, double* eta_steric, double* eta_thermo, double* eta_halo, double* rho_ref_out,
                     double* sums, double* partials, cudaStream_t st);
 
+// the three global masses per step from one pass (ml_tma3.cu), each bit-identical to one launch_global with
+// BC = 0 / 2 / 1; eligibility is variants_eligible.  sums != NULL: T_ref / S_ref are the step-0 slabs of T / S and
+// {volo, masso} of the reference state are reduced on the way.  Any masso may be NULL.  `partials` holds
+// global_variants_partials(nt, ncol) bytes.
+size_t global_variants_partials(int64_t nt, int64_t ncol);
+int launch_global_variants(int eos, const void* T, const void* S, const void* T_ref, const void* S_ref, const void* v_ref,
+                           const double* p_level, int nt, int nz, int64_t ncol, double* masso_steric,
+                           double* masso_thermo, double* masso_halo, double* sums, double* partials, cudaStream_t st);
+
 // fixed-order second reduction stage (defined in ml_api.cu): out[r] = sum_b partials[r][b]
 int reduce_rows(const double* partials, int64_t nblk, double* out, int nrows, cudaStream_t st);
 

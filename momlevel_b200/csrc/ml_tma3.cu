@@ -292,6 +292,210 @@ __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
   }
 }
 
+// ------------------------------------------------------------------ global masses from one pass
+// The global branch (steric.py:134-135) of the three variants: per step the volume-weighted sums
+//     M_steric = sum rho(T, S) V     M_thermo = sum rho(T, S_ref) V     M_halo = sum rho(T_ref, S) V
+// with V = reference["volcello"] and skipna sums (derived.py:435-438).  The stage layout is the local kernel's
+// (TC rows of T, TC rows of S, one T_ref and one S_ref row per level); there is no z_i / deptho / rho_ref, the weight
+// is the reference volume of the level.  Everything that decides the bits of a mass is the single-height global kernel's
+// (ml_tma.cu, kGlobal): 256-column tiles, columns ranked by the number of levels with a present volume, the dry lane
+// that borrows the first wet lane's column, the per-density instructions, the repair pass and the warp / CTA reduction
+// order, so each mass is bit-identical to one ml_steric_global launch with BC = 0 / 2 / 1.
+//   kGlobal3         T_ref, S_ref supplied
+//   kGlobalSelfRef3  T_ref, S_ref are the step-0 slabs of T, S; the chunk that starts at step 0 also reduces
+//                    {volo, masso} of the reference state (reference.py:71-80) -- the reference density is not stored
+enum GlobalMode3 { kGlobal3 = 1, kGlobalSelfRef3 = 3 };
+
+struct ParamsG3 {
+  const float *T, *S;        // [nt][nz][ncol]  (repair pass)
+  const float *Tref, *Sref;  // [nz][ncol]
+  const float* v_ref;        // [nz][ncol]
+  const double* p_level;
+  int nt, nz, t_start;
+  unsigned nchunks, tiles;
+  i64 ncol;
+  double* partials;          // [3][nt][tiles] masses; kGlobalSelfRef3: then [2][tiles] = {volo, masso}
+};
+
+template <int EOS, int TC, int MODE>
+__global__ void __launch_bounds__(kTile, ctas_per_sm3(TC))
+    k_steric_tma3_global(const __grid_constant__ CUtensorMap mapT, const __grid_constant__ CUtensorMap mapS,
+                         const __grid_constant__ CUtensorMap mapTr, const __grid_constant__ CUtensorMap mapSr,
+                         const ParamsG3 P) {
+  constexpr bool SELFREF = MODE == kGlobalSelfRef3;
+  constexpr int kStages = stages3(TC);
+  constexpr int kRows = 2 * TC + 2;
+  constexpr uint32_t kStageBytes = (uint32_t)kRows * kTile * sizeof(float);
+  constexpr int kStageFloats = kRows * kTile;
+  constexpr int kOffS = TC * kTile, kOffTr = 2 * TC * kTile, kOffSr = (2 * TC + 1) * kTile;
+
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  float* stage_base = reinterpret_cast<float*>(smem_raw);
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)kStages * kStageBytes);
+  uint64_t* empty = full + kStages;
+  int* released = reinterpret_cast<int*>(full + 2 * kStages);
+  double* red = reinterpret_cast<double*>(full + 3 * kStages);  // [kConsumerWarps][3 TC + 2]
+  double* s_p = red + kConsumerWarps * (3 * TC + 2);
+  int* s_key = reinterpret_cast<int*>(s_p + P.nz);
+  int* s_col = s_key + kTile;
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const unsigned tile = blockIdx.x / P.nchunks;
+  const int c0 = (int)tile * kTile;
+  const int t0 = P.t_start + (int)(blockIdx.x - tile * P.nchunks) * TC;
+  const int nz = P.nz;
+  const bool chunk0 = SELFREF && t0 == 0;  // this CTA's chunk starts at the reference step
+
+  auto refill_stage = [&](int z) {
+    const int s = z % kStages;
+    float* d = stage_base + (size_t)s * kStageFloats;
+    mbar_expect_tx(full + s, kStageBytes);
+    tma_load_3d(d, &mapT, full + s, c0, z, t0);
+    tma_load_3d(d + kOffS, &mapS, full + s, c0, z, t0);
+    tma_load_2d(d + kOffTr, &mapTr, full + s, c0, z);
+    tma_load_2d(d + kOffSr, &mapSr, full + s, c0, z);
+  };
+
+  if (tid == 0) {
+#pragma unroll
+    for (int s = 0; s < kStages; ++s) {
+      mbar_init(full + s, 1);
+      mbar_init(empty + s, kConsumerWarps);
+      released[s] = 0;
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    for (int z = 0; z < kStages && z < nz; ++z) refill_stage(z);
+  }
+  for (int i = threadIdx.x; i < nz; i += kTile) s_p[i] = __ldg(P.p_level + i);
+  __syncthreads();
+
+  // the single-height global kernel's column order: ranked by the number of levels whose reference volume is present
+  int col;
+  {
+    const i64 cg = (i64)c0 + tid;
+    int key = 0;
+    if (cg < P.ncol)
+      for (int z = 0; z < nz; ++z) key += vraw_isnan(ld_vraw(P.v_ref, (i64)z * P.ncol + cg)) ? 0 : 1;
+    col = sorted_column(key, reinterpret_cast<unsigned*>(s_key), s_col);
+  }
+
+  const i64 c = (i64)c0 + col;
+  const bool in = c < P.ncol;
+  const i64 cc = in ? c : (P.ncol - 1);
+  Eos<EOS> eos;
+  double acc[3][TC];
+#pragma unroll
+  for (int v = 0; v < 3; ++v)
+#pragma unroll
+    for (int k = 0; k < TC; ++k) acc[v][k] = 0.0;
+  double vol = 0.0, mass = 0.0;
+  unsigned v_n = ld_vraw(P.v_ref, cc);
+
+  for (int z = 0; z < nz; ++z) {
+    const unsigned v_z = v_n;
+    if (z + 1 < nz) v_n = ld_vraw(P.v_ref, (i64)(z + 1) * P.ncol + cc);
+    const bool dry = vraw_isnan(v_z);
+    const double w = dry ? 0.0 : vraw_value(v_z);  // rho * NaN is dropped by the skipna sum (derived.py:435-438)
+    eos.set_level(s_p[z]);
+    const bool live = nonzero(w);
+    const unsigned live_lanes = __ballot_sync(0xffffffffu, live);
+    const int s = z % kStages;
+    const float* st = stage_base + (size_t)s * kStageFloats;
+    mbar_wait(full + s, (uint32_t)(z / kStages) & 1u);
+    if (live_lanes != 0u) {
+      const int first_wet = __shfl_sync(0xffffffffu, col, __ffs(live_lanes) - 1);
+      const int src = live ? col : first_wet;
+      const typename Eos<EOS>::Pinned qs = eos.pin_s((double)st[kOffSr + src]);  // thermosteric: S held at S_ref
+      const typename Eos<EOS>::Pinned qt = eos.pin_t((double)st[kOffTr + src]);  // halosteric: T held at T_ref
+#pragma unroll
+      for (int kk = 0; kk < TC; ++kk) {
+        const double Tv = (double)st[kk * kTile + src];
+        const double Sv = (double)st[kOffS + kk * kTile + src];
+        acc[0][kk] = fma(w, eos.rho(Tv, Sv), acc[0][kk]);
+        acc[1][kk] = fma(w, eos.rho_pinned_s(qs, Tv), acc[1][kk]);
+        acc[2][kk] = fma(w, eos.rho_pinned_t(qt, Sv), acc[2][kk]);
+      }
+    }
+    if (chunk0 && in && !dry) {  // volo, masso of the reference state: skipna sums (derived.py:787-789, :435-438)
+      const double r = eos.rho((double)st[kOffTr + col], (double)st[kOffSr + col]);  // reference.py:71
+      vol += w;
+      const double m = r * w;
+      if (!is_nan_q(m)) mass += m;
+    }
+    __syncwarp();
+    if (lane == 0 && stage_done(empty + s, released + s, kConsumerWarps, (uint32_t)(z / kStages) & 1u) && z + kStages < nz)
+      refill_stage(z + kStages);
+  }
+
+  // Repair pass (ml_tma.cu): a column whose sums met a hole at a wet cell is summed again from global memory with the
+  // skipna rule.  A mass that met no hole comes out as it was (same FMAs in the same order), so repairing the three
+  // together keeps each of them identical to its single-height launch.
+  bool poisoned = false;
+#pragma unroll
+  for (int v = 0; v < 3; ++v)
+#pragma unroll
+    for (int k = 0; k < TC; ++k) poisoned |= is_nan_q(acc[v][k]);
+  if (poisoned && in) {
+#pragma unroll
+    for (int v = 0; v < 3; ++v)
+#pragma unroll
+      for (int k = 0; k < TC; ++k) acc[v][k] = 0.0;
+    const i64 lvl = (i64)nz * P.ncol;
+    for (int z = 0; z < nz; ++z) {
+      const i64 j = (i64)z * P.ncol + c;
+      const unsigned vr = ld_vraw(P.v_ref, j);
+      const double w = vraw_isnan(vr) ? 0.0 : vraw_value(vr);
+      if (!nonzero(w)) continue;
+      eos.set_level(s_p[z]);
+      const typename Eos<EOS>::Pinned qs = eos.pin_s((double)__ldg(P.Sref + j));
+      const typename Eos<EOS>::Pinned qt = eos.pin_t((double)__ldg(P.Tref + j));
+#pragma unroll
+      for (int k = 0; k < TC; ++k) {
+        if (t0 + k >= P.nt) continue;
+        const double Tv = (double)__ldg(P.T + (i64)(t0 + k) * lvl + j);
+        const double Sv = (double)__ldg(P.S + (i64)(t0 + k) * lvl + j);
+        fma_skipnan(acc[0][k], w, eos.rho(Tv, Sv));
+        fma_skipnan(acc[1][k], w, eos.rho_pinned_s(qs, Tv));
+        fma_skipnan(acc[2][k], w, eos.rho_pinned_t(qt, Sv));
+      }
+    }
+  }
+
+  // warp sums, then the CTA's warps in order (the single-height kernel's order per mass)
+  constexpr int kRed = 3 * TC + 2;
+#pragma unroll
+  for (int v = 0; v < 3; ++v)
+#pragma unroll
+    for (int k = 0; k < TC; ++k) {
+      const double sacc = warp_sum(in ? acc[v][k] : 0.0);
+      if (lane == 0) red[warp * kRed + v * TC + k] = sacc;
+    }
+  if (chunk0) {  // uniform per CTA
+    vol = warp_sum(vol);
+    mass = warp_sum(mass);
+    if (lane == 0) {
+      red[warp * kRed + 3 * TC] = vol;
+      red[warp * kRed + 3 * TC + 1] = mass;
+    }
+  }
+  __syncthreads();
+  if (tid < 3 * TC) {
+    const int v = tid / TC, k = tid - v * TC;
+    if (t0 + k < P.nt) {
+      double sacc = 0.0;
+#pragma unroll
+      for (int w8 = 0; w8 < kConsumerWarps; ++w8) sacc += red[w8 * kRed + tid];
+      P.partials[((i64)v * P.nt + t0 + k) * P.tiles + tile] = sacc;
+    }
+  } else if (chunk0 && tid < 3 * TC + 2) {
+    double sacc = 0.0;
+#pragma unroll
+    for (int w8 = 0; w8 < kConsumerWarps; ++w8) sacc += red[w8 * kRed + tid];
+    P.partials[((i64)3 * P.nt + (tid - 3 * TC)) * P.tiles + tile] = sacc;
+  }
+}
+
 // ----------------------------------------------------------------------- host side
 template <int TC, int TILE>
 static size_t smem_bytes3(int nz) {
@@ -426,6 +630,93 @@ int launch_variants(int eos, const void* T, const void* S, const void* T_ref, co
                        : launch_all3<kSelfRef3, 256>(eos, T, S, T_ref, S_ref, P, st);
   if (rc) return rc;
   return reduce_rows(partials, (ncol + tile - 1) / tile, sums, 2, st);
+}
+
+// global masses: 256-column tiles whatever ML_TMA3_TILE says (the column order inside a tile decides the bits)
+template <int TC>
+static size_t smem_bytes_g3(int nz) {
+  return (size_t)stages3(TC) * (size_t)((2 * TC + 2) * kTile * 4) + 3 * stages3(TC) * sizeof(uint64_t) +
+         (size_t)kConsumerWarps * (3 * TC + 2) * sizeof(double) + (size_t)nz * sizeof(double) + 2 * kTile * sizeof(int) + 128;
+}
+
+template <int EOS, int TC, int MODE>
+static int launch_one_g3(const CUtensorMap maps[4], const ParamsG3& P, unsigned tiles, unsigned chunks, cudaStream_t st) {
+  auto kern = k_steric_tma3_global<EOS, TC, MODE>;
+  const size_t smem = smem_bytes_g3<TC>(P.nz);
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(k_steric_tma3_global)");
+  ParamsG3 Q = P;
+  Q.tiles = tiles;
+  Q.nchunks = chunks;
+  kern<<<tiles * chunks, kTile, smem, st>>>(maps[0], maps[1], maps[2], maps[3], Q);
+  return launched("k_steric_tma3_global");
+}
+
+template <int MODE>
+static int launch_span_g3(int eos, ParamsG3 P, int t_begin, int t_end, int tc, cudaStream_t st) {
+  CUtensorMap maps[4];
+  const bool ok = make_map(&maps[0], P.T, 3, P.ncol, P.nz, P.nt, tc) && make_map(&maps[1], P.S, 3, P.ncol, P.nz, P.nt, tc) &&
+                  make_map(&maps[2], P.Tref, 2, P.ncol, P.nz, 1, 1) && make_map(&maps[3], P.Sref, 2, P.ncol, P.nz, 1, 1);
+  if (!ok) return fail(ML_ERR_ALIGN, "cuTensorMapEncodeTiled rejected the field layout");
+  P.t_start = t_begin;
+  const unsigned tiles = (unsigned)((P.ncol + kTile - 1) / kTile);
+  const unsigned chunks = (unsigned)((t_end - t_begin + tc - 1) / tc);
+#define ML_TMA3G_GO(E, TCV) return launch_one_g3<E, TCV, MODE>(maps, P, tiles, chunks, st)
+  if (eos == ML_EOS_WRIGHT) {
+    if (tc == 12) ML_TMA3G_GO(0, 12);
+    if (tc == 8) ML_TMA3G_GO(0, 8);
+    if (tc == 6) ML_TMA3G_GO(0, 6);
+    ML_TMA3G_GO(0, 4);
+  }
+  if (tc == 12) ML_TMA3G_GO(1, 12);
+  if (tc == 8) ML_TMA3G_GO(1, 8);
+  if (tc == 6) ML_TMA3G_GO(1, 6);
+  ML_TMA3G_GO(1, 4);
+#undef ML_TMA3G_GO
+}
+
+template <int MODE>
+static int launch_all_g3(int eos, const ParamsG3& P, cudaStream_t st) {
+  const int main_tc = main_tc3();
+  const int full = P.nt / main_tc, rest = P.nt % main_tc;
+  int rc = ML_OK;
+  if (full > 0) rc = launch_span_g3<MODE>(eos, P, 0, full * main_tc, main_tc, st);
+  if (rc == ML_OK && rest > 0) {
+    const int tc = rest <= 4 ? 4 : (rest <= 6 ? 6 : (rest <= 8 ? 8 : 12));
+    rc = launch_span_g3<MODE>(eos, P, full * main_tc, P.nt, tc, st);
+  }
+  return rc;
+}
+
+size_t global_variants_partials(int64_t nt, int64_t ncol) {
+  return (size_t)(3 * nt + 2) * (size_t)((ncol + kTile - 1) / kTile) * sizeof(double);
+}
+
+int launch_global_variants(int eos, const void* T, const void* S, const void* T_ref, const void* S_ref, const void* v_ref,
+                           const double* p_level, int nt, int nz, int64_t ncol, double* masso_steric,
+                           double* masso_thermo, double* masso_halo, double* sums, double* partials, cudaStream_t st) {
+  ParamsG3 P;
+  P.T = static_cast<const float*>(T);
+  P.S = static_cast<const float*>(S);
+  P.Tref = static_cast<const float*>(T_ref);
+  P.Sref = static_cast<const float*>(S_ref);
+  P.v_ref = static_cast<const float*>(v_ref);
+  P.p_level = p_level;
+  P.nt = nt;
+  P.nz = nz;
+  P.t_start = 0;
+  P.nchunks = 1;
+  P.tiles = 0;
+  P.ncol = ncol;
+  P.partials = partials;
+  int rc = sums != nullptr ? launch_all_g3<kGlobalSelfRef3>(eos, P, st) : launch_all_g3<kGlobal3>(eos, P, st);
+  if (rc) return rc;
+  const int64_t tiles = (ncol + kTile - 1) / kTile;
+  double* outs[3] = {masso_steric, masso_thermo, masso_halo};
+  for (int v = 0; v < 3; ++v)
+    if (outs[v] != nullptr && (rc = reduce_rows(partials + (size_t)v * nt * tiles, tiles, outs[v], nt, st))) return rc;
+  if (sums != nullptr) rc = reduce_rows(partials + (size_t)3 * nt * tiles, tiles, sums, 2, st);
+  return rc;
 }
 
 }  // namespace tma

@@ -83,8 +83,9 @@ def steric(
         # (core.HostStream), never asked for as whole arrays
         if reference is not None:
             assert isinstance(reference, Dataset), "`reference` must be an xarray Dataset"
-        reference, streamed = _streamed(dset, reference, pres, equation_of_state, variant, domain, rhozero, tcoord,
+        reference, streamed = _streamed(dset, reference, pres, equation_of_state, (variant,), domain, rhozero, tcoord,
                                         zcoord, zbounds, verbose)
+        streamed = streamed[variant]
         if domain != "global":
             fused_eta = streamed
     elif reference is not None:
@@ -135,7 +136,7 @@ def steric(
             # fields in host memory (a daily series does not fit in HBM): streamed through device windows, level rows
             # packed to the cells of the reference volume on the way; the thermo- / halosteric variants keep their
             # reference slab on the device for the whole series (ml_host_stream_*)
-            masso = _global_host(dset, reference, variant, pres, equation_of_state).numpy()
+            masso = _global_host(dset, reference, (variant,), pres, equation_of_state)[variant].numpy()
         else:
             masso = core.steric_global(thetao.data, so.data, v_ref, pres, eos=equation_of_state,
                                        t_bcast=t_bcast, s_bcast=s_bcast).cpu().numpy()
@@ -419,27 +420,30 @@ def _selfref(dset, pres, eos, variant, rhozero, tcoord, zcoord, zbounds, deferre
     return _reference_from_pass(dset, tcoord, eos, rho, sums, pres), eta, area_total
 
 
-def _global_host(dset, reference, variant, pres, eos):
-    """``calc_masso(rho, reference.volcello)`` per step (steric.py:135) for fields in host memory, any variant."""
+def _global_host(dset, reference, variants, pres, eos, tcoord="time"):
+    """``calc_masso(rho, reference.volcello)`` per step (steric.py:135) for fields in host memory, for each of
+    ``variants`` -- two or more of them from one pass over the fields.  ``reference=None``: the reference state is
+    step 0 of the fields (its volume taken from ``dset``).  Returns ``{variant: CPU tensor [nt]}``."""
     T, S = dset["thetao"].data, dset["so"].data
     nt = int(T.shape[0])
     step_bytes = 2 * int(np.prod(T.shape[1:])) * (4 if str(T.dtype).endswith("float32") else 8)
     spw = int(min(max(1, -(-(1 << 28) // step_bytes)), nt))  # windows of >= 256 MB
     ref = None
-    if variant != "steric":
+    if reference is not None and any(v != "steric" for v in variants):
         ref = {"thetao": _host_array(reference["thetao"]), "so": _host_array(reference["so"])}
+    V = reference["volcello"] if reference is not None else dset["volcello"].isel({tcoord: 0}).squeeze()
     f32 = str(T.dtype).endswith("float32") and str(S.dtype).endswith("float32")
-    hs = core.HostStream("global", _host_array(reference["volcello"]), _host_numpy(pres), variants=(variant,), reference=ref,
+    hs = core.HostStream("global", _host_array(V), _host_numpy(pres), variants=tuple(variants), reference=ref,
                          eos=eos, max_block_steps=spw, dtype=torch.float32 if f32 else torch.float64)
     outs = []
     try:
         for t in range(0, nt, spw):
-            outs.append(hs.push(T[t: t + spw], S[t: t + spw])[variant])
+            outs.append(hs.push(T[t: t + spw], S[t: t + spw]))
         hs.finish()
     except BaseException:
         hs.abort()
         raise
-    return torch.cat(outs) if len(outs) != 1 else outs[0]
+    return {v: torch.cat([o[v] for o in outs]) if len(outs) != 1 else outs[0][v] for v in variants}
 
 
 def _chunked(dset):
@@ -486,13 +490,15 @@ def _host_array(x):
     return x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else np.asarray(x)
 
 
-def _streamed(dset, reference, pres, eos, variant, domain, rhozero, tcoord, zcoord, zbounds, verbose=False):
+def _streamed(dset, reference, pres, eos, variants, domain, rhozero, tcoord, zcoord, zbounds, verbose=False,
+              first_step_sums=None):
     """The heights (local) or masses (global) of fields that arrive block by block, and the reference Dataset.
 
-    One pass over the blocks of ``thetao`` / ``so`` through ``core.HostStream``: a block is packed, copied and
-    integrated while the next one is being produced, and at most two blocks are alive at a time.  With
-    ``reference=None`` the reference state is step 0 of the first block (steric.py:105-107).
-    Returns ``(reference, CPU tensor)``.
+    One pass over the blocks of ``thetao`` / ``so`` through ``core.HostStream`` for all of ``variants``: a block is
+    packed, copied and integrated while the next one is being produced, and at most two blocks are alive at a time.
+    With ``reference=None`` the reference state is step 0 of the first block (steric.py:105-107); its
+    ``{volo, masso}`` come from the stream, or from ``first_step_sums(T0, S0, V0)`` when that is given.
+    Returns ``(reference, {variant: CPU tensor})``.
     """
     from .util import eos_func_from_str
 
@@ -511,7 +517,7 @@ def _streamed(dset, reference, pres, eos, variant, domain, rhozero, tcoord, zcoo
             print("Using supplied reference state")
         V0 = _host_array(reference["volcello"])
         ref = {"rho": _host_array(reference["rho"])} if local else {}
-        if variant != "steric":
+        if any(v != "steric" for v in variants):
             ref.update(thetao=_host_array(reference["thetao"]), so=_host_array(reference["so"]))
         if not ref:  # the masses of the steric variant need the reference volume only
             ref = None
@@ -524,20 +530,23 @@ def _streamed(dset, reference, pres, eos, variant, domain, rhozero, tcoord, zcoo
     dt = torch.float32 if str(T._data.dtype).endswith("float32") and str(S._data.dtype).endswith("float32") else torch.float64
     hs = core.HostStream("local" if local else "global", V0, _host_numpy(pres),
                          z_i=_host_array(dset[zbounds]) if local else None,
-                         deptho=_host_array(dset["deptho"]) if local else None, variants=(variant,), reference=ref,
-                         rhozero=rhozero, eos=eos, max_block_steps=max_len, dtype=dt, want_sums=not supplied)
+                         deptho=_host_array(dset["deptho"]) if local else None, variants=tuple(variants), reference=ref,
+                         rhozero=rhozero, eos=eos, max_block_steps=max_len, dtype=dt,
+                         want_sums=not supplied and first_step_sums is None)
     outs, first = [], None
     try:
         for Tb, Sb in blocks:
             if first is None and not supplied:  # step 0 becomes the reference Dataset (reference.py:60-68)
                 first = (np.array(Tb[0]), np.array(Sb[0]))
-            outs.append(hs.push(Tb, Sb)[variant])
+            outs.append(hs.push(Tb, Sb))
         _, sums = hs.finish()
     except BaseException:
         hs.abort()
         raise
-    out = torch.cat(outs) if len(outs) != 1 else outs[0]
+    out = {v: torch.cat([o[v] for o in outs]) if len(outs) != 1 else outs[0][v] for v in variants}
     if not supplied:
+        if first_step_sums is not None:
+            sums = first_step_sums(first[0], first[1], V0)
         sub = Dataset()
         hdims = T.dims[1:]
         sub["thetao"] = DataArray(first[0], hdims, attrs=T.attrs)
@@ -548,7 +557,8 @@ def _streamed(dset, reference, pres, eos, variant, domain, rhozero, tcoord, zcoo
             if name in dset.variables:
                 sub[name] = dset[name]
         sub = _with_time_axis(sub, tcoord)
-        reference = _reference_from_pass(sub, tcoord, eos, None, torch.tensor(sums, dtype=torch.float64), pres)
+        sums = sums if isinstance(sums, torch.Tensor) else torch.tensor(sums, dtype=torch.float64)
+        reference = _reference_from_pass(sub, tcoord, eos, None, sums, pres)
     return reference, out
 
 
@@ -587,25 +597,138 @@ VARIANTS = ("steric", "thermosteric", "halosteric")
 
 
 def steric_variants(dset, reference=None, coord_names=None, varname_map=None, rhozero=1035.0, patm=101325.0,
-                    equation_of_state="Wright", dtype="float32", strict=True, verbose=False):
-    """Steric, thermosteric and halosteric height (``domain="local"``) from one call.
+                    equation_of_state="Wright", dtype="float32", strict=True, verbose=False, domain="local", annual=False,
+                    days_in_month=None):
+    """Steric, thermosteric and halosteric sea level from one call, in either domain.
 
     Equivalent to ``steric(dset)``, ``thermosteric(dset)`` and ``halosteric(dset)`` (steric.py:115-121 only
     changes which operand of the equation of state is held at its reference value) with the validation, the
-    reference state and the result assembly done once.  Arguments as :func:`steric`.  Returns
-    ``(result, reference)``; ``result`` holds the three height variables (no ``delta_rho``: there is one per
-    variant -- ask :func:`steric` for the variant whose 4-D anomaly is wanted).
+    reference state and the result assembly done once, and T and S read once for the three.  Arguments as
+    :func:`steric`.  Returns ``(result, reference)``: ``domain="local"`` gives the three height fields,
+    ``domain="global"`` the three ``(time,)`` series and ``reference_height``.  There is no ``delta_rho`` (one per
+    variant): ask :func:`steric` for the variant whose 4-D anomaly is wanted.
     """
-    from .util import eos_func_from_str
+    xarray_in = type(dset).__module__.startswith("xarray")
+    if xarray_in:
+        from . import xarray_io
 
+        dset_x = dset
+        # only what the path reads is converted; dask-backed fields stay in blocks (labeled.ChunkedArray)
+        t_, z_, zb_ = default_coords(coord_names)
+        needed = {"thetao", "so", "volcello", "areacello", "deptho", t_, z_, zb_}
+        needed |= {k for k, v in (varname_map or {}).items() if v in needed}
+        dset = xarray_io.from_xarray(dset, names=sorted(needed))
+        if reference is not None:
+            assert type(reference).__module__.startswith("xarray"), "`reference` must be an xarray Dataset"
+            reference = xarray_io.from_xarray(reference)
     dset = dset.rename(varname_map)
     tcoord, zcoord, zbounds = default_coords(coord_names)
+    args = (dset, reference, tcoord, zcoord, zbounds, rhozero, patm, equation_of_state, strict, verbose)
+    if domain == "global":
+        result, reference = _global_variants(*args)
+    else:
+        result, reference = _local_variants(*args)
+    for variant in VARIANTS:
+        result[variant].attrs = {"long_name": f"{variant.capitalize()} height adjustment", "units": "m"}  # steric.py:169-172
+        result[variant].encoding["dtype"] = dtype
+    if "reference_height" in result.variables:
+        result["reference_height"].encoding["dtype"] = dtype
+    for var in set(result.dims):
+        if var in dset.variables:
+            coord = dset[var].copy(deep=False)
+            coord.attrs = dict(dset[var].attrs)
+            result[var] = coord
+    if annual:  # steric.py:181-182
+        result = annual_average(result, tcoord=tcoord, days_in_month=days_in_month)
+    if xarray_in:
+        return xarray_io.to_xarray(result, like=dset_x), xarray_io.to_xarray(reference, like=dset_x)
+    return (result, reference)
+
+
+def _variants_route(dset, pres, tcoord, zcoord, zbounds, domain):
+    """Where the fields of a three-variant call live, which decides how they are read once for the three:
+    ``"chunked"`` (blocks along time: one ``core.HostStream`` pass over the blocks), ``"host"`` (whole arrays in host
+    memory, large enough for the streaming to pay: one ``HostStream`` pass / ``ml_steric_local_variants_host``) or
+    ``"device"`` (one call of the one-pass entry point on device tensors)."""
+    if _chunked(dset):
+        return "chunked"
+    if not isinstance(pres, core.Pressure) and _host_resident(dset, tcoord, zcoord, zbounds, need_depth=domain != "global"):
+        return "host"
+    return "device"
+
+
+def _first_step_sums(eos):
+    """``{volo, masso}`` of the reference state that is step 0 of the fields, as the device route evaluates them (the
+    self-reference pass of ``ml_steric_global_variants``), for the routes that stream the fields from host memory:
+    all three routes then give the same reference scalars, and so the same series, bit for bit."""
+
+    def sums(T0, S0, V0, pres):
+        return core.steric_global_variants(np.asarray(T0)[None], np.asarray(S0)[None], V0, pres, eos=eos)[1]
+
+    return sums
+
+
+def _global_variants(dset, reference, tcoord, zcoord, zbounds, rhozero, patm, eos, strict, verbose):
+    """The global branch (steric.py:134-147) for the three variants: masses from one pass, then the ln formula."""
+    from .util import eos_func_from_str
+
+    validate_dataset(dset, strict=strict, additional_vars=None)  # steric.py:84-91: no z_i / deptho in this domain
+    pres = _pressure(dset, zcoord, patm)
+    eos_func_from_str(eos)
+    T, S = dset["thetao"], dset["so"]
+    if T.dims[0] != tcoord or T.dims[1] != zcoord or S.dims != T.dims:
+        raise ValueError(f"expecting fields laid out ({tcoord}, {zcoord}, y, x), got {T.dims}")
+    supplied = reference is not None
+    if supplied:
+        assert isinstance(reference, Dataset), "`reference` must be an xarray Dataset"
+        if verbose:
+            print("Using supplied reference state")
+        validate_dataset(reference, reference=True, strict=strict)
+    elif verbose:
+        print("Generating reference state from first timestep")
+    route = _variants_route(dset, pres, tcoord, zcoord, zbounds, "global")
+    sums_of = _first_step_sums(eos)
+    if route == "chunked":
+        reference, masso = _streamed(dset, reference, pres, eos, VARIANTS, "global", rhozero, tcoord, zcoord, zbounds,
+                                     first_step_sums=lambda T0, S0, V0: sums_of(T0, S0, V0, pres))
+    elif route == "host":
+        masso = _global_host(dset, reference, VARIANTS, pres, eos, tcoord)
+        if not supplied:
+            T0, S0 = (_host_array(dset[k].isel({tcoord: 0}).squeeze()) for k in ("thetao", "so"))
+            V0 = _host_array(dset["volcello"].isel({tcoord: 0}).squeeze())
+            reference = _reference_from_pass(dset, tcoord, eos, None, sums_of(T0, S0, V0, pres), pres)
+    elif supplied:
+        masso, _ = core.steric_global_variants(T.data, S.data, reference["volcello"].data, pres, T_ref=reference["thetao"].data,
+                                               S_ref=reference["so"].data, eos=eos)
+    else:
+        V0 = dset["volcello"].isel({tcoord: 0}).squeeze().data
+        masso, sums = core.steric_global_variants(T.data, S.data, V0, pres, eos=eos)
+        reference = _reference_from_pass(dset, tcoord, eos, None, sums, pres)
+    if not supplied:
+        validate_dataset(reference, reference=True, strict=strict)
+    # steric.py:136-147
+    volo, rhoga = float(reference["volo"]), float(reference["rhoga"])
+    reference_height = volo / float(reference["areacello"].sum())
+    result = Dataset()
+    result["reference_height"] = DataArray(np.float64(reference_height), (), attrs={
+        "long_name": "Reference column height", "units": "m"})
+    for variant in VARIANTS:
+        m = masso[variant]
+        m = m.cpu().numpy() if isinstance(m, torch.Tensor) else np.asarray(m)
+        result[variant] = DataArray(reference_height * np.log(rhoga / (m / volo)), (tcoord,))
+    return result, reference
+
+
+def _local_variants(dset, reference, tcoord, zcoord, zbounds, rhozero, patm, eos, strict, verbose):
+    """The local branch (steric.py:150-166) for the three variants: the heights from one pass over T and S."""
+    from .util import eos_func_from_str
+
     # device-resident fields without a supplied reference: the value checks ride behind the launch, as in steric()
     deferred = reference is None and _on_one_cuda_device(
         dset, ("thetao", "so", "volcello", "areacello", "deptho", zcoord, zbounds))
     validate_dataset(dset, strict=strict, additional_vars=[zbounds, "deptho"], area_total=False if deferred else None)
     pres = _pressure(dset, zcoord, patm)
-    eos_func_from_str(equation_of_state)
+    eos_func_from_str(eos)
     if not deferred:
         _check_depths(dset, zcoord, zbounds)
     area_total = None
@@ -614,44 +737,43 @@ def steric_variants(dset, reference=None, coord_names=None, varname_map=None, rh
         raise ValueError(f"expecting fields laid out ({tcoord}, {zcoord}, y, x), got {full.dims}")
     args = (full.data, dset["so"].data)
     tail = (dset[zbounds].data, dset["deptho"].data, pres)
-    kw = dict(rhozero=rhozero, eos=equation_of_state)
+    kw = dict(rhozero=rhozero, eos=eos)
+    route = _variants_route(dset, pres, tcoord, zcoord, zbounds, "local")
     if reference is not None:
         assert isinstance(reference, Dataset), "`reference` must be an xarray Dataset"
         if verbose:
             print("Using supplied reference state")
         validate_dataset(reference, reference=True, strict=strict)
-        etas, _, _ = core.steric_local_variants(*args, reference["volcello"].data, *tail, T_ref=reference["thetao"].data,
-                                                S_ref=reference["so"].data, rho_ref=reference["rho"].data, **kw)
+        if route == "chunked":
+            _, etas = _streamed(dset, reference, pres, eos, VARIANTS, "local", rhozero, tcoord, zcoord, zbounds)
+        else:
+            etas, _, _ = core.steric_local_variants(*args, reference["volcello"].data, *tail, T_ref=reference["thetao"].data,
+                                                    S_ref=reference["so"].data, rho_ref=reference["rho"].data, **kw)
     else:
         if verbose:
             print("Generating reference state from first timestep")
         V0 = dset["volcello"].isel({tcoord: 0}).squeeze().data
-        if not isinstance(pres, core.Pressure) and _host_resident(dset, tcoord, zcoord, zbounds):
+        if route == "chunked":
+            reference, etas = _streamed(dset, None, pres, eos, VARIANTS, "local", rhozero, tcoord, zcoord, zbounds)
+        elif route == "host":
             # fields in host memory: one pass over PCIe feeds the three integrations (ml_steric_local_variants_host)
             step_bytes = 2 * int(np.prod(full.shape[1:])) * 4
             spw = int(min(max(1, -(-(1 << 28) // step_bytes)), full.shape[0]))
             etas, _, (volo, masso) = core.steric_local_host(
                 *args, V0, _host_numpy(dset[zbounds].data), _host_numpy(dset["deptho"].data), _host_numpy(pres),
                 steps_per_window=spw, variants=True, **kw)
-            reference = _reference_from_pass(dset, tcoord, equation_of_state, None,
+            reference = _reference_from_pass(dset, tcoord, eos, None,
                                              torch.tensor([volo, masso], dtype=torch.float64), pres)
         else:
             etas, rho, sums = core.steric_local_variants(*args, V0, *tail, **kw)
             if deferred:
                 area_total = _device_grid_checks(dset, zcoord, zbounds, strict, [zbounds, "deptho"])
-            reference = _reference_from_pass(dset, tcoord, equation_of_state, rho, sums)
+            reference = _reference_from_pass(dset, tcoord, eos, rho, sums)
         validate_dataset(reference, reference=True, strict=strict, area_total=area_total)
     result = Dataset()
     for variant in VARIANTS:
-        result[variant] = DataArray(etas[variant], (tcoord,) + full.dims[2:], attrs={
-            "long_name": f"{variant.capitalize()} height adjustment", "units": "m"})  # steric.py:169-172
-        result[variant].encoding["dtype"] = dtype
-    for var in set(result.dims):
-        if var in dset.variables:
-            coord = dset[var].copy(deep=False)
-            coord.attrs = dict(dset[var].attrs)
-            result[var] = coord
-    return (result, reference)
+        result[variant] = DataArray(etas[variant], (tcoord,) + full.dims[2:])
+    return result, reference
 
 
 def halosteric(*args, **kwargs):
