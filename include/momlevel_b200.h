@@ -230,6 +230,25 @@ int ml_steric_local_variants(int eos, int dtype, const void* T, const void* S, c
                              void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------
+ * ml_steric_local_layers -- the local height of ml_steric_local split by depth layer, from one pass:
+ *   eta[t][b][col] = coef * sum_z calc_dz(top=edges[b], bottom=edges[b+1]) * (rho - rho_ref),
+ * masked where v_ref at the surface is missing (NaN in every layer); a layer wholly below a wet column's
+ * sea floor is 0.0.  calc_dz is derived.calc_dz (derived.py:295-318), so at a partial bottom cell that
+ * straddles an inner edge the layers add up to more than the full column, as in the reference.
+ *   edges       HOST pointer to nlayers + 1 strictly increasing values >= 0; the last may be +inf
+ *               (to the sea floor).  1 <= nlayers <= ML_MAX_LAYERS; anything else returns ML_ERR_SHAPE
+ *   eta         [nt][nlayers][ncol] fp64 out
+ * Other arguments as ml_steric_local (no delta_rho output); reads the thread's column pressure like it.
+ * nlayers == 1 with edges {0, +inf} is bit-identical to ml_steric_local.
+ * ------------------------------------------------------------------------------------- */
+#define ML_MAX_LAYERS 8
+int ml_steric_local_layers(int eos, int dtype, const void* T, const void* S, int t_bcast, int s_bcast,
+                           const double* rho_ref, const void* v_ref, int vref_dtype, const double* z_i,
+                           const double* deptho, const double* p_level, double neg_inv_rhozero,
+                           const double* edges, int nlayers, int64_t nt, int64_t nz, int64_t ncol,
+                           double* eta, void* stream);
+
+/* ---------------------------------------------------------------------------------------
  * ml_steric_global -- fused EOS -> sum_{z,col} rho * v_ref per time step.
  * Replaces calc_masso(rho, reference["volcello"]) in the global branch
  * (src/momlevel/steric.py:135, derived.py:435-438); the ln() formula (steric.py:136-142)

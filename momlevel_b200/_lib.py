@@ -11,7 +11,7 @@ import pathlib
 from . import _build
 
 __all__ = ["lib", "check", "MLError", "F32", "F64", "EOS_IDS", "FUNC_IDS", "P_SCALAR", "P_PER_LEVEL", "P_FULL",
-           "PATH_DIRECT", "PATH_TMA", "EXPORTS"]
+           "PATH_DIRECT", "PATH_TMA", "MAX_LAYERS", "EXPORTS"]
 
 F32, F64 = 0, 1
 EOS_IDS = {"wright": 0, "linear": 1}
@@ -19,6 +19,7 @@ FUNC_IDS = {"density": 0, "drho_dtemp": 1, "drho_dsal": 2, "alpha": 3, "beta": 4
 P_SCALAR, P_PER_LEVEL, P_FULL = 0, 1, 2
 DOMAIN_LOCAL, DOMAIN_GLOBAL = 0, 1
 PATH_DIRECT, PATH_TMA = 1, 2
+MAX_LAYERS = 8  # ML_MAX_LAYERS
 
 _vp, _i, _i64, _d, _sz = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double, ctypes.c_size_t
 
@@ -37,6 +38,8 @@ EXPORTS = {
     "ml_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "ml_reference_state": (_i, [_i, _i, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ml_steric_local": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _d, _i64, _i64, _i64, _vp, _vp, _vp]),
+    "ml_steric_local_layers": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _d, _vp, _i, _i64, _i64, _i64, _vp,
+                                    _vp]),
     "ml_delta_rho": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_delta_rho_annual": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_steric_local_selfref": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _d, _i64, _i64, _i64, _vp, _vp, _vp,

@@ -22,6 +22,8 @@ __all__ = [
     "reference_state",
     "steric_local",
     "steric_local_selfref",
+    "steric_local_layers",
+    "layer_edges",
     "delta_rho",
     "steric_global",
     "steric_global_variants",
@@ -403,6 +405,63 @@ def steric_local(T, S, rho_ref, v_ref, z_i, deptho, p_level, rhozero=1035.0, eos
                               drho.data_ptr() if drho is not None else None, _stream())
         )
     return eta, drho
+
+
+def layer_edges(edges):
+    """Depth-layer edges as a float64 numpy array: ``None`` as the last edge means "to the sea floor" and becomes
+    ``inf`` (``calc_dz(bottom=None)`` is ``calc_dz(bottom=inf)``, derived.py:297-298).  Raises ``ValueError`` unless
+    there are 2 to ``MAX_LAYERS + 1`` edges, strictly increasing, >= 0, with only the last one infinite."""
+    try:
+        vals = list(edges)
+    except TypeError:
+        raise ValueError(f"depth edges must be a sequence of depths, got {edges!r}") from None
+    if not 2 <= len(vals) <= _lib.MAX_LAYERS + 1:
+        raise ValueError(f"depth edges must give 1 to {_lib.MAX_LAYERS} layers, got {len(vals)} edges")
+    out = []
+    for i, v in enumerate(vals):
+        if v is None:
+            if i != len(vals) - 1:
+                raise ValueError("only the last depth edge may be None (to the sea floor)")
+            v = np.inf
+        try:
+            v = float(v)
+        except (TypeError, ValueError):
+            raise ValueError(f"depth edge {v!r} is not a number") from None
+        if np.isnan(v) or v < 0.0 or (np.isinf(v) and i != len(vals) - 1):
+            raise ValueError(f"depth edges must be >= 0 and finite except the last, got {v!r}")
+        if out and not v > out[-1]:
+            raise ValueError(f"depth edges must be strictly increasing, got {vals!r}")
+        out.append(v)
+    return np.asarray(out, dtype=np.float64)
+
+
+def steric_local_layers(T, S, rho_ref, v_ref, z_i, deptho, p_level, edges, rhozero=1035.0, eos="Wright", t_bcast=False,
+                        s_bcast=False):
+    """The local branch (steric.py:150-166) split by depth layer: layer ``b`` integrates with
+    ``calc_dz(top=edges[b], bottom=edges[b+1])`` (derived.py:249-325) in place of the full-column thickness.
+
+    ``edges`` as :func:`layer_edges`.  Returns ``eta [nt, nlayers, ...]`` fp64 on the device, from one pass over
+    T and S (``ml_steric_local_layers``).
+    """
+    L = _lib.lib()
+    e = layer_edges(edges)
+    p_level, _pcol = _pressure_parts(p_level)
+    T, S, nt, nz, ncol, hshape = _steric_operands(T, S, t_bcast, s_bcast)
+    rho_ref = _f64(rho_ref)
+    v_ref = to_device(v_ref)
+    z_i, depth, p = _f64(z_i), _f64(deptho), _f64(p_level)
+    assert rho_ref.numel() == nz * ncol and v_ref.numel() == nz * ncol and depth.numel() == ncol
+    assert z_i.numel() == nz + 1 and p.numel() == nz
+    nl = e.size - 1
+    eta = torch.empty((nt, nl) + hshape, dtype=torch.float64, device=T.device)
+    with _pcol:
+        _lib.check(
+            L.ml_steric_local_layers(_eos_id(eos), _dt_id(T), T.data_ptr(), S.data_ptr(), int(t_bcast), int(s_bcast),
+                                     rho_ref.data_ptr(), v_ref.data_ptr(), _dt_id(v_ref), z_i.data_ptr(),
+                                     depth.data_ptr(), p.data_ptr(), -1.0 / rhozero,
+                                     e.ctypes.data_as(ctypes.c_void_p), nl, nt, nz, ncol, eta.data_ptr(), _stream())
+        )
+    return eta
 
 
 def delta_rho(T, S, rho_ref, v_ref, p_level, eos="Wright", t_bcast=False, s_bcast=False):

@@ -339,13 +339,22 @@ __global__ void __launch_bounds__(kBlock) k_reference_state_vec(const TIn* __res
 }
 
 // ------------------------------------------------------------- K3 direct: local steric
-template <typename TIn, int EOS, bool WRITE_DRHO>
+// Layer edges of ml_steric_local_layers, passed by value.
+struct LayerEdges {
+  int n;                           // layers
+  double e[ML_MAX_LAYERS + 1];     // increasing; the last may be +inf
+};
+
+// LAYERS: the height split by depth layer (ml_steric_local_layers), eta [nt][nlayers][ncol]; level z feeds layer b
+// with calc_dz(top=e[b], bottom=e[b+1]) (derived.py:295-318) and a layer is stored when the sweep leaves it.
+template <typename TIn, int EOS, bool WRITE_DRHO, bool LAYERS = false>
 __global__ void __launch_bounds__(kBlock)
     k_steric_local_direct(const TIn* __restrict__ T, const TIn* __restrict__ S, i64 t_stride, i64 s_stride,
                           const double* __restrict__ rho_ref, const void* __restrict__ v_ref, int v_f32,
                           const double* __restrict__ z_i, const double* __restrict__ deptho,
                           const double* __restrict__ p_level, const double* __restrict__ p_col, double coef, int nt,
-                          int nz, i64 ncol, double* __restrict__ eta, double* __restrict__ drho) {
+                          int nz, i64 ncol, double* __restrict__ eta, double* __restrict__ drho,
+                          const LayerEdges L = LayerEdges()) {
   const i64 c = (i64)blockIdx.x * kBlock + threadIdx.x;
   if (c >= ncol) return;
   const int t0 = blockIdx.y * kTC;
@@ -360,10 +369,36 @@ __global__ void __launch_bounds__(kBlock)
   for (int k = 0; k < kTC; ++k) acc[k] = 0.0;
   Eos<EOS> eos;
   const double pc = p_col != nullptr ? __ldg(p_col + c) : 0.0;  // a 2-D patm (steric.py:96)
+  int cur = 0;  // LAYERS: the layer the sums belong to
+  auto store_layer = [&](int b, int k, double a) {
+    if (t0 + k < nt) eta[((i64)(t0 + k) * L.n + b) * ncol + c] = surface_wet ? coef * a : nan("");
+  };
+  auto close_layer = [&](int b) {
+#pragma unroll
+    for (int k = 0; k < kTC; ++k) {
+      store_layer(b, k, acc[k]);
+      acc[k] = 0.0;
+    }
+  };
 
   for (int z = 0; z < nz; ++z) {
     const i64 i = (i64)z * lvl + c;
-    const double dz = clipped_dz(depth, __ldg(z_i + z), __ldg(z_i + z + 1));
+    const double ztop = __ldg(z_i + z), zbot = __ldg(z_i + z + 1);
+    const double dz = clipped_dz(depth, ztop, zbot);
+    // LAYERS: layers lo .. hi touch this level (z_i[z+1] > e[b] && z_i[z] < e[b+1]); a level no layer touches
+    // adds nothing.  Layers that ended above it are stored first.
+    int lo = -1, hi = -1;
+    if (LAYERS) {
+      for (int b = 0; b < L.n; ++b)
+        if (zbot > L.e[b] && ztop < L.e[b + 1]) {
+          if (lo < 0) lo = b;
+          hi = b;
+        }
+      if (lo < 0) continue;
+      for (; cur < lo; ++cur) close_layer(cur);
+    }
+    auto layer_w = [&](int b) { return fmin(fmax(zbot - L.e[b], 0.0), clipped_dz(fmin(depth, L.e[b + 1]), ztop, zbot)); };
+    const double wl = LAYERS ? layer_w(lo) : dz;
     // steric.py:151-153: delta_rho is NaN wherever the reference volume is missing
     const double rref = vref_wet(v_ref, v_f32, i) ? __ldg(rho_ref + i) : nan("");
     eos.set_level(__ldg(p_level + z) + pc);
@@ -382,8 +417,21 @@ __global__ void __launch_bounds__(kBlock)
       if (WRITE_DRHO) {
         if (t0 + k < nt) drho[((i64)(t0 + k) * nz + z) * lvl + c] = d;
       }
-      if (!is_nan_q(d)) acc[k] = fma(dz, d, acc[k]);  // skipna sum, steric.py:163
+      if (LAYERS && lo < hi) {
+        // the level closes layers lo .. hi - 1 and opens hi
+        const bool skip = is_nan_q(d);
+        store_layer(lo, k, skip ? acc[k] : fma(wl, d, acc[k]));
+        for (int b = lo + 1; b < hi; ++b) store_layer(b, k, skip ? 0.0 : layer_w(b) * d);
+        acc[k] = skip ? 0.0 : layer_w(hi) * d;
+      } else if (!is_nan_q(d)) {
+        acc[k] = fma(wl, d, acc[k]);  // skipna sum, steric.py:163
+      }
     }
+    if (LAYERS && lo < hi) cur = hi;  // layers lo .. hi - 1 are stored; the sums now belong to layer hi
+  }
+  if (LAYERS) {
+    for (; cur < L.n; ++cur) close_layer(cur);  // the last layer, and those wholly below the grid: 0
+    return;
   }
 #pragma unroll
   for (int k = 0; k < kTC; ++k) {
@@ -514,6 +562,15 @@ int launch_local_direct(const void* T, const void* S, i64 ts, i64 ss, const doub
     k_steric_local_direct<TIn, EOS, true><<<grid, kBlock, 0, st>>>((const TIn*)T, (const TIn*)S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, tls().p_col, coef, nt, nz, ncol, eta, drho);
   else
     k_steric_local_direct<TIn, EOS, false><<<grid, kBlock, 0, st>>>((const TIn*)T, (const TIn*)S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, tls().p_col, coef, nt, nz, ncol, eta, drho);
+  return launched("k_steric_local_direct");
+}
+
+template <typename TIn, int EOS>
+int launch_layers_direct(const void* T, const void* S, i64 ts, i64 ss, const double* rho_ref, const void* v_ref,
+                         int v_f32, const double* z_i, const double* deptho, const double* p_level, double coef, int nt,
+                         int nz, i64 ncol, double* eta, const LayerEdges& L, cudaStream_t st) {
+  dim3 grid((unsigned)cdiv(ncol, kBlock), (unsigned)cdiv(nt, kTC));
+  k_steric_local_direct<TIn, EOS, false, true><<<grid, kBlock, 0, st>>>((const TIn*)T, (const TIn*)S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, tls().p_col, coef, nt, nz, ncol, eta, nullptr, L);
   return launched("k_steric_local_direct");
 }
 
@@ -816,6 +873,60 @@ int ml_steric_local(int eos, int dtype, const void* T, const void* S, int t_bcas
   }
   if (eos == ML_EOS_WRIGHT) return launch_local_direct<double, 0>(T, S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, eta, delta_rho, st);
   return launch_local_direct<double, 1>(T, S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, eta, delta_rho, st);
+}
+
+int ml_steric_local_layers(int eos, int dtype, const void* T, const void* S, int t_bcast, int s_bcast,
+                           const double* rho_ref, const void* v_ref, int vref_dtype, const double* z_i,
+                           const double* deptho, const double* p_level, double neg_inv_rhozero, const double* edges,
+                           int nlayers, int64_t nt, int64_t nz, int64_t ncol, double* eta, void* stream) {
+  int rc = check_common(eos, dtype);
+  if (rc) return rc;
+  if ((rc = check_bcast(t_bcast, s_bcast))) return rc;
+  if (vref_dtype != ML_F32 && vref_dtype != ML_F64) return fail(ML_ERR_DTYPE, "unknown vref dtype id %d", vref_dtype);
+  ML_REQUIRE_PTR(T);
+  ML_REQUIRE_PTR(S);
+  ML_REQUIRE_PTR(rho_ref);
+  ML_REQUIRE_PTR(v_ref);
+  ML_REQUIRE_PTR(z_i);
+  ML_REQUIRE_PTR(deptho);
+  ML_REQUIRE_PTR(p_level);
+  ML_REQUIRE_PTR(edges);
+  ML_REQUIRE_PTR(eta);
+  if (nlayers < 1 || nlayers > ML_MAX_LAYERS)
+    return fail(ML_ERR_SHAPE, "nlayers=%d: between 1 and %d depth layers", nlayers, ML_MAX_LAYERS);
+  for (int b = 0; b <= nlayers; ++b) {
+    const double e = edges[b];
+    if (isnan(e) || e < 0.0 || (isinf(e) && b != nlayers) || (b > 0 && !(e > edges[b - 1])))
+      return fail(ML_ERR_SHAPE, "layer edges must be strictly increasing values >= 0, only the last may be +inf; "
+                                "edges[%d] = %g", b, e);
+  }
+  if (nt < 0 || nz <= 0 || ncol < 0 || nt > INT32_MAX || nz > INT32_MAX) return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ncol=%lld", (long long)nt, (long long)nz, (long long)ncol);
+  if (int rcp = check_column_pressure(ncol)) return rcp;
+  ML_REQUIRE_ALIGNED(T, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(S, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(v_ref, elem_size(vref_dtype));
+  if (nt == 0 || ncol == 0) return ML_OK;
+  const i64 lvl = nz * ncol;
+  const i64 ts = t_bcast ? 0 : lvl, ss = s_bcast ? 0 : lvl;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int v_f32 = vref_dtype == ML_F32;
+
+  if (direct_only() == false &&
+      tma::local_eligible(dtype, T, S, t_bcast, s_bcast, rho_ref, v_ref, vref_dtype, nt, nz, ncol, eta, nullptr)) {
+    tls().last_path = ML_PATH_TMA;
+    return tma::launch_local_layers(eos, T, S, t_bcast, s_bcast, rho_ref, v_ref, vref_dtype, z_i, deptho, p_level,
+                                    neg_inv_rhozero, edges, nlayers, (int)nt, (int)nz, ncol, eta, st);
+  }
+  tls().last_path = ML_PATH_DIRECT;
+  LayerEdges L;
+  L.n = nlayers;
+  for (int b = 0; b <= ML_MAX_LAYERS; ++b) L.e[b] = b <= nlayers ? edges[b] : 0.0;
+  if (dtype == ML_F32) {
+    if (eos == ML_EOS_WRIGHT) return launch_layers_direct<float, 0>(T, S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, eta, L, st);
+    return launch_layers_direct<float, 1>(T, S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, eta, L, st);
+  }
+  if (eos == ML_EOS_WRIGHT) return launch_layers_direct<double, 0>(T, S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, eta, L, st);
+  return launch_layers_direct<double, 1>(T, S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, eta, L, st);
 }
 
 static int delta_rho_impl(int eos, int dtype, const void* T, const void* S, int t_bcast, int s_bcast,

@@ -25,6 +25,8 @@
 #include "ml_tma_dev.cuh"
 #include "ml_tma.cuh"
 
+#include <type_traits>
+
 namespace ml {
 namespace tma {
 
@@ -64,6 +66,7 @@ __host__ __device__ constexpr int ctas_per_sm_of(int mode) { return mode == 1 /*
 #ifndef ML_TMA_EXPERIMENT
 #define ML_TMA_EXPERIMENT 0
 #endif
+constexpr int kNoLayer = 0xffff;  // kLocalLayers: no layer touches the level
 
 
 struct Params {
@@ -88,6 +91,65 @@ struct Params {
   double* partials;       // kGlobal: [nt][tiles];  kSelfRef: [2][tiles] = {volo, masso}
 };
 
+// kLocalLayers: the depth layers, a kernel parameter of their own (the other modes take an empty one: a larger
+// Params cost the kLocal kernel four registers)
+struct LayerParams {
+  int nlayers;                      // eta is [nt][nlayers][ncol]
+  double edges[ML_MAX_LAYERS + 1];  // increasing; the last may be +inf
+};
+struct NoLayers {};
+__device__ __forceinline__ int layer_count(const LayerParams& L) { return L.nlayers; }
+__device__ __forceinline__ int layer_count(const NoLayers&) { return 0; }
+__device__ __forceinline__ double layer_edge(const LayerParams& L, int b) { return L.edges[b]; }
+__device__ __forceinline__ double layer_edge(const NoLayers&, int) { return 0.0; }
+// where a thread stores the heights of its column (kLocalLayers)
+struct LayerOut {
+  double* eta;
+  double coef;
+  int nt;
+  i64 ncol, c;
+  int t0;
+  bool in, surface_wet;
+};
+// weight of level z in layer b: derived.py:295-318 with top = edges[b], bottom = edges[b+1] (the arithmetic of
+// k_calc_dz); depth and z_i are never NaN here
+template <typename LP>
+__device__ __forceinline__ double layer_w(const LP& L, const double* s_zi, double depth, int z, int b) {
+  return fmin(fmax(s_zi[z + 1] - layer_edge(L, b), 0.0), level_dz(fmin(depth, layer_edge(L, b + 1)), s_zi[z], s_zi[z + 1]));
+}
+template <typename LP>
+__device__ __forceinline__ void store_height(const LayerOut& o, const LP& L, int b, int k, double a) {
+  if (o.in && o.t0 + k < o.nt) o.eta[((i64)(o.t0 + k) * layer_count(L) + b) * o.ncol + o.c] = o.surface_wet ? o.coef * a : nan("");
+}
+// the sweep has left layer b: store its sums and start the next layer from zero
+template <int TC, typename LP>
+__device__ __forceinline__ void close_layer(double (&acc)[TC], bool& poisoned, const LayerOut& o, const LP& L, int b) {
+#pragma unroll
+  for (int k = 0; k < TC; ++k) {
+    poisoned |= is_nan_q(acc[k]);
+    store_height(o, L, b, k, acc[k]);
+    acc[k] = 0.0;
+  }
+}
+// level z closes layers lo .. hi - 1 and opens hi (an edge falls inside it).  acc already holds layer lo with the
+// level's share of d = rho - rho_ref of step k added: store it, store the layers that lie inside the level, and
+// start layer hi with its share of d
+template <typename LP>
+__device__ __forceinline__ void split_level(double& acc, bool& poisoned, const LayerOut& o, const LP& L, const double* s_zi,
+                                            double depth, int z, int lo, int hi, bool live, int k, double d) {
+  poisoned |= is_nan_q(acc);
+  store_height(o, L, lo, k, acc);
+  for (int b = lo + 1; b < hi; ++b) {
+    const double a = (live ? layer_w(L, s_zi, depth, z, b) : 0.0) * d;
+    poisoned |= is_nan_q(a);
+    store_height(o, L, b, k, a);
+  }
+  acc = (live ? layer_w(L, s_zi, depth, z, hi) : 0.0) * d;
+}
+
+template <int MODE>
+using LayersOf = typename std::conditional<MODE == 3 /* kLocalLayers */, LayerParams, NoLayers>::type;
+
 // What a launch computes.
 //   kLocal   eta from rho - rho_ref with rho_ref read from memory          (steric.py:150-166)
 //   kGlobal  per-step sums of rho * v_ref                                    (steric.py:135)
@@ -95,7 +157,13 @@ struct Params {
 //            density of row 0 of every stage, evaluated here, stored for the caller and
 //            reduced into volo / masso on the way -- the reference-state pass
 //            (reference.py:71-80) costs no extra read of T, S.
-enum Mode { kLocal = 0, kGlobal = 1, kSelfRef = 2 };
+//   kLocalLayers  kLocal split by depth layer: level z feeds layer b with the weight
+//            calc_dz(top=edges[b], bottom=edges[b+1]) (derived.py:295-318) and the height of a layer is stored
+//            when the sweep leaves its last level.  One set of TC sums lives in registers: the layers a level
+//            touches are the same for every column (only the bottom clip varies, and it can only zero a weight),
+//            so they are worked out once per CTA, and a level feeds more than one layer only where an edge
+//            falls inside it.
+enum Mode { kLocal = 0, kGlobal = 1, kSelfRef = 2, kLocalLayers = 3 };
 
 // BC: 0 = T and S both [t][z][col]; 1 = T is [z][col] (halosteric); 2 = S is [z][col] (thermosteric)
 #ifdef ML_TMA_MAXNREG  // experiment builds: explicit register cap instead of the occupancy hint
@@ -106,9 +174,12 @@ enum Mode { kLocal = 0, kGlobal = 1, kSelfRef = 2 };
 
 template <typename TIn, int EOS, int TC, int BC, int MODE, bool FLAT>
 __global__ void ML_TMA_KERNEL_ATTR
-    k_steric_tma(const __grid_constant__ CUtensorMap mapT, const __grid_constant__ CUtensorMap mapS, const Params P) {
+    k_steric_tma(const __grid_constant__ CUtensorMap mapT, const __grid_constant__ CUtensorMap mapS, const Params P,
+                 const LayersOf<MODE> L) {
   constexpr bool GLOBAL = MODE == kGlobal;
   constexpr bool SELFREF = MODE == kSelfRef;
+  constexpr bool LAYERS = MODE == kLocalLayers;
+  constexpr bool READREF = MODE == kLocal || LAYERS;  // rho_ref is read from memory
   constexpr int kStages = stages_of(MODE, BC, (int)sizeof(TIn));
   constexpr int SORT = ML_TMA_SORT;
   constexpr int kRowsT = (BC == 1) ? 1 : TC;
@@ -135,6 +206,7 @@ __global__ void ML_TMA_KERNEL_ATTR
   double* s_zi = s_p + P.nz;                                 // [nz+1] interfaces (local modes)
   int* s_key = reinterpret_cast<int*>(s_zi + P.nz + 1);      // [kTile] wet levels per column (SORT)
   int* s_col = s_key + kTile;                                // [kTile] column handled by each thread (SORT)
+  int* s_lay = s_col + kTile;                                // [nz] kLocalLayers: layers touching the level
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   // The chunks of one tile are neighbours in launch order, so they are resident together and the
@@ -194,6 +266,20 @@ __global__ void ML_TMA_KERNEL_ATTR
   for (int i = threadIdx.x; i < P.nz; i += kThreads) s_p[i] = __ldg(P.p_level + i);
   if (!GLOBAL)
     for (int i = threadIdx.x; i <= P.nz; i += kThreads) s_zi[i] = __ldg(P.z_i + i);
+  if (LAYERS) {
+    // layer b touches level k iff z_i[k+1] > edges[b] && z_i[k] < edges[b+1]; the layers touching a level are
+    // consecutive: lo | hi << 8, or kNoLayer
+    for (int i = threadIdx.x; i < P.nz; i += kThreads) {
+      const double zt = __ldg(P.z_i + i), zb = __ldg(P.z_i + i + 1);
+      int lo = -1, hi = -1;
+      for (int b = 0; b < layer_count(L); ++b)
+        if (zb > layer_edge(L, b) && zt < layer_edge(L, b + 1)) {
+          if (lo < 0) lo = b;
+          hi = b;
+        }
+      s_lay[i] = lo < 0 ? kNoLayer : (lo | (hi << 8));
+    }
+  }
   __syncthreads();
 
   int col = tid;  // column of the tile this thread integrates
@@ -229,9 +315,15 @@ __global__ void ML_TMA_KERNEL_ATTR
     // per-level operands, fetched one level ahead (raw bits, see ld_vraw)
     double rref_n = 0.0;
     vbits v_n = ld_vraw(gV, cc);
-    if (MODE == kLocal) rref_n = __ldg(P.rho_ref + cc);
+    if (READREF) rref_n = __ldg(P.rho_ref + cc);
     const bool surface_wet = !vraw_isnan(v_n);  // steric.py:166
     const bool zero_first = MODE == kLocal && P.first_is_reference != 0 && t0 == 0;
+    // kLocalLayers: the layer the sums belong to, and whether a closed layer met a missing value
+    int cur = 0;
+    bool poisoned = false;
+    // (the layered steps are free functions, not lambdas: an unused closure that holds &acc cost the kSelfRef
+    // kernels four registers)
+    const LayerOut out = {P.eta, P.coef, P.nt, P.ncol, c, t0, in, surface_wet};
     // kSelfRef: the reference density of level z+1 is evaluated together with the points of
     // level z (from row 0 of the next stage, inside the same unrolled block so the scheduler
     // interleaves it), stored for the caller and used one iteration later.
@@ -248,7 +340,7 @@ __global__ void ML_TMA_KERNEL_ATTR
       if (z + 1 < nz) {
         const i64 j = (i64)(z + 1) * P.ncol + cc;
         v_n = ld_vraw(gV, j);
-        if (MODE == kLocal) rref_n = __ldg(P.rho_ref + j);
+        if (READREF) rref_n = __ldg(P.rho_ref + j);
       }
       // weight of this cell in the sum and the value subtracted from rho
       const bool dry = vraw_isnan(v_z);
@@ -260,7 +352,8 @@ __global__ void ML_TMA_KERNEL_ATTR
         w = level_dz(depth, s_zi[z], s_zi[z + 1]);
         // steric.py:151-153: delta_rho is NaN (and skipped) wherever the reference volume is missing
         sub = rref_z;
-        if (dry || (MODE == kLocal && isnan(rref_z))) w = 0.0;
+        if (dry || (READREF && isnan(rref_z))) w = 0.0;
+        if (LAYERS && s_lay[z] == kNoLayer) w = 0.0;  // no layer takes this level
         if (SELFREF && in && !dry) {  // volo, masso: skipna sums (derived.py:787-789, :435-438)
           const double v = vraw_value(v_z);
           vol += v;
@@ -271,6 +364,16 @@ __global__ void ML_TMA_KERNEL_ATTR
       eos.set_level(s_p[z]);
       const bool live = nonzero(w);
       if (!live) sub = 0.0;  // a dry lane adds 0 * (rho of a borrowed column - sub): keep a missing rho_ref out of it
+      // kLocalLayers: close the layers that ended above this level (in every warp, wet or not); `wl` is the weight
+      // of the level in its one layer, or -- where an edge falls inside the level (lo < hi) -- in layer lo
+      int lo = 0, hi = 0;
+      double wl = w;
+      if (LAYERS && s_lay[z] != kNoLayer) {
+        lo = s_lay[z] & 255;
+        hi = s_lay[z] >> 8;
+        for (; cur < lo; ++cur) close_layer<TC>(acc, poisoned, out, L, cur);
+        wl = live ? layer_w(L, s_zi, depth, z, lo) : 0.0;
+      }
       const unsigned live_lanes = __ballot_sync(0xffffffffu, live);
       // kSelfRef: row 0 of the NEXT level (clamped at the bottom level, where the value is
       // recomputed and discarded) -- wait for it up front so that the reference point and the
@@ -298,14 +401,26 @@ __global__ void ML_TMA_KERNEL_ATTR
         typename Eos<EOS>::Pinned pin = {};
         if (BC == 1) pin = eos.pin_t((double)sT[flat_off(z, 0, true)]);
         if (BC == 2) pin = eos.pin_s((double)sS[flat_off(z, 0, true)]);
+        double d[LAYERS ? TC : 1];  // kLocalLayers: rho - rho_ref of each step, for a level that closes layers
 #pragma unroll
         for (int kk = SELFREF ? 1 : 0; kk < TC; ++kk) {  // kSelfRef: step 0 is the reference itself
           if (MODE == kLocal && kk == 0 && zero_first) continue;  // ... and so it is here, by the caller's word
           const double Tv = (double)sT[(BC == 1 ? 0 : kk) * kPitch + flat_off(z, t0 + kk, BC == 1)];
           const double Sv = (double)sS[(BC == 2 ? 0 : kk) * kPitch + flat_off(z, t0 + kk, BC == 2)];
           const double rho = BC == 1 ? eos.rho_pinned_t(pin, Sv) : (BC == 2 ? eos.rho_pinned_s(pin, Tv) : eos.rho(Tv, Sv));
-          acc[kk] = fma(w, GLOBAL ? rho : rho - sub, acc[kk]);
+          // kLocalLayers: the sum of layer lo takes the kLocal kernel's FMA in the same straight-line block (where
+          // the compiler folds the subtraction of rho_ref into the EOS's last multiply), so one layer (0, inf) is
+          // bit-identical to ml_steric_local, and the TC evaluations stay free to interleave
+          acc[kk] = fma(LAYERS ? wl : w, GLOBAL ? rho : rho - sub, acc[kk]);
+          if (LAYERS) d[LAYERS ? kk : 0] = rho - sub;
         }
+        if (LAYERS && lo < hi)
+#pragma unroll
+          for (int kk = 0; kk < TC; ++kk) split_level(acc[kk], poisoned, out, L, s_zi, depth, z, lo, hi, live, kk, d[LAYERS ? kk : 0]);
+      } else if (LAYERS && lo < hi) {
+#pragma unroll
+        for (int kk = 0; kk < TC; ++kk)  // a warp without water still closes its layers
+          split_level(acc[kk], poisoned, out, L, s_zi, depth, z, lo, hi, live, kk, 0.0);
       } else if (SELFREF) {
         // a warp without water still owes rho_ref of the next level (reference.py:71 evaluates the
         // EOS everywhere); over land T, S are missing and so is the result -- no arithmetic needed
@@ -313,6 +428,7 @@ __global__ void ML_TMA_KERNEL_ATTR
         sub_n = nan("");
         if (__any_sync(0xffffffffu, !(isnan(tN) || isnan(sN)))) sub_n = eos.rho_at((double)tN, (double)sN, p_next);
       }
+      if (LAYERS && lo < hi) cur = hi;  // layers lo .. hi - 1 are stored; the sums now belong to layer hi
       if (SELFREF && in && z + 1 < nz && P.rho_ref_out) P.rho_ref_out[(i64)(z + 1) * P.ncol + c] = sub_n;
       __syncwarp();
       if (lane == 0) {
@@ -322,46 +438,58 @@ __global__ void ML_TMA_KERNEL_ATTR
           refill_stage(z + kStages);
       }
     }
+    if (LAYERS)
+      for (; cur < layer_count(L); ++cur) close_layer<TC>(acc, poisoned, out, L, cur);  // the last layer, and those wholly below the grid: 0
     // Repair pass (rare: consistent model output has no holes at wet cells).  xarray's sum skips a
     // missing term (steric.py:163, derived.py:435-438); the sweep above does not, so a column whose
-    // sums turned NaN is integrated again from global memory with the skipna rule.
-    bool poisoned = false;
+    // sums turned NaN is integrated again from global memory with the skipna rule.  kLocalLayers: every
+    // layer of the column is integrated again and overwritten.
 #pragma unroll
     for (int k = 0; k < TC; ++k) poisoned |= is_nan_q(acc[k]);
     if (poisoned && in) {
+      for (int b = 0; b < (LAYERS ? layer_count(L) : 1); ++b) {
 #pragma unroll
-      for (int k = 0; k < TC; ++k) acc[k] = 0.0;
-      const i64 lvl = (i64)nz * P.ncol;
-      for (int z = 0; z < nz; ++z) {
-        const i64 j = (i64)z * P.ncol + c;
-        const vbits v = ld_vraw(gV, j);
-        double w, sub = 0.0;
-        if (GLOBAL) {
-          w = vraw_isnan(v) ? 0.0 : vraw_value(v);
-        } else {
-          w = vraw_isnan(v) ? 0.0 : level_dz(depth, s_zi[z], s_zi[z + 1]);
-          if (!SELFREF) sub = __ldg(P.rho_ref + j);
-        }
-        if (!nonzero(w)) continue;
-        eos.set_level(s_p[z]);
-        if (SELFREF)  // the reference density again, from step 0 of this column (same arithmetic as in the sweep)
-          sub = eos.rho((double)__ldg(gT + j), (double)__ldg(gS + j));
-        // the same evaluation as the sweep (a pinned operand folded into the coefficients), so that a repaired
-        // column does not depend on how the time axis was cut into chunks
-        typename Eos<EOS>::Pinned pin = {};
-        if (BC == 1) pin = eos.pin_t((double)__ldg(gT + j));
-        if (BC == 2) pin = eos.pin_s((double)__ldg(gS + j));
+        for (int k = 0; k < TC; ++k) acc[k] = 0.0;
+        const i64 lvl = (i64)nz * P.ncol;
+        for (int z = 0; z < nz; ++z) {
+          const i64 j = (i64)z * P.ncol + c;
+          const vbits v = ld_vraw(gV, j);
+          double w, sub = 0.0;
+          if (GLOBAL) {
+            w = vraw_isnan(v) ? 0.0 : vraw_value(v);
+          } else if (LAYERS) {
+            const int lay = s_lay[z];
+            const bool touches = lay != kNoLayer && (lay & 255) <= b && b <= (lay >> 8);
+            w = (vraw_isnan(v) || !touches) ? 0.0 : layer_w(L, s_zi, depth, z, b);
+            sub = __ldg(P.rho_ref + j);
+          } else {
+            w = vraw_isnan(v) ? 0.0 : level_dz(depth, s_zi[z], s_zi[z + 1]);
+            if (!SELFREF) sub = __ldg(P.rho_ref + j);
+          }
+          if (!nonzero(w)) continue;
+          eos.set_level(s_p[z]);
+          if (SELFREF)  // the reference density again, from step 0 of this column (same arithmetic as in the sweep)
+            sub = eos.rho((double)__ldg(gT + j), (double)__ldg(gS + j));
+          // the same evaluation as the sweep (a pinned operand folded into the coefficients), so that a repaired
+          // column does not depend on how the time axis was cut into chunks
+          typename Eos<EOS>::Pinned pin = {};
+          if (BC == 1) pin = eos.pin_t((double)__ldg(gT + j));
+          if (BC == 2) pin = eos.pin_s((double)__ldg(gS + j));
 #pragma unroll
-        for (int k = SELFREF ? 1 : 0; k < TC; ++k) {
-          if (t0 + k >= P.nt || (k == 0 && zero_first)) continue;
-          const double Tv = (double)__ldg(gT + (BC == 1 ? 0 : (i64)(t0 + k) * lvl) + j);
-          const double Sv = (double)__ldg(gS + (BC == 2 ? 0 : (i64)(t0 + k) * lvl) + j);
-          const double rho = BC == 1 ? eos.rho_pinned_t(pin, Sv) : (BC == 2 ? eos.rho_pinned_s(pin, Tv) : eos.rho(Tv, Sv));
-          fma_skipnan(acc[k], w, GLOBAL ? rho : rho - sub);
+          for (int k = SELFREF ? 1 : 0; k < TC; ++k) {
+            if (t0 + k >= P.nt || (k == 0 && zero_first)) continue;
+            const double Tv = (double)__ldg(gT + (BC == 1 ? 0 : (i64)(t0 + k) * lvl) + j);
+            const double Sv = (double)__ldg(gS + (BC == 2 ? 0 : (i64)(t0 + k) * lvl) + j);
+            const double rho = BC == 1 ? eos.rho_pinned_t(pin, Sv) : (BC == 2 ? eos.rho_pinned_s(pin, Tv) : eos.rho(Tv, Sv));
+            fma_skipnan(acc[k], w, GLOBAL ? rho : rho - sub);
+          }
         }
+        if (LAYERS)
+#pragma unroll
+          for (int k = 0; k < TC; ++k) store_height(out, L, b, k, acc[k]);
       }
     }
-    if (!GLOBAL) {
+    if (!GLOBAL && !LAYERS) {
       if (in) {
 #pragma unroll
         for (int k = 0; k < TC; ++k)
@@ -435,12 +563,13 @@ template <int TC>
 inline size_t smem_bytes(int bc, int nz, int mode, int es) {
   const int kStages = stages_of(mode, bc, es);
   return (size_t)kStages * (size_t)((bc == 0 ? 2 * TC : TC + 1) * kTile * es) + 3 * kStages * sizeof(uint64_t) +
-         (size_t)kConsumerWarps * TC * sizeof(double) + (size_t)(2 * nz + 1) * sizeof(double) + 2 * kTile * sizeof(int) + 128;
+         (size_t)kConsumerWarps * TC * sizeof(double) + (size_t)(2 * nz + 1) * sizeof(double) + 2 * kTile * sizeof(int) + 128 +
+         (mode == kLocalLayers ? (size_t)nz * sizeof(int) : 0);
 }
 
 template <typename TIn, int EOS, int TC, int BC, int MODE, bool FLAT>
 static int launch_one(const CUtensorMap& mT, const CUtensorMap& mS, const Params& P, unsigned tiles, unsigned chunks,
-                      cudaStream_t st) {
+                      cudaStream_t st, const LayerParams* lp) {
   auto kern = k_steric_tma<TIn, EOS, TC, BC, MODE, FLAT>;
   const size_t smem = smem_bytes<TC>(BC, P.nz, MODE, (int)sizeof(TIn));
   // opt in to > 48 KB of dynamic shared memory; the attribute is per device and per context, so it
@@ -450,20 +579,22 @@ static int launch_one(const CUtensorMap& mT, const CUtensorMap& mS, const Params
   Params Q = P;
   Q.tiles = tiles;
   Q.nchunks = chunks;
-  kern<<<tiles * chunks, kThreads, smem, st>>>(mT, mS, Q);
+  LayersOf<MODE> L{};
+  if constexpr (MODE == kLocalLayers) L = *lp;
+  kern<<<tiles * chunks, kThreads, smem, st>>>(mT, mS, Q, L);
   return launched("k_steric_tma");
 }
 
 template <typename TIn, int EOS, int TC, int MODE, bool FLAT>
 static int launch_bc(int bc, const CUtensorMap& mT, const CUtensorMap& mS, const Params& P, unsigned tiles,
-                     unsigned chunks, cudaStream_t st) {
+                     unsigned chunks, cudaStream_t st, const LayerParams* lp) {
 #ifdef ML_TMA_FAST_BUILD  // experiment builds: only the fp32 / Wright / 12-step / no-broadcast kernels
   if (sizeof(TIn) != 4 || EOS != 0 || TC != 12 || bc != 0) return fail(ML_ERR_MODE, "kernel not instantiated in a fast build");
-  return launch_one<float, 0, 12, 0, MODE, FLAT>(mT, mS, P, tiles, chunks, st);
+  return launch_one<float, 0, 12, 0, MODE, FLAT>(mT, mS, P, tiles, chunks, st, lp);
 #else
-  if (bc == 0) return launch_one<TIn, EOS, TC, 0, MODE, FLAT>(mT, mS, P, tiles, chunks, st);
-  if (bc == 1) return launch_one<TIn, EOS, TC, 1, MODE, FLAT>(mT, mS, P, tiles, chunks, st);
-  return launch_one<TIn, EOS, TC, 2, MODE, FLAT>(mT, mS, P, tiles, chunks, st);
+  if (bc == 0) return launch_one<TIn, EOS, TC, 0, MODE, FLAT>(mT, mS, P, tiles, chunks, st, lp);
+  if (bc == 1) return launch_one<TIn, EOS, TC, 1, MODE, FLAT>(mT, mS, P, tiles, chunks, st, lp);
+  return launch_one<TIn, EOS, TC, 2, MODE, FLAT>(mT, mS, P, tiles, chunks, st, lp);
 #endif
 }
 
@@ -528,9 +659,9 @@ static int make_plan(Plan* pl, const void* T, const void* S, int t_bcast, int s_
 }
 
 template <int MODE, bool FLAT>
-static int launch_segment(int eos, const Plan& pl, const Segment& g, Params P, cudaStream_t st) {
+static int launch_segment(int eos, const Plan& pl, const Segment& g, Params P, cudaStream_t st, const LayerParams* lp) {
   P.t_start = g.t_start;
-#define ML_TMA_GO(TIN, E, TCV) return launch_bc<TIN, E, TCV, MODE, FLAT>(pl.bc, g.mT, g.mS, P, pl.tiles, g.chunks, st)
+#define ML_TMA_GO(TIN, E, TCV) return launch_bc<TIN, E, TCV, MODE, FLAT>(pl.bc, g.mT, g.mS, P, pl.tiles, g.chunks, st, lp)
   if (P.es == 8) {  // fields stored as fp64
 #ifndef ML_TMA_FAST_BUILD
     if (eos == ML_EOS_WRIGHT) {
@@ -558,20 +689,24 @@ static int launch_segment(int eos, const Plan& pl, const Segment& g, Params P, c
 // translation unit (ml_tma_flat.cu includes this file with ML_TMA_FLAT_TU defined): a second set of instantiations
 // next to these would double the compile time of this file, and a run-time switch inside one kernel cost the
 // headline kernel a spill in its level loop.
-int launch_segment_flat(int mode, int eos, const Plan& pl, const Segment& g, const Params& P, cudaStream_t st);
+int launch_segment_flat(int mode, int eos, const Plan& pl, const Segment& g, const Params& P, cudaStream_t st,
+                        const LayerParams* lp);
 
 #ifdef ML_TMA_FLAT_TU
-int launch_segment_flat(int mode, int eos, const Plan& pl, const Segment& g, const Params& P, cudaStream_t st) {
-  if (mode == kLocal) return launch_segment<kLocal, true>(eos, pl, g, P, st);
-  if (mode == kGlobal) return launch_segment<kGlobal, true>(eos, pl, g, P, st);
-  return launch_segment<kSelfRef, true>(eos, pl, g, P, st);
+int launch_segment_flat(int mode, int eos, const Plan& pl, const Segment& g, const Params& P, cudaStream_t st,
+                        const LayerParams* lp) {
+  if (mode == kLocal) return launch_segment<kLocal, true>(eos, pl, g, P, st, lp);
+  if (mode == kLocalLayers) return launch_segment<kLocalLayers, true>(eos, pl, g, P, st, lp);
+  if (mode == kGlobal) return launch_segment<kGlobal, true>(eos, pl, g, P, st, lp);
+  return launch_segment<kSelfRef, true>(eos, pl, g, P, st, lp);
 }
 #else
 
 template <int MODE>
-static int launch_plan(int eos, const Plan& pl, const Params& P, cudaStream_t st) {
+static int launch_plan(int eos, const Plan& pl, const Params& P, cudaStream_t st, const LayerParams* lp = nullptr) {
   for (int i = 0; i < pl.nseg; ++i) {
-    int rc = P.flat ? launch_segment_flat(MODE, eos, pl, pl.seg[i], P, st) : launch_segment<MODE, false>(eos, pl, pl.seg[i], P, st);
+    int rc = P.flat ? launch_segment_flat(MODE, eos, pl, pl.seg[i], P, st, lp)
+                    : launch_segment<MODE, false>(eos, pl, pl.seg[i], P, st, lp);
     if (rc) return rc;
   }
   return ML_OK;
@@ -618,6 +753,25 @@ int launch_local(int eos, int, const void* T, const void* S, int t_bcast, int s_
   int rc = make_plan(&pl, T, S, t_bcast, s_bcast, P, 0);
   if (rc) return rc;
   return launch_plan<kLocal>(eos, pl, P, st);
+}
+
+int launch_local_layers(int eos, const void* T, const void* S, int t_bcast, int s_bcast, const double* rho_ref,
+                        const void* v_ref, int vref_dtype, const double* z_i, const double* deptho, const double* p_level,
+                        double coef, const double* edges, int nlayers, int nt, int nz, int64_t ncol, double* eta,
+                        cudaStream_t st) {
+  Params P = base_params(T, S, v_ref, vref_dtype, p_level, nt, nz, ncol);
+  P.rho_ref = rho_ref;
+  P.z_i = z_i;
+  P.deptho = deptho;
+  P.coef = coef;
+  P.eta = eta;
+  LayerParams lp;
+  lp.nlayers = nlayers;
+  for (int b = 0; b <= ML_MAX_LAYERS; ++b) lp.edges[b] = b <= nlayers ? edges[b] : 0.0;
+  Plan pl;
+  int rc = make_plan(&pl, T, S, t_bcast, s_bcast, P, 0);
+  if (rc) return rc;
+  return launch_plan<kLocalLayers>(eos, pl, P, st, &lp);
 }
 
 int launch_selfref(int eos, const void* T, const void* S, int t_bcast, int s_bcast, const void* v_ref, int vref_dtype,

@@ -14,6 +14,13 @@ int launch_local(int eos, int dtype, const void* T, const void* S, int t_bcast, 
                  double coef, int nt, int nz, int64_t ncol, double* eta, double* delta_rho, cudaStream_t st,
                  int first_is_reference = 0);  // step 0 of the fields is the reference state: its height is exactly 0
 
+// kLocalLayers: launch_local split by depth layer, eta [nt][nlayers][ncol]; edges (host) as ml_steric_local_layers,
+// eligibility is local_eligible without delta_rho
+int launch_local_layers(int eos, const void* T, const void* S, int t_bcast, int s_bcast, const double* rho_ref,
+                        const void* v_ref, int vref_dtype, const double* z_i, const double* deptho, const double* p_level,
+                        double coef, const double* edges, int nlayers, int nt, int nz, int64_t ncol, double* eta,
+                        cudaStream_t st);
+
 // kSelfRef: reference state (rho_ref, volo, masso) and eta from one pass; reference = step 0
 int launch_selfref(int eos, const void* T, const void* S, int t_bcast, int s_bcast, const void* v_ref, int vref_dtype,
                    const double* z_i, const double* deptho, const double* p_level, double coef, int nt, int nz,

@@ -17,7 +17,7 @@ from .labeled import ChunkedArray, DataArray, Dataset
 from .reference import _pressure, setup_reference_state
 from .util import annual_average, calendar_axis, default_coords, validate_dataset, whole_years_in_order
 
-__all__ = ["halosteric", "steric", "steric_variants", "thermosteric"]
+__all__ = ["halosteric", "steric", "steric_layers", "steric_variants", "thermosteric"]
 
 
 def steric(
@@ -774,6 +774,95 @@ def _local_variants(dset, reference, tcoord, zcoord, zbounds, rhozero, patm, eos
     for variant in VARIANTS:
         result[variant] = DataArray(etas[variant], (tcoord,) + full.dims[2:])
     return result, reference
+
+
+def steric_layers(dset, depth_edges=(0.0, 700.0, 2000.0, None), reference=None, coord_names=None, varname_map=None,
+                  rhozero=1035.0, patm=101325.0, equation_of_state="Wright", variant="steric", dtype="float32",
+                  strict=True, annual=False, days_in_month=None, verbose=False):
+    """Local steric, thermosteric or halosteric sea level change split by depth layer (0-700 m, 700-2000 m and
+    2000 m to the sea floor by default), from one pass over T and S.
+
+    Layer ``b`` is the local height of :func:`steric` with ``calc_dz(top=depth_edges[b], bottom=depth_edges[b+1])``
+    (derived.py:249-325) as the cell thickness; ``None`` as the last edge means "to the sea floor".  A layer wholly
+    below a wet column's floor is 0.0; a column whose surface is dry is NaN in every layer.  Like ``calc_dz``, a
+    partial bottom cell that straddles an inner edge counts in full towards the layer above the edge, so there the
+    layers add up to more than the full-column height.  The remaining arguments are those of :func:`steric` with
+    ``domain="local"``; ``reference=None`` builds the reference state from the first step first.
+
+    Returns ``(result, reference)``: ``result[variant]`` has dims ``(time, depth_layer, y, x)``, ``result["layer_top"]``
+    and ``result["layer_bottom"]`` are ``(depth_layer,)`` (``inf``: the sea floor).  There is no ``delta_rho``:
+    it is the field :func:`steric` returns.
+    """
+    edges = core.layer_edges(depth_edges)
+    xarray_in = type(dset).__module__.startswith("xarray")
+    if xarray_in:
+        from . import xarray_io
+
+        dset_x = dset
+        t_, z_, zb_ = default_coords(coord_names)
+        needed = {"thetao", "so", "volcello", "areacello", "deptho", t_, z_, zb_}
+        needed |= {k for k, v in (varname_map or {}).items() if v in needed}
+        dset = xarray_io.from_xarray(dset, names=sorted(needed))
+        if reference is not None:
+            assert type(reference).__module__.startswith("xarray"), "`reference` must be an xarray Dataset"
+            reference = xarray_io.from_xarray(reference)
+
+    # steric.py:84-91
+    dset = dset.rename(varname_map)
+    tcoord, zcoord, zbounds = default_coords(coord_names)
+    if _chunked(dset):
+        raise NotImplementedError("steric_layers takes device-resident or in-memory fields; chunked (dask-backed) "
+                                  "fields are not supported yet")
+    validate_dataset(dset, strict=strict, additional_vars=[zbounds, "deptho"])
+    pres = _pressure(dset, zcoord, patm)  # steric.py:96
+
+    # steric.py:98-112
+    if reference is not None:
+        assert isinstance(reference, Dataset), "`reference` must be an xarray Dataset"
+        if verbose:
+            print("Using supplied reference state")
+    else:
+        reference = setup_reference_state(dset, patm=patm, eos=equation_of_state, coord_names=coord_names)
+        if verbose:
+            print("Generating reference state from first timestep")
+    validate_dataset(reference, reference=True, strict=strict)
+
+    # steric.py:115-125
+    if variant == "thermosteric":
+        thetao, so, t_bcast, s_bcast = dset["thetao"], reference["so"], False, True
+    elif variant == "halosteric":
+        thetao, so, t_bcast, s_bcast = reference["thetao"], dset["so"], True, False
+    elif variant == "steric":
+        thetao, so, t_bcast, s_bcast = dset["thetao"], dset["so"], False, False
+    else:
+        raise ValueError(f"Unknown variant '{variant}' passed to `steric`")
+    full = dset["so"] if t_bcast else dset["thetao"]
+    if full.dims[0] != tcoord or full.dims[1] != zcoord:
+        raise ValueError(f"expecting fields laid out ({tcoord}, {zcoord}, y, x), got {full.dims}")
+
+    _check_depths(dset, zcoord, zbounds)
+    eta = core.steric_local_layers(thetao.data, so.data, reference["rho"].data, reference["volcello"].data,
+                                   dset[zbounds].data, dset["deptho"].data, pres, edges, rhozero=rhozero,
+                                   eos=equation_of_state, t_bcast=t_bcast, s_bcast=s_bcast)
+    result = Dataset()
+    # steric.py:169-179, plus the edges
+    result[variant] = DataArray(eta, (tcoord, "depth_layer") + full.dims[2:], attrs={
+        "long_name": f"{variant.capitalize()} height adjustment", "units": "m", "depth_edges": [float(e) for e in edges]})
+    result[variant].encoding["dtype"] = dtype
+    result["layer_top"] = DataArray(edges[:-1].copy(), ("depth_layer",), attrs={
+        "long_name": "Top of depth layer", "units": "m"})
+    result["layer_bottom"] = DataArray(edges[1:].copy(), ("depth_layer",), attrs={
+        "long_name": "Bottom of depth layer (inf: the sea floor)", "units": "m"})
+    for var in set(result.dims):
+        if var in dset.variables:
+            coord = dset[var].copy(deep=False)
+            coord.attrs = dict(dset[var].attrs)
+            result[var] = coord
+    if annual:  # steric.py:181-182
+        result = annual_average(result, tcoord=tcoord, days_in_month=days_in_month)
+    if xarray_in:
+        return xarray_io.to_xarray(result, like=dset_x), xarray_io.to_xarray(reference, like=dset_x)
+    return (result, reference)
 
 
 def halosteric(*args, **kwargs):
