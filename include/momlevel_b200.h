@@ -76,7 +76,7 @@ int ml_last_path(void);
 /* number of kernels this library has launched from the calling thread (monotonic) */
 int64_t ml_launch_count(void);
 /* force ML_PATH_DIRECT (1) / allow ML_PATH_TMA (0) for this thread; 2 = TMA family without the one-pass
- * three-height kernel of ml_steric_local_variants (A/B); returns previous */
+ * three-height kernels of the *_variants entry points (A/B); returns previous */
 int ml_set_force_direct(int on);
 /* Per-column pressure offset for this thread's next calls, until cleared with (NULL, 0): `patm` given as a 2-D
  * field instead of a scalar (src/momlevel/steric.py:96 and reference.py:54 broadcast `z_l * 1e4 + patm` by
@@ -247,6 +247,30 @@ int ml_steric_local_layers(int eos, int dtype, const void* T, const void* S, int
                            const double* deptho, const double* p_level, double neg_inv_rhozero,
                            const double* edges, int nlayers, int64_t nt, int64_t nz, int64_t ncol,
                            double* eta, void* stream);
+
+/* ---------------------------------------------------------------------------------------
+ * ml_steric_local_layers_variants -- the steric, thermosteric and halosteric heights of
+ * ml_steric_local_variants split by depth layer as ml_steric_local_layers, in one call: how much of a
+ * layer's change is warming and how much is freshening.
+ * Fields that suit the one-pass kernel of ml_steric_local_variants (fp32, 16-byte aligned, ncol % 4 == 0,
+ * ncol >= 256) take ONE pass over T and S for all the heights asked for (csrc/ml_tma3.cu), each bit-identical
+ * to its ml_steric_local_layers launch; anything else, a column pressure (ml_set_column_pressure) or a call
+ * that asks for one height only runs one ml_steric_local_layers per height.  ml_set_force_direct(2) turns
+ * the one-pass kernel off (A/B).
+ *   T, S          [nt][nz][ncol] of `dtype`
+ *   T_ref, S_ref  [nz][ncol] of `dtype`: reference["thetao"], reference["so"]
+ *   rho_ref       [nz][ncol] fp64: reference["rho"] (ml_reference_state or a supplied reference); required
+ *   edges         HOST pointer, nlayers as ml_steric_local_layers (ML_ERR_SHAPE otherwise)
+ *   eta_*         [nt][nlayers][ncol] fp64 out each; a NULL pointer skips that variant; at least one is
+ *                 required (ML_ERR_NULL)
+ * Other arguments as ml_steric_local_layers; reads the thread's column pressure like it.
+ * ------------------------------------------------------------------------------------- */
+int ml_steric_local_layers_variants(int eos, int dtype, const void* T, const void* S, const void* T_ref,
+                                    const void* S_ref, const double* rho_ref, const void* v_ref,
+                                    int vref_dtype, const double* z_i, const double* deptho,
+                                    const double* p_level, double neg_inv_rhozero, const double* edges,
+                                    int nlayers, int64_t nt, int64_t nz, int64_t ncol, double* eta_steric,
+                                    double* eta_thermosteric, double* eta_halosteric, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * ml_steric_global -- fused EOS -> sum_{z,col} rho * v_ref per time step.

@@ -40,6 +40,8 @@ EXPORTS = {
     "ml_steric_local": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _d, _i64, _i64, _i64, _vp, _vp, _vp]),
     "ml_steric_local_layers": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _d, _vp, _i, _i64, _i64, _i64, _vp,
                                     _vp]),
+    "ml_steric_local_layers_variants": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _d, _vp, _i, _i64,
+                                             _i64, _i64, _vp, _vp, _vp, _vp]),
     "ml_delta_rho": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_delta_rho_annual": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_steric_local_selfref": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _d, _i64, _i64, _i64, _vp, _vp, _vp,

@@ -23,6 +23,7 @@ __all__ = [
     "steric_local",
     "steric_local_selfref",
     "steric_local_layers",
+    "steric_local_layers_variants",
     "layer_edges",
     "delta_rho",
     "steric_global",
@@ -464,6 +465,58 @@ def steric_local_layers(T, S, rho_ref, v_ref, z_i, deptho, p_level, edges, rhoze
     return eta
 
 
+VARIANTS = ("steric", "thermosteric", "halosteric")
+
+
+def variant_names(variants):
+    """``variants`` as a tuple of distinct names from :data:`VARIANTS`; ``ValueError`` for an empty sequence, a
+    duplicate or an unknown name."""
+    names = (variants,) if isinstance(variants, str) else tuple(variants)
+    unknown = [v for v in names if v not in VARIANTS]
+    if unknown:
+        raise ValueError(f"Unknown variants {unknown}: expected names from {VARIANTS}")
+    if not names:
+        raise ValueError("at least one variant is required")
+    if len(set(names)) != len(names):
+        raise ValueError(f"variants must be distinct, got {list(names)}")
+    return names
+
+
+def steric_local_layers_variants(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho, p_level, edges, rhozero=1035.0,
+                                 eos="Wright", variants=VARIANTS):
+    """:func:`steric_local_layers` for the steric, thermosteric and halosteric heights (steric.py:115-121) in one call.
+
+    ``T_ref, S_ref, rho_ref`` are the reference state (``reference["thetao"]``, ``["so"]``, ``["rho"]``); ``variants``
+    may name a subset.  Returns ``{variant: eta [nt, nlayers, ...]}`` fp64 on the device, from one pass over T and S
+    when the fields suit it (``ml_steric_local_layers_variants``).
+    """
+    L = _lib.lib()
+    names = variant_names(variants)
+    e = layer_edges(edges)
+    p_level, _pcol = _pressure_parts(p_level)
+    T, S, nt, nz, ncol, hshape = _steric_operands(T, S, False, False)
+    Tr, Sr = to_device(T_ref), to_device(S_ref)
+    dt = _field_dtype(T, S, Tr, Sr)
+    T, S, Tr, Sr = T.to(dt), S.to(dt), Tr.to(dt), Sr.to(dt)
+    rho_ref = _f64(rho_ref)
+    v_ref = to_device(v_ref)
+    z_i, depth, p = _f64(z_i), _f64(deptho), _f64(p_level)
+    assert Tr.numel() == nz * ncol and Sr.numel() == nz * ncol and rho_ref.numel() == nz * ncol
+    assert v_ref.numel() == nz * ncol and depth.numel() == ncol and z_i.numel() == nz + 1 and p.numel() == nz
+    nl = e.size - 1
+    eta = {v: torch.empty((nt, nl) + hshape, dtype=torch.float64, device=T.device) for v in names}
+    ptr = lambda v: eta[v].data_ptr() if v in eta else None  # noqa: E731
+    with _pcol:
+        _lib.check(
+            L.ml_steric_local_layers_variants(_eos_id(eos), _dt_id(T), T.data_ptr(), S.data_ptr(), Tr.data_ptr(),
+                                              Sr.data_ptr(), rho_ref.data_ptr(), v_ref.data_ptr(), _dt_id(v_ref),
+                                              z_i.data_ptr(), depth.data_ptr(), p.data_ptr(), -1.0 / rhozero,
+                                              e.ctypes.data_as(ctypes.c_void_p), nl, nt, nz, ncol, ptr("steric"),
+                                              ptr("thermosteric"), ptr("halosteric"), _stream())
+        )
+    return eta
+
+
 def delta_rho(T, S, rho_ref, v_ref, p_level, eos="Wright", t_bcast=False, s_bcast=False):
     """``where(v_ref.notnull(), rho - rho_ref, nan)`` time-first (steric.py:151-158), fp64 on the device."""
     L = _lib.lib()
@@ -624,7 +677,7 @@ def steric_global(T, S, v_ref, p_level, eos="Wright", t_bcast=False, s_bcast=Fal
     return masso
 
 
-GLOBAL_VARIANTS = ("steric", "thermosteric", "halosteric")
+GLOBAL_VARIANTS = VARIANTS
 
 
 def steric_global_variants(T, S, v_ref, p_level, T_ref=None, S_ref=None, eos="Wright", variants=GLOBAL_VARIANTS):

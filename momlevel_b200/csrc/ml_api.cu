@@ -598,6 +598,20 @@ int reduce_rows(const double* partials, int64_t nblk, double* out, int nrows, cu
 
 using namespace ml;
 
+// depth layers of the layered entry points: 1 <= nlayers <= ML_MAX_LAYERS, edges strictly increasing values >= 0, only
+// the last may be +inf
+static int check_layers(const double* edges, int nlayers) {
+  if (nlayers < 1 || nlayers > ML_MAX_LAYERS)
+    return fail(ML_ERR_SHAPE, "nlayers=%d: between 1 and %d depth layers", nlayers, ML_MAX_LAYERS);
+  for (int b = 0; b <= nlayers; ++b) {
+    const double e = edges[b];
+    if (isnan(e) || e < 0.0 || (isinf(e) && b != nlayers) || (b > 0 && !(e > edges[b - 1])))
+      return fail(ML_ERR_SHAPE, "layer edges must be strictly increasing values >= 0, only the last may be +inf; "
+                                "edges[%d] = %g", b, e);
+  }
+  return ML_OK;
+}
+
 extern "C" {
 
 int ml_version(void) { return ML_ABI_VERSION; }
@@ -892,14 +906,7 @@ int ml_steric_local_layers(int eos, int dtype, const void* T, const void* S, int
   ML_REQUIRE_PTR(p_level);
   ML_REQUIRE_PTR(edges);
   ML_REQUIRE_PTR(eta);
-  if (nlayers < 1 || nlayers > ML_MAX_LAYERS)
-    return fail(ML_ERR_SHAPE, "nlayers=%d: between 1 and %d depth layers", nlayers, ML_MAX_LAYERS);
-  for (int b = 0; b <= nlayers; ++b) {
-    const double e = edges[b];
-    if (isnan(e) || e < 0.0 || (isinf(e) && b != nlayers) || (b > 0 && !(e > edges[b - 1])))
-      return fail(ML_ERR_SHAPE, "layer edges must be strictly increasing values >= 0, only the last may be +inf; "
-                                "edges[%d] = %g", b, e);
-  }
+  if ((rc = check_layers(edges, nlayers))) return rc;
   if (nt < 0 || nz <= 0 || ncol < 0 || nt > INT32_MAX || nz > INT32_MAX) return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ncol=%lld", (long long)nt, (long long)nz, (long long)ncol);
   if (int rcp = check_column_pressure(ncol)) return rcp;
   ML_REQUIRE_ALIGNED(T, elem_size(dtype));
@@ -927,6 +934,62 @@ int ml_steric_local_layers(int eos, int dtype, const void* T, const void* S, int
   }
   if (eos == ML_EOS_WRIGHT) return launch_layers_direct<double, 0>(T, S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, eta, L, st);
   return launch_layers_direct<double, 1>(T, S, ts, ss, rho_ref, v_ref, v_f32, z_i, deptho, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, eta, L, st);
+}
+
+int ml_steric_local_layers_variants(int eos, int dtype, const void* T, const void* S, const void* T_ref,
+                                    const void* S_ref, const double* rho_ref, const void* v_ref, int vref_dtype,
+                                    const double* z_i, const double* deptho, const double* p_level,
+                                    double neg_inv_rhozero, const double* edges, int nlayers, int64_t nt, int64_t nz,
+                                    int64_t ncol, double* eta_steric, double* eta_thermosteric,
+                                    double* eta_halosteric, void* stream) {
+  int rc = check_common(eos, dtype);
+  if (rc) return rc;
+  if (vref_dtype != ML_F32 && vref_dtype != ML_F64) return fail(ML_ERR_DTYPE, "unknown vref dtype id %d", vref_dtype);
+  ML_REQUIRE_PTR(T);
+  ML_REQUIRE_PTR(S);
+  ML_REQUIRE_PTR(T_ref);
+  ML_REQUIRE_PTR(S_ref);
+  ML_REQUIRE_PTR(rho_ref);
+  ML_REQUIRE_PTR(v_ref);
+  ML_REQUIRE_PTR(z_i);
+  ML_REQUIRE_PTR(deptho);
+  ML_REQUIRE_PTR(p_level);
+  ML_REQUIRE_PTR(edges);
+  const int wanted = (eta_steric != nullptr) + (eta_thermosteric != nullptr) + (eta_halosteric != nullptr);
+  if (wanted == 0) return fail(ML_ERR_NULL, "eta_steric, eta_thermosteric and eta_halosteric are all NULL");
+  if ((rc = check_layers(edges, nlayers))) return rc;
+  if (nt < 0 || nz <= 0 || ncol < 0 || nt > INT32_MAX || nz > INT32_MAX) return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ncol=%lld", (long long)nt, (long long)nz, (long long)ncol);
+  if (int rcp = check_column_pressure(ncol)) return rcp;
+  ML_REQUIRE_ALIGNED(T, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(S, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(T_ref, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(S_ref, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(v_ref, elem_size(vref_dtype));
+  if (nt == 0 || ncol == 0) return ML_OK;
+  // One pass over T and S for all the layered heights asked for (csrc/ml_tma3.cu, kLocalLayers3), on the fields the
+  // one-pass kernel of ml_steric_local_variants takes and when more than one height is wanted.
+  if (tls().force_direct == 0 && !direct_only() && wanted >= 2 &&
+      tma::variants_eligible(dtype, T, S, T_ref, S_ref, vref_dtype, nt, nz, ncol)) {
+    tls().last_path = ML_PATH_TMA;
+    return tma::launch_local_layers_variants(eos, T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho, p_level,
+                                             neg_inv_rhozero, edges, nlayers, (int)nt, (int)nz, ncol, eta_steric,
+                                             eta_thermosteric, eta_halosteric, (cudaStream_t)stream);
+  }
+  // one ml_steric_local_layers per wanted height; steric.py:115-121: thermosteric holds S at the reference slab,
+  // halosteric holds T
+  struct Variant {
+    double* eta;
+    const void *T, *S;
+    int t_bcast, s_bcast;
+  };
+  const Variant todo[3] = {{eta_steric, T, S, 0, 0}, {eta_thermosteric, T, S_ref, 0, 1}, {eta_halosteric, T_ref, S, 1, 0}};
+  for (const Variant& v : todo) {
+    if (v.eta == nullptr) continue;
+    if ((rc = ml_steric_local_layers(eos, dtype, v.T, v.S, v.t_bcast, v.s_bcast, rho_ref, v_ref, vref_dtype, z_i, deptho,
+                                     p_level, neg_inv_rhozero, edges, nlayers, nt, nz, ncol, v.eta, stream)))
+      return rc;
+  }
+  return ML_OK;
 }
 
 static int delta_rho_impl(int eos, int dtype, const void* T, const void* S, int t_bcast, int s_bcast,

@@ -66,8 +66,6 @@ __host__ __device__ constexpr int ctas_per_sm_of(int mode) { return mode == 1 /*
 #ifndef ML_TMA_EXPERIMENT
 #define ML_TMA_EXPERIMENT 0
 #endif
-constexpr int kNoLayer = 0xffff;  // kLocalLayers: no layer touches the level
-
 
 struct Params {
   const void* T;          // the fields themselves (the streaming path goes through the tensor maps;
@@ -90,62 +88,6 @@ struct Params {
   double* eta;            // local modes: [nt][ncol]
   double* partials;       // kGlobal: [nt][tiles];  kSelfRef: [2][tiles] = {volo, masso}
 };
-
-// kLocalLayers: the depth layers, a kernel parameter of their own (the other modes take an empty one: a larger
-// Params cost the kLocal kernel four registers)
-struct LayerParams {
-  int nlayers;                      // eta is [nt][nlayers][ncol]
-  double edges[ML_MAX_LAYERS + 1];  // increasing; the last may be +inf
-};
-struct NoLayers {};
-__device__ __forceinline__ int layer_count(const LayerParams& L) { return L.nlayers; }
-__device__ __forceinline__ int layer_count(const NoLayers&) { return 0; }
-__device__ __forceinline__ double layer_edge(const LayerParams& L, int b) { return L.edges[b]; }
-__device__ __forceinline__ double layer_edge(const NoLayers&, int) { return 0.0; }
-// where a thread stores the heights of its column (kLocalLayers)
-struct LayerOut {
-  double* eta;
-  double coef;
-  int nt;
-  i64 ncol, c;
-  int t0;
-  bool in, surface_wet;
-};
-// weight of level z in layer b: derived.py:295-318 with top = edges[b], bottom = edges[b+1] (the arithmetic of
-// k_calc_dz); depth and z_i are never NaN here
-template <typename LP>
-__device__ __forceinline__ double layer_w(const LP& L, const double* s_zi, double depth, int z, int b) {
-  return fmin(fmax(s_zi[z + 1] - layer_edge(L, b), 0.0), level_dz(fmin(depth, layer_edge(L, b + 1)), s_zi[z], s_zi[z + 1]));
-}
-template <typename LP>
-__device__ __forceinline__ void store_height(const LayerOut& o, const LP& L, int b, int k, double a) {
-  if (o.in && o.t0 + k < o.nt) o.eta[((i64)(o.t0 + k) * layer_count(L) + b) * o.ncol + o.c] = o.surface_wet ? o.coef * a : nan("");
-}
-// the sweep has left layer b: store its sums and start the next layer from zero
-template <int TC, typename LP>
-__device__ __forceinline__ void close_layer(double (&acc)[TC], bool& poisoned, const LayerOut& o, const LP& L, int b) {
-#pragma unroll
-  for (int k = 0; k < TC; ++k) {
-    poisoned |= is_nan_q(acc[k]);
-    store_height(o, L, b, k, acc[k]);
-    acc[k] = 0.0;
-  }
-}
-// level z closes layers lo .. hi - 1 and opens hi (an edge falls inside it).  acc already holds layer lo with the
-// level's share of d = rho - rho_ref of step k added: store it, store the layers that lie inside the level, and
-// start layer hi with its share of d
-template <typename LP>
-__device__ __forceinline__ void split_level(double& acc, bool& poisoned, const LayerOut& o, const LP& L, const double* s_zi,
-                                            double depth, int z, int lo, int hi, bool live, int k, double d) {
-  poisoned |= is_nan_q(acc);
-  store_height(o, L, lo, k, acc);
-  for (int b = lo + 1; b < hi; ++b) {
-    const double a = (live ? layer_w(L, s_zi, depth, z, b) : 0.0) * d;
-    poisoned |= is_nan_q(a);
-    store_height(o, L, b, k, a);
-  }
-  acc = (live ? layer_w(L, s_zi, depth, z, hi) : 0.0) * d;
-}
 
 template <int MODE>
 using LayersOf = typename std::conditional<MODE == 3 /* kLocalLayers */, LayerParams, NoLayers>::type;
@@ -266,20 +208,7 @@ __global__ void ML_TMA_KERNEL_ATTR
   for (int i = threadIdx.x; i < P.nz; i += kThreads) s_p[i] = __ldg(P.p_level + i);
   if (!GLOBAL)
     for (int i = threadIdx.x; i <= P.nz; i += kThreads) s_zi[i] = __ldg(P.z_i + i);
-  if (LAYERS) {
-    // layer b touches level k iff z_i[k+1] > edges[b] && z_i[k] < edges[b+1]; the layers touching a level are
-    // consecutive: lo | hi << 8, or kNoLayer
-    for (int i = threadIdx.x; i < P.nz; i += kThreads) {
-      const double zt = __ldg(P.z_i + i), zb = __ldg(P.z_i + i + 1);
-      int lo = -1, hi = -1;
-      for (int b = 0; b < layer_count(L); ++b)
-        if (zb > layer_edge(L, b) && zt < layer_edge(L, b + 1)) {
-          if (lo < 0) lo = b;
-          hi = b;
-        }
-      s_lay[i] = lo < 0 ? kNoLayer : (lo | (hi << 8));
-    }
-  }
+  if (LAYERS) fill_layer_table<kThreads>(s_lay, P.z_i, P.nz, L);
   __syncthreads();
 
   int col = tid;  // column of the tile this thread integrates
@@ -458,8 +387,7 @@ __global__ void ML_TMA_KERNEL_ATTR
           if (GLOBAL) {
             w = vraw_isnan(v) ? 0.0 : vraw_value(v);
           } else if (LAYERS) {
-            const int lay = s_lay[z];
-            const bool touches = lay != kNoLayer && (lay & 255) <= b && b <= (lay >> 8);
+            const bool touches = layer_touches(s_lay[z], b);
             w = (vraw_isnan(v) || !touches) ? 0.0 : layer_w(L, s_zi, depth, z, b);
             sub = __ldg(P.rho_ref + j);
           } else {

@@ -42,6 +42,13 @@ int launch_variants(int eos, const void* T, const void* S, const void* T_ref, co
                     int nz, int64_t ncol, double* eta_steric, double* eta_thermo, double* eta_halo, double* rho_ref_out,
                     double* sums, double* partials, cudaStream_t st);
 
+// kLocalLayers3: launch_variants with a supplied reference (rho_ref read), split by depth layer; eta_* [nt][nlayers][ncol]
+// each (NULL = not wanted), edges (host) as ml_steric_local_layers; eligibility is variants_eligible
+int launch_local_layers_variants(int eos, const void* T, const void* S, const void* T_ref, const void* S_ref,
+                                 const double* rho_ref, const void* v_ref, const double* z_i, const double* deptho,
+                                 const double* p_level, double coef, const double* edges, int nlayers, int nt, int nz,
+                                 int64_t ncol, double* eta_steric, double* eta_thermo, double* eta_halo, cudaStream_t st);
+
 // the three global masses per step from one pass (ml_tma3.cu), each bit-identical to one launch_global with
 // BC = 0 / 2 / 1; eligibility is variants_eligible.  sums != NULL: T_ref / S_ref are the step-0 slabs of T / S and
 // {volo, masso} of the reference state are reduced on the way.  Any masso may be NULL.  `partials` holds

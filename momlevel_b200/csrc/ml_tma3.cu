@@ -22,9 +22,17 @@
 //                    chunk: 17 fp64 instructions per level and column instead of an 8-byte load), and the
 //                    chunk that starts at step 0 also reduces volo / masso, stores rho_ref when asked and
 //                    leaves its step-0 heights at exactly zero.
+//         kLocalLayers3  kLocal3 split by depth layer (ml_tma.cu, kLocalLayers): level z feeds layer b with the weight
+//                    calc_dz(top=edges[b], bottom=edges[b+1]); the 3 x TC sums belong to one layer at a time and are
+//                    stored ([t][layer][col] per height) when the sweep leaves the layer's last level.  A level that
+//                    holds an edge (at most nlayers - 1 of them) evaluates its three densities again after the
+//                    straight-line block instead of keeping 3 x TC differences live through it; the evaluation is the
+//                    same, so are the bits.
 // Eligibility is the single-height family's (fp32, 16-byte aligned, ncol % 4 == 0, ncol >= 256).
 #include "ml_tma_dev.cuh"
 #include "ml_tma.cuh"
+
+#include <type_traits>
 
 namespace ml {
 namespace tma {
@@ -36,12 +44,14 @@ namespace tma {
 #define ML_TMA3_MONTGOMERY 0
 #endif
 
-enum Mode3 { kLocal3 = 0, kSelfRef3 = 2 };
+enum Mode3 { kLocal3 = 0, kSelfRef3 = 2, kLocalLayers3 = 4 };
+template <int MODE>
+using LayersOf3 = typename std::conditional<MODE == kLocalLayers3, LayerParams, NoLayers>::type;
 
 struct Params3 {
   const float *T, *S;        // [nt][nz][ncol]  (repair pass; the sweep goes through the tensor maps)
   const float *Tref, *Sref;  // [nz][ncol]
-  const double* rho_ref;     // kLocal3: read
+  const double* rho_ref;     // kLocal3, kLocalLayers3: read
   double* rho_ref_out;       // kSelfRef3, chunk 0: written (may be NULL)
   const float* v_ref;
   const double *z_i, *deptho, *p_level;
@@ -49,7 +59,8 @@ struct Params3 {
   int nt, nz, t_start;
   unsigned nchunks, tiles;
   i64 ncol;
-  double* eta[3];            // steric, thermosteric, halosteric: [nt][ncol] each (NULL = not wanted)
+  double* eta[3];            // steric, thermosteric, halosteric: [nt][ncol] each, kLocalLayers3 [nt][nlayers][ncol]
+                             // (NULL = not wanted)
   double* partials;          // kSelfRef3: [2][tiles] = {volo, masso}, written by the chunk that starts at step 0
 };
 
@@ -64,8 +75,10 @@ __host__ __device__ constexpr int stages3(int tc) { return tc > 8 ? 6 : 4; }
 template <int EOS, int TC, int MODE, int TILE>
 __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
     k_steric_tma3(const __grid_constant__ CUtensorMap mapT, const __grid_constant__ CUtensorMap mapS,
-                  const __grid_constant__ CUtensorMap mapTr, const __grid_constant__ CUtensorMap mapSr, const Params3 P) {
+                  const __grid_constant__ CUtensorMap mapTr, const __grid_constant__ CUtensorMap mapSr, const Params3 P,
+                  const LayersOf3<MODE> L) {
   constexpr bool SELFREF = MODE == kSelfRef3;
+  constexpr bool LAYERS = MODE == kLocalLayers3;
   constexpr int kWarpsT = TILE / 32;
   constexpr int kStages = stages3(TC);
   constexpr int kRows = 2 * TC + 2;
@@ -83,6 +96,7 @@ __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
   double* s_zi = s_p + P.nz;
   int* s_key = reinterpret_cast<int*>(s_zi + P.nz + 1);
   int* s_col = s_key + TILE;
+  int* s_lay = s_col + TILE;  // [nz] kLocalLayers3: layers touching the level
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const unsigned tile = blockIdx.x / P.nchunks;
@@ -114,6 +128,7 @@ __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
   }
   for (int i = threadIdx.x; i < nz; i += TILE) s_p[i] = __ldg(P.p_level + i);
   for (int i = threadIdx.x; i <= nz; i += TILE) s_zi[i] = __ldg(P.z_i + i);
+  if (LAYERS) fill_layer_table<TILE>(s_lay, P.z_i, nz, L);
   __syncthreads();
 
   // columns of the tile ranked by wet depth (see ml_tma.cu): thread i integrates the i-th deepest column
@@ -142,6 +157,12 @@ __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
   unsigned v_n = ld_vraw(P.v_ref, cc);
   if (!SELFREF) rref_n = __ldg(P.rho_ref + cc);
   const bool surface_wet = !vraw_isnan(v_n);  // steric.py:166
+  // kLocalLayers3: the layer the sums belong to, whether a stored sum met a missing value, and where each height goes
+  int cur = 0;
+  bool poisoned = false;
+  LayerOut out[3];
+#pragma unroll
+  for (int v = 0; v < 3; ++v) out[v] = {P.eta[v], P.coef, P.nt, P.ncol, c, t0, in && P.eta[v] != nullptr, surface_wet};
 
   for (int z = 0; z < nz; ++z) {
     const double rref_z = rref_n;
@@ -156,8 +177,21 @@ __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
     const bool dry = vraw_isnan(v_z);
     double w = level_dz(depth, s_zi[z], s_zi[z + 1]);
     if (dry || (!SELFREF && isnan(rref_z))) w = 0.0;  // steric.py:151-153
+    if (LAYERS && s_lay[z] == kNoLayer) w = 0.0;      // no layer takes this level
     eos.set_level(s_p[z]);
     const bool live = nonzero(w);
+    // kLocalLayers3: close the layers that ended above this level (in every warp, wet or not); `wl` is the weight of
+    // the level in its one layer, or -- where an edge falls inside the level (lo < hi) -- in layer lo
+    int lo = 0, hi = 0;
+    double wl = w;
+    if (LAYERS && s_lay[z] != kNoLayer) {
+      lo = s_lay[z] & 255;
+      hi = s_lay[z] >> 8;
+      for (; cur < lo; ++cur)
+#pragma unroll
+        for (int v = 0; v < 3; ++v) close_layer<TC>(acc[v], poisoned, out[v], L, cur);
+      wl = live ? layer_w(L, s_zi, depth, z, lo) : 0.0;
+    }
     const unsigned live_lanes = __ballot_sync(0xffffffffu, live);
     const int s = z % kStages;
     const float* st = stage_base + (size_t)s * kStageFloats;
@@ -195,9 +229,9 @@ __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
           acc[1][kk] = fma(w, p2 * (R12 * d1) - rsub, acc[1][kk]);
           acc[2][kk] = fma(w, p3 * (R * d12) - rsub, acc[2][kk]);
         } else {
-          acc[0][kk] = fma(w, eos.rho(Tv, Sv) - rsub, acc[0][kk]);
-          acc[1][kk] = fma(w, eos.rho_pinned_s(qs, Tv) - rsub, acc[1][kk]);
-          acc[2][kk] = fma(w, eos.rho_pinned_t(qt, Sv) - rsub, acc[2][kk]);
+          acc[0][kk] = fma(LAYERS ? wl : w, eos.rho(Tv, Sv) - rsub, acc[0][kk]);
+          acc[1][kk] = fma(LAYERS ? wl : w, eos.rho_pinned_s(qs, Tv) - rsub, acc[1][kk]);
+          acc[2][kk] = fma(LAYERS ? wl : w, eos.rho_pinned_t(qt, Sv) - rsub, acc[2][kk]);
         }
       }
     } else if (chunk0) {
@@ -216,6 +250,32 @@ __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
       }
       if (P.rho_ref_out) P.rho_ref_out[(i64)z * P.ncol + c] = sub;
     }
+    if (LAYERS && lo < hi) {
+      // an edge falls inside level z: layers lo .. hi - 1 are stored and the sums start layer hi.  The differences
+      // rho - rho_ref of the level are evaluated again here, out of the straight-line block above (a layer test
+      // inside it broke the folding of - rho_ref into the EOS's last multiply: other bits, 1.77x the time)
+      if (live_lanes != 0u) {
+        const int first_wet = __shfl_sync(0xffffffffu, col, __ffs(live_lanes) - 1);
+        const int src = live ? col : first_wet;
+        const typename Eos<EOS>::Pinned qs = eos.pin_s((double)st[kOffSr + src]);
+        const typename Eos<EOS>::Pinned qt = eos.pin_t((double)st[kOffTr + src]);
+        const double rsub = live ? sub : 0.0;
+#pragma unroll
+        for (int kk = 0; kk < TC; ++kk) {
+          const double Tv = (double)st[kk * TILE + src];
+          const double Sv = (double)st[kOffS + kk * TILE + src];
+          split_level(acc[0][kk], poisoned, out[0], L, s_zi, depth, z, lo, hi, live, kk, eos.rho(Tv, Sv) - rsub);
+          split_level(acc[1][kk], poisoned, out[1], L, s_zi, depth, z, lo, hi, live, kk, eos.rho_pinned_s(qs, Tv) - rsub);
+          split_level(acc[2][kk], poisoned, out[2], L, s_zi, depth, z, lo, hi, live, kk, eos.rho_pinned_t(qt, Sv) - rsub);
+        }
+      } else {
+#pragma unroll
+        for (int kk = 0; kk < TC; ++kk)  // a warp without water still closes its layers
+#pragma unroll
+          for (int v = 0; v < 3; ++v) split_level(acc[v][kk], poisoned, out[v], L, s_zi, depth, z, lo, hi, live, kk, 0.0);
+      }
+      cur = hi;
+    }
     __syncwarp();
     if (lane == 0 && stage_done(empty + s, released + s, kWarpsT, (uint32_t)(z / kStages) & 1u) && z + kStages < nz)
       refill_stage(z + kStages);
@@ -233,40 +293,55 @@ __global__ void __launch_bounds__(TILE, ctas_per_sm3(TC, TILE))
   // from global memory with that rule -- all three heights, with the sweep's own evaluation: a height that met no
   // hole comes out as it was, and a repaired one does not depend on how the time axis was cut into chunks, so the
   // fields stay identical to the single-height kernels'.  (Kept in this simple form on purpose: repairing per height,
-  // or out of line, changed the register allocation of the sweep above and cost it 4 %.)
-  bool poisoned = false;
+  // or out of line, changed the register allocation of the sweep above and cost it 4 %.)  kLocalLayers3: every layer of
+  // every height of the column is integrated again and overwritten.
+  if (LAYERS)
+    for (; cur < layer_count(L); ++cur)  // the last layer, and those wholly below the grid: 0
+#pragma unroll
+      for (int v = 0; v < 3; ++v) close_layer<TC>(acc[v], poisoned, out[v], L, cur);
 #pragma unroll
   for (int v = 0; v < 3; ++v)
 #pragma unroll
     for (int k = 0; k < TC; ++k) poisoned |= is_nan_q(acc[v][k]);
   if (poisoned && in) {
+    for (int b = 0; b < (LAYERS ? layer_count(L) : 1); ++b) {
 #pragma unroll
-    for (int v = 0; v < 3; ++v)
+      for (int v = 0; v < 3; ++v)
 #pragma unroll
-      for (int k = 0; k < TC; ++k) acc[v][k] = 0.0;
-    const i64 lvl = (i64)nz * P.ncol;
-    for (int z = 0; z < nz; ++z) {
-      const i64 j = (i64)z * P.ncol + c;
-      const unsigned v = ld_vraw(P.v_ref, j);
-      const double w = vraw_isnan(v) ? 0.0 : level_dz(depth, s_zi[z], s_zi[z + 1]);
-      if (!nonzero(w)) continue;
-      eos.set_level(s_p[z]);
-      const double Tr = (double)__ldg(P.Tref + j), Sr = (double)__ldg(P.Sref + j);
-      const double sub = SELFREF ? eos.rho(Tr, Sr) : __ldg(P.rho_ref + j);
-      const typename Eos<EOS>::Pinned qs = eos.pin_s(Sr);
-      const typename Eos<EOS>::Pinned qt = eos.pin_t(Tr);
+        for (int k = 0; k < TC; ++k) acc[v][k] = 0.0;
+      const i64 lvl = (i64)nz * P.ncol;
+      for (int z = 0; z < nz; ++z) {
+        const i64 j = (i64)z * P.ncol + c;
+        const unsigned v = ld_vraw(P.v_ref, j);
+        double w = vraw_isnan(v) ? 0.0 : level_dz(depth, s_zi[z], s_zi[z + 1]);
+        if (LAYERS) {
+          const bool touches = layer_touches(s_lay[z], b);
+          w = (vraw_isnan(v) || !touches) ? 0.0 : layer_w(L, s_zi, depth, z, b);
+        }
+        if (!nonzero(w)) continue;
+        eos.set_level(s_p[z]);
+        const double Tr = (double)__ldg(P.Tref + j), Sr = (double)__ldg(P.Sref + j);
+        const double sub = SELFREF ? eos.rho(Tr, Sr) : __ldg(P.rho_ref + j);
+        const typename Eos<EOS>::Pinned qs = eos.pin_s(Sr);
+        const typename Eos<EOS>::Pinned qt = eos.pin_t(Tr);
 #pragma unroll
-      for (int k = 0; k < TC; ++k) {
-        if (t0 + k >= P.nt || (chunk0 && k == 0)) continue;
-        const double Tv = (double)__ldg(P.T + (i64)(t0 + k) * lvl + j);
-        const double Sv = (double)__ldg(P.S + (i64)(t0 + k) * lvl + j);
-        fma_skipnan(acc[0][k], w, eos.rho(Tv, Sv) - sub);
-        fma_skipnan(acc[1][k], w, eos.rho_pinned_s(qs, Tv) - sub);
-        fma_skipnan(acc[2][k], w, eos.rho_pinned_t(qt, Sv) - sub);
+        for (int k = 0; k < TC; ++k) {
+          if (t0 + k >= P.nt || (chunk0 && k == 0)) continue;
+          const double Tv = (double)__ldg(P.T + (i64)(t0 + k) * lvl + j);
+          const double Sv = (double)__ldg(P.S + (i64)(t0 + k) * lvl + j);
+          fma_skipnan(acc[0][k], w, eos.rho(Tv, Sv) - sub);
+          fma_skipnan(acc[1][k], w, eos.rho_pinned_s(qs, Tv) - sub);
+          fma_skipnan(acc[2][k], w, eos.rho_pinned_t(qt, Sv) - sub);
+        }
       }
+      if (LAYERS)
+#pragma unroll
+        for (int v = 0; v < 3; ++v)
+#pragma unroll
+          for (int k = 0; k < TC; ++k) store_height(out[v], L, b, k, acc[v][k]);
     }
   }
-  if (in) {
+  if (in && !LAYERS) {
 #pragma unroll
     for (int v = 0; v < 3; ++v) {
       if (P.eta[v] == nullptr) continue;
@@ -498,21 +573,25 @@ __global__ void __launch_bounds__(kTile, ctas_per_sm3(TC))
 
 // ----------------------------------------------------------------------- host side
 template <int TC, int TILE>
-static size_t smem_bytes3(int nz) {
+static size_t smem_bytes3(int nz, bool layers) {
   return (size_t)stages3(TC) * (size_t)((2 * TC + 2) * TILE * 4) + 3 * stages3(TC) * sizeof(uint64_t) +
-         (size_t)(TILE / 32) * 2 * sizeof(double) + (size_t)(2 * nz + 1) * sizeof(double) + 2 * TILE * sizeof(int) + 128;
+         (size_t)(TILE / 32) * 2 * sizeof(double) + (size_t)(2 * nz + 1) * sizeof(double) + 2 * TILE * sizeof(int) + 128 +
+         (layers ? (size_t)nz * sizeof(int) : 0);
 }
 
 template <int EOS, int TC, int MODE, int TILE>
-static int launch_one3(const CUtensorMap maps[4], const Params3& P, unsigned tiles, unsigned chunks, cudaStream_t st) {
+static int launch_one3(const CUtensorMap maps[4], const Params3& P, unsigned tiles, unsigned chunks, cudaStream_t st,
+                       const LayerParams* lp) {
   auto kern = k_steric_tma3<EOS, TC, MODE, TILE>;
-  const size_t smem = smem_bytes3<TC, TILE>(P.nz);
+  const size_t smem = smem_bytes3<TC, TILE>(P.nz, MODE == kLocalLayers3);
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(k_steric_tma3)");
   Params3 Q = P;
   Q.tiles = tiles;
   Q.nchunks = chunks;
-  kern<<<tiles * chunks, TILE, smem, st>>>(maps[0], maps[1], maps[2], maps[3], Q);
+  LayersOf3<MODE> L{};
+  if constexpr (MODE == kLocalLayers3) L = *lp;
+  kern<<<tiles * chunks, TILE, smem, st>>>(maps[0], maps[1], maps[2], maps[3], Q, L);
   return launched("k_steric_tma3");
 }
 
@@ -548,10 +627,24 @@ static int main_tc3() {
   const int t = tls().variants_chunk % 100;  // ml_set_variants_chunk
   return (t == 4 || t == 6 || t == 8 || t == 12) ? t : from_env;
 }
+// kLocalLayers3 carries the 3 x TC sums of kLocal3 plus the layer bookkeeping; only the widths that compile without
+// spills are instantiated: 4, 6 and 12 (the Wright kernel spills at 8 under the 128-register cap of two CTAs per SM;
+// ptxas, sm_100a: profiles/r05_ptxas_registers.txt).  Main width measured on OM4p25 x 12, one B200 at 1000 W
+// (profiles/r05_layers_variants.json, medians): 6-step chunks, two CTAs per SM: 5.42 ms; 4-step: 6.01 ms; 12-step, one
+// CTA per SM (222 registers): 6.78 ms.  ml_set_variants_chunk / ML_TMA3_TC select among the instantiated ones.
+__host__ __device__ constexpr bool has_tc3(int mode, int tc) { return mode != kLocalLayers3 || tc != 8; }
+#ifndef ML_TMA3L_TC
+#define ML_TMA3L_TC 6
+#endif
+static int main_tc_layers3() {
+  const int t = main_tc3();
+  const bool asked = tls().variants_chunk % 100 != 0 || getenv("ML_TMA3_TC") != nullptr;
+  return asked && has_tc3(kLocalLayers3, t) ? t : ML_TMA3L_TC;
+}
 
 template <int MODE, int TILE>
 static int launch_span3(int eos, const void* T, const void* S, const void* Tr, const void* Sr, Params3 P, int t_begin,
-                        int t_end, int tc, cudaStream_t st) {
+                        int t_end, int tc, cudaStream_t st, const LayerParams* lp) {
   // one launch: chunks of `tc` steps covering [t_begin, t_end)
   CUtensorMap maps[4];
   const bool ok = make_map(&maps[0], T, 3, P.ncol, P.nz, P.nt, tc, TILE) && make_map(&maps[1], S, 3, P.ncol, P.nz, P.nt, tc, TILE) &&
@@ -560,30 +653,35 @@ static int launch_span3(int eos, const void* T, const void* S, const void* Tr, c
   P.t_start = t_begin;
   const unsigned tiles = (unsigned)((P.ncol + TILE - 1) / TILE);
   const unsigned chunks = (unsigned)((t_end - t_begin + tc - 1) / tc);
-#define ML_TMA3_GO(E, TCV) return launch_one3<E, TCV, MODE, TILE>(maps, P, tiles, chunks, st)
+#define ML_TMA3_GO(E, TCV) \
+  if constexpr (has_tc3(MODE, TCV)) return launch_one3<E, TCV, MODE, TILE>(maps, P, tiles, chunks, st, lp)
   if (eos == ML_EOS_WRIGHT) {
     if (tc == 12) ML_TMA3_GO(0, 12);
     if (tc == 8) ML_TMA3_GO(0, 8);
     if (tc == 6) ML_TMA3_GO(0, 6);
-    ML_TMA3_GO(0, 4);
+    if (tc == 4) ML_TMA3_GO(0, 4);
+  } else {
+    if (tc == 12) ML_TMA3_GO(1, 12);
+    if (tc == 8) ML_TMA3_GO(1, 8);
+    if (tc == 6) ML_TMA3_GO(1, 6);
+    if (tc == 4) ML_TMA3_GO(1, 4);
   }
-  if (tc == 12) ML_TMA3_GO(1, 12);
-  if (tc == 8) ML_TMA3_GO(1, 8);
-  if (tc == 6) ML_TMA3_GO(1, 6);
-  ML_TMA3_GO(1, 4);
 #undef ML_TMA3_GO
+  return fail(ML_ERR_MODE, "no %d-step chunk kernel for this mode", tc);
 }
 
 template <int MODE, int TILE>
 static int launch_all3(int eos, const void* T, const void* S, const void* Tr, const void* Sr, const Params3& P,
-                       cudaStream_t st) {
-  const int main_tc = main_tc3();
+                       cudaStream_t st, const LayerParams* lp = nullptr) {
+  const int main_tc = MODE == kLocalLayers3 ? main_tc_layers3() : main_tc3();
   const int full = P.nt / main_tc, rest = P.nt % main_tc;
   int rc = ML_OK;
-  if (full > 0) rc = launch_span3<MODE, TILE>(eos, T, S, Tr, Sr, P, 0, full * main_tc, main_tc, st);
+  if (full > 0) rc = launch_span3<MODE, TILE>(eos, T, S, Tr, Sr, P, 0, full * main_tc, main_tc, st, lp);
   if (rc == ML_OK && rest > 0) {
-    const int tc = rest <= 4 ? 4 : (rest <= 6 ? 6 : (rest <= 8 ? 8 : 12));
-    rc = launch_span3<MODE, TILE>(eos, T, S, Tr, Sr, P, full * main_tc, P.nt, tc, st);
+    int tc = 12;
+    for (const int w : {8, 6, 4})
+      if (w >= rest && has_tc3(MODE, w)) tc = w;
+    rc = launch_span3<MODE, TILE>(eos, T, S, Tr, Sr, P, full * main_tc, P.nt, tc, st, lp);
   }
   return rc;
 }
@@ -630,6 +728,38 @@ int launch_variants(int eos, const void* T, const void* S, const void* T_ref, co
                        : launch_all3<kSelfRef3, 256>(eos, T, S, T_ref, S_ref, P, st);
   if (rc) return rc;
   return reduce_rows(partials, (ncol + tile - 1) / tile, sums, 2, st);
+}
+
+int launch_local_layers_variants(int eos, const void* T, const void* S, const void* T_ref, const void* S_ref,
+                                 const double* rho_ref, const void* v_ref, const double* z_i, const double* deptho,
+                                 const double* p_level, double coef, const double* edges, int nlayers, int nt, int nz,
+                                 int64_t ncol, double* eta_steric, double* eta_thermo, double* eta_halo, cudaStream_t st) {
+  Params3 P;
+  P.T = static_cast<const float*>(T);
+  P.S = static_cast<const float*>(S);
+  P.Tref = static_cast<const float*>(T_ref);
+  P.Sref = static_cast<const float*>(S_ref);
+  P.rho_ref = rho_ref;
+  P.rho_ref_out = nullptr;
+  P.v_ref = static_cast<const float*>(v_ref);
+  P.z_i = z_i;
+  P.deptho = deptho;
+  P.p_level = p_level;
+  P.coef = coef;
+  P.nt = nt;
+  P.nz = nz;
+  P.t_start = 0;
+  P.nchunks = 1;
+  P.tiles = 0;
+  P.ncol = ncol;
+  P.eta[0] = eta_steric;
+  P.eta[1] = eta_thermo;
+  P.eta[2] = eta_halo;
+  P.partials = nullptr;
+  LayerParams lp;
+  lp.nlayers = nlayers;
+  for (int b = 0; b <= ML_MAX_LAYERS; ++b) lp.edges[b] = b <= nlayers ? edges[b] : 0.0;
+  return launch_all3<kLocalLayers3, kTile>(eos, T, S, T_ref, S_ref, P, st, &lp);
 }
 
 // global masses: 256-column tiles whatever ML_TMA3_TILE says (the column order inside a tile decides the bits)

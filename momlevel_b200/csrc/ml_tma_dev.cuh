@@ -186,6 +186,83 @@ __device__ __forceinline__ int sorted_column(int key, unsigned* s_key, int* s_co
   return sorted_column_t<kTile>(key, s_key, s_col);
 }
 
+// ----------------------------------------------------------------------- depth layers
+// The layered modes (kLocalLayers in ml_tma.cu, kLocalLayers3 in ml_tma3.cu): level z feeds layer b with the weight
+// calc_dz(top=edges[b], bottom=edges[b+1]) (derived.py:295-318) and the height of a layer is stored when the sweep
+// leaves its last level.  The edges are a kernel parameter of their own (a larger Params cost the kLocal kernel four
+// registers); the other modes take an empty one.
+constexpr int kNoLayer = 0xffff;  // no layer touches the level
+struct LayerParams {
+  int nlayers;                      // eta is [nt][nlayers][ncol]
+  double edges[ML_MAX_LAYERS + 1];  // increasing; the last may be +inf
+};
+struct NoLayers {};
+__device__ __forceinline__ int layer_count(const LayerParams& L) { return L.nlayers; }
+__device__ __forceinline__ int layer_count(const NoLayers&) { return 0; }
+__device__ __forceinline__ double layer_edge(const LayerParams& L, int b) { return L.edges[b]; }
+__device__ __forceinline__ double layer_edge(const NoLayers&, int) { return 0.0; }
+// The layers that touch each level, worked out once per CTA: layer b touches level k iff z_i[k+1] > edges[b] &&
+// z_i[k] < edges[b+1]; they are consecutive: lo | hi << 8, or kNoLayer.  The layers a level touches are the same
+// for every column (only the bottom clip varies, and it can only zero a weight).
+template <int NTHREADS, typename LP>
+__device__ __forceinline__ void fill_layer_table(int* s_lay, const double* z_i, int nz, const LP& L) {
+  for (int i = threadIdx.x; i < nz; i += NTHREADS) {
+    const double zt = __ldg(z_i + i), zb = __ldg(z_i + i + 1);
+    int lo = -1, hi = -1;
+    for (int b = 0; b < layer_count(L); ++b)
+      if (zb > layer_edge(L, b) && zt < layer_edge(L, b + 1)) {
+        if (lo < 0) lo = b;
+        hi = b;
+      }
+    s_lay[i] = lo < 0 ? kNoLayer : (lo | (hi << 8));
+  }
+}
+__device__ __forceinline__ bool layer_touches(int lay, int b) { return lay != kNoLayer && (lay & 255) <= b && b <= (lay >> 8); }
+// where a thread stores the heights of its column; one per output field (in == false: nothing is stored)
+struct LayerOut {
+  double* eta;
+  double coef;
+  int nt;
+  i64 ncol, c;
+  int t0;
+  bool in, surface_wet;
+};
+// weight of level z in layer b: derived.py:295-318 with top = edges[b], bottom = edges[b+1] (the arithmetic of
+// k_calc_dz); depth and z_i are never NaN here
+template <typename LP>
+__device__ __forceinline__ double layer_w(const LP& L, const double* s_zi, double depth, int z, int b) {
+  return fmin(fmax(s_zi[z + 1] - layer_edge(L, b), 0.0), level_dz(fmin(depth, layer_edge(L, b + 1)), s_zi[z], s_zi[z + 1]));
+}
+template <typename LP>
+__device__ __forceinline__ void store_height(const LayerOut& o, const LP& L, int b, int k, double a) {
+  if (o.in && o.t0 + k < o.nt) o.eta[((i64)(o.t0 + k) * layer_count(L) + b) * o.ncol + o.c] = o.surface_wet ? o.coef * a : nan("");
+}
+// the sweep has left layer b: store its sums and start the next layer from zero
+template <int TC, typename LP>
+__device__ __forceinline__ void close_layer(double (&acc)[TC], bool& poisoned, const LayerOut& o, const LP& L, int b) {
+#pragma unroll
+  for (int k = 0; k < TC; ++k) {
+    poisoned |= is_nan_q(acc[k]);
+    store_height(o, L, b, k, acc[k]);
+    acc[k] = 0.0;
+  }
+}
+// level z closes layers lo .. hi - 1 and opens hi (an edge falls inside it).  acc already holds layer lo with the
+// level's share of d = rho - rho_ref of step k added: store it, store the layers that lie inside the level, and
+// start layer hi with its share of d
+template <typename LP>
+__device__ __forceinline__ void split_level(double& acc, bool& poisoned, const LayerOut& o, const LP& L, const double* s_zi,
+                                            double depth, int z, int lo, int hi, bool live, int k, double d) {
+  poisoned |= is_nan_q(acc);
+  store_height(o, L, lo, k, acc);
+  for (int b = lo + 1; b < hi; ++b) {
+    const double a = (live ? layer_w(L, s_zi, depth, z, b) : 0.0) * d;
+    poisoned |= is_nan_q(a);
+    store_height(o, L, b, k, a);
+  }
+  acc = (live ? layer_w(L, s_zi, depth, z, hi) : 0.0) * d;
+}
+
 // ----------------------------------------------------------------------- host side
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,

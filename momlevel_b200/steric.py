@@ -789,11 +789,17 @@ def steric_layers(dset, depth_edges=(0.0, 700.0, 2000.0, None), reference=None, 
     layers add up to more than the full-column height.  The remaining arguments are those of :func:`steric` with
     ``domain="local"``; ``reference=None`` builds the reference state from the first step first.
 
+    ``variant`` may also be a list or tuple of distinct names from ``("steric", "thermosteric", "halosteric")``: the
+    validation, the reference state and the move of T and S to the device are then done once, and one pass over T
+    and S gives every height asked for (a sea-level budget: how much of a layer's change is warming and how much is
+    freshening).  Each result variable is the one a call with that name alone returns, bit for bit.
+
     Returns ``(result, reference)``: ``result[variant]`` has dims ``(time, depth_layer, y, x)``, ``result["layer_top"]``
     and ``result["layer_bottom"]`` are ``(depth_layer,)`` (``inf``: the sea floor).  There is no ``delta_rho``:
     it is the field :func:`steric` returns.
     """
     edges = core.layer_edges(depth_edges)
+    names = None if isinstance(variant, str) else core.variant_names(variant)
     xarray_in = type(dset).__module__.startswith("xarray")
     if xarray_in:
         from . import xarray_io
@@ -827,28 +833,42 @@ def steric_layers(dset, depth_edges=(0.0, 700.0, 2000.0, None), reference=None, 
             print("Generating reference state from first timestep")
     validate_dataset(reference, reference=True, strict=strict)
 
-    # steric.py:115-125
-    if variant == "thermosteric":
-        thetao, so, t_bcast, s_bcast = dset["thetao"], reference["so"], False, True
-    elif variant == "halosteric":
-        thetao, so, t_bcast, s_bcast = reference["thetao"], dset["so"], True, False
-    elif variant == "steric":
-        thetao, so, t_bcast, s_bcast = dset["thetao"], dset["so"], False, False
+    if names is not None:
+        # the heights asked for from one call: T_ref, S_ref are the reference slabs (steric.py:115-121)
+        full = dset["thetao"]
+        if full.dims[0] != tcoord or full.dims[1] != zcoord or dset["so"].dims != full.dims:
+            raise ValueError(f"expecting fields laid out ({tcoord}, {zcoord}, y, x), got {full.dims}")
+        _check_depths(dset, zcoord, zbounds)
+        etas = core.steric_local_layers_variants(full.data, dset["so"].data, reference["thetao"].data,
+                                                 reference["so"].data, reference["rho"].data,
+                                                 reference["volcello"].data, dset[zbounds].data, dset["deptho"].data,
+                                                 pres, edges, rhozero=rhozero, eos=equation_of_state, variants=names)
     else:
-        raise ValueError(f"Unknown variant '{variant}' passed to `steric`")
-    full = dset["so"] if t_bcast else dset["thetao"]
-    if full.dims[0] != tcoord or full.dims[1] != zcoord:
-        raise ValueError(f"expecting fields laid out ({tcoord}, {zcoord}, y, x), got {full.dims}")
+        # steric.py:115-125
+        if variant == "thermosteric":
+            thetao, so, t_bcast, s_bcast = dset["thetao"], reference["so"], False, True
+        elif variant == "halosteric":
+            thetao, so, t_bcast, s_bcast = reference["thetao"], dset["so"], True, False
+        elif variant == "steric":
+            thetao, so, t_bcast, s_bcast = dset["thetao"], dset["so"], False, False
+        else:
+            raise ValueError(f"Unknown variant '{variant}' passed to `steric`")
+        full = dset["so"] if t_bcast else dset["thetao"]
+        if full.dims[0] != tcoord or full.dims[1] != zcoord:
+            raise ValueError(f"expecting fields laid out ({tcoord}, {zcoord}, y, x), got {full.dims}")
 
-    _check_depths(dset, zcoord, zbounds)
-    eta = core.steric_local_layers(thetao.data, so.data, reference["rho"].data, reference["volcello"].data,
-                                   dset[zbounds].data, dset["deptho"].data, pres, edges, rhozero=rhozero,
-                                   eos=equation_of_state, t_bcast=t_bcast, s_bcast=s_bcast)
+        _check_depths(dset, zcoord, zbounds)
+        etas = {variant: core.steric_local_layers(thetao.data, so.data, reference["rho"].data,
+                                                  reference["volcello"].data, dset[zbounds].data, dset["deptho"].data,
+                                                  pres, edges, rhozero=rhozero, eos=equation_of_state, t_bcast=t_bcast,
+                                                  s_bcast=s_bcast)}
     result = Dataset()
     # steric.py:169-179, plus the edges
-    result[variant] = DataArray(eta, (tcoord, "depth_layer") + full.dims[2:], attrs={
-        "long_name": f"{variant.capitalize()} height adjustment", "units": "m", "depth_edges": [float(e) for e in edges]})
-    result[variant].encoding["dtype"] = dtype
+    for name in names or (variant,):
+        result[name] = DataArray(etas[name], (tcoord, "depth_layer") + full.dims[2:], attrs={
+            "long_name": f"{name.capitalize()} height adjustment", "units": "m",
+            "depth_edges": [float(e) for e in edges]})
+        result[name].encoding["dtype"] = dtype
     result["layer_top"] = DataArray(edges[:-1].copy(), ("depth_layer",), attrs={
         "long_name": "Top of depth layer", "units": "m"})
     result["layer_bottom"] = DataArray(edges[1:].copy(), ("depth_layer",), attrs={
