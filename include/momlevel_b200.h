@@ -475,7 +475,13 @@ int ml_pack_simd(void);
  * `fill_mode` selects which cells adjust_negative_n2's `adjusted[0] = adjusted[0].fillna(1e-8)`
  * (src/momlevel/derived.py:63) touches: index 0 of the array's FIRST axis, i.e.
  *   0 = the surface level of every slab   (a 3-D field [z][y][x], passed with nouter = 1)
- *   1 = every level of outer slab 0       (a 4-D field [t][z][y][x]: its first time step)
+ *   k = every level of outer slabs [0, k), 1 <= k <= nouter: the outer slabs whose first index
+ *       is 0, i.e. the product of the extents between the first axis and the level axis --
+ *       1 for [t][z][y][x] (its first time step), nt for [member][t][z][y][x] (every time
+ *       step of member 0), nx for a level-last [y][x][z] (the row y = 0, with ncol = 1).
+ *   Any other value returns ML_ERR_MODE.
+ * nouter has no upper limit: above 65535 slabs (the grid.y limit of one launch) the entry points
+ * launch their kernel once per 65535 slabs, and the fill follows the slab index of the whole call.
  * ===================================================================================== */
 
 /* ml_calc_n2 -- squared buoyancy frequency at cell centres, g * (alpha dT/dz - beta dS/dz) with

@@ -236,10 +236,14 @@ def _column_view(x, z_axis):
             int(np.prod(x.shape[z_axis + 1:], dtype=np.int64)))
 
 
-def _fill_mode(ndim, z_axis):
+def _fill_mode(shape, z_axis):
     # adjust_negative_n2's ``adjusted[0]`` is index 0 of the FIRST axis (derived.py:63): the surface level
-    # when the level axis leads, the first outer (time) slab otherwise
-    return 0 if z_axis % ndim == 0 else 1
+    # when the level axis leads, otherwise every outer slab whose first index is 0 -- the first time step of
+    # (time, z, y, x), every time step of member 0 of (member, time, z, y, x), the row y = 0 of (y, x, z)
+    z_axis = z_axis % len(shape)
+    if z_axis == 0:
+        return 0
+    return int(np.prod(shape[1:z_axis], dtype=np.int64))
 
 
 def calc_n2(T, S, z_l, eos="Wright", gravity=-9.8, patm=101325.0, z_axis=1, adjust_negative=False):
@@ -255,7 +259,7 @@ def calc_n2(T, S, z_l, eos="Wright", gravity=-9.8, patm=101325.0, z_axis=1, adju
     out = torch.empty(T.shape, dtype=torch.float64, device=T.device)
     _lib.check(
         L.ml_calc_n2(_eos_id(eos), _dt_id(T), T.data_ptr(), S.data_ptr(), z.data_ptr(), float(gravity), float(patm),
-                     int(bool(adjust_negative)), _fill_mode(T.dim(), z_axis), nouter, nz, ncol, out.data_ptr(), _stream())
+                     int(bool(adjust_negative)), _fill_mode(T.shape, z_axis), nouter, nz, ncol, out.data_ptr(), _stream())
     )
     return out
 
@@ -266,7 +270,7 @@ def adjust_negative_n2(n2, z_axis=1):
     n2 = _f64(n2)
     nouter, nz, ncol = _column_view(n2, z_axis)
     out = torch.empty_like(n2)
-    _lib.check(L.ml_adjust_negative_n2(n2.data_ptr(), _fill_mode(n2.dim(), z_axis), nouter, nz, ncol, out.data_ptr(),
+    _lib.check(L.ml_adjust_negative_n2(n2.data_ptr(), _fill_mode(n2.shape, z_axis), nouter, nz, ncol, out.data_ptr(),
                                        _stream()))
     return out
 
@@ -297,7 +301,7 @@ def wave_speed(n2, dz, z_axis=1):
     assert dz.numel() == nz * ncol, "dz must be [nz][columns]"
     z_axis = z_axis % n2.dim()
     out = torch.empty(tuple(n2.shape[:z_axis]) + tuple(n2.shape[z_axis + 1:]), dtype=torch.float64, device=n2.device)
-    _lib.check(L.ml_wave_speed(n2.data_ptr(), dz.data_ptr(), _fill_mode(n2.dim(), z_axis), nouter, nz, ncol,
+    _lib.check(L.ml_wave_speed(n2.data_ptr(), dz.data_ptr(), _fill_mode(n2.shape, z_axis), nouter, nz, ncol,
                                out.data_ptr(), _stream()))
     return out
 

@@ -92,6 +92,8 @@ enum StratOut { kN2 = 0, kN2Adjusted = 1, kTurnerAngle = 2 };
 // adjust_negative_n2 for one value (derived.py:56-69).  `fill` = this cell belongs to index 0 of
 // the array's FIRST axis, which the reference fills with 1e-8 (time step 0 of a 4-D field, the
 // surface level of a 3-D one); `carry` is the last positive value met further up the column.
+// The kernels take the fill as `fill_slabs`, relative to the slabs of their own launch: < 0 fills
+// the surface level of every slab, n >= 0 every level of the launch's slabs [0, n).
 __device__ __forceinline__ double adjust_step(double n2, bool fill, double& carry) {
   const bool missing = isnan(n2);
   double adj = (missing || n2 <= 0.0) ? nan("") : n2;
@@ -123,7 +125,7 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 template <typename TIn, int EOS, int OUT>
 __global__ void __launch_bounds__(kBlock) k_strat(const TIn* __restrict__ T, const TIn* __restrict__ S,
                                                   const double* __restrict__ z_l, const double* __restrict__ p_level,
-                                                  double gravity, double patm, int fill_mode, int nz, i64 ncol,
+                                                  double gravity, double patm, int fill_slabs, int nz, i64 ncol,
                                                   double* __restrict__ out) {
   extern __shared__ double s_coef[];  // [nz][3] gradient coefficients, [nz] pressure, then the two rings
   double* s_p = s_coef + 3 * nz;
@@ -151,7 +153,7 @@ __global__ void __launch_bounds__(kBlock) k_strat(const TIn* __restrict__ T, con
     cp_async_commit();
   };
   for (int l = 0; l < kRing - 1; ++l) fetch();
-  const bool fill_slab = fill_mode == 1 && blockIdx.y == 0;  // adjusted[0] of a 4-D field is its first time step
+  const bool fill_slab = (int)blockIdx.y < fill_slabs;  // this slab belongs to adjusted[0]
   double carry = nan("");
   // one output cell: the EOS derivatives at (Tc, Sc, p_z) combined with the vertical gradients
   auto emit = [&](int z, double Tc, double Sc, double dtdz, double dsdz) {
@@ -163,7 +165,7 @@ __global__ void __launch_bounds__(kBlock) k_strat(const TIn* __restrict__ T, con
       r = atan((1.0 + ratio) / (1.0 - ratio)) * 57.29577951308232;  // np.degrees: x * (180 / pi)
     } else {
       r = gravity * (alpha * dtdz - beta * dsdz);  // derived.py:401
-      if (OUT == kN2Adjusted) r = adjust_step(r, fill_slab || (fill_mode == 0 && z == 0), carry);
+      if (OUT == kN2Adjusted) r = adjust_step(r, fill_slab || (fill_slabs < 0 && z == 0), carry);
     }
     asm volatile("st.global.cs.f64 [%0], %1;" ::"l"(oc + (i64)z * ncol), "d"(r) : "memory");  // streamed, never re-read
   };
@@ -194,50 +196,80 @@ __global__ void __launch_bounds__(kBlock) k_strat(const TIn* __restrict__ T, con
 }
 
 // adjust_negative_n2 on an existing field (derived.py:30-71)
-__global__ void __launch_bounds__(kBlock) k_adjust_n2(const double* __restrict__ n2, int fill_mode, int nz, i64 ncol,
+__global__ void __launch_bounds__(kBlock) k_adjust_n2(const double* __restrict__ n2, int fill_slabs, int nz, i64 ncol,
                                                       double* __restrict__ out) {
   const i64 c = (i64)blockIdx.x * kBlock + threadIdx.x;
   if (c >= ncol) return;
   const i64 slab = (i64)blockIdx.y * nz * ncol + c;
-  const bool fill_slab = fill_mode == 1 && blockIdx.y == 0;
+  const bool fill_slab = (int)blockIdx.y < fill_slabs;
   double carry = nan("");
   for (int z = 0; z < nz; ++z) {
     const double v = __ldg(n2 + slab + (i64)z * ncol);
-    out[slab + (i64)z * ncol] = adjust_step(v, fill_slab || (fill_mode == 0 && z == 0), carry);
+    out[slab + (i64)z * ncol] = adjust_step(v, fill_slab || (fill_slabs < 0 && z == 0), carry);
   }
 }
 
 // calc_wave_speed (derived.py:821): sum_z sqrt(adjusted n2) dz / pi, skipna.  dz is [nz][ncol].
 __global__ void __launch_bounds__(kBlock) k_wave_speed(const double* __restrict__ n2, const double* __restrict__ dz,
-                                                       int fill_mode, int nz, i64 ncol, double* __restrict__ out) {
+                                                       int fill_slabs, int nz, i64 ncol, double* __restrict__ out) {
   const i64 c = (i64)blockIdx.x * kBlock + threadIdx.x;
   if (c >= ncol) return;
   const i64 slab = (i64)blockIdx.y * nz * ncol + c;
-  const bool fill_slab = fill_mode == 1 && blockIdx.y == 0;
+  const bool fill_slab = (int)blockIdx.y < fill_slabs;
   double carry = nan(""), acc = 0.0;
   for (int z = 0; z < nz; ++z) {
     const double v = __ldg(n2 + slab + (i64)z * ncol);
-    const double term = sqrt(adjust_step(v, fill_slab || (fill_mode == 0 && z == 0), carry)) * __ldg(dz + (i64)z * ncol + c);
+    const double term = sqrt(adjust_step(v, fill_slab || (fill_slabs < 0 && z == 0), carry)) * __ldg(dz + (i64)z * ncol + c);
     if (!isnan(term)) acc += term;
   }
   out[(i64)blockIdx.y * ncol + c] = acc / 3.141592653589793;
+}
+
+// The outer slabs run on grid.y, which holds at most 65535 of them: a longer field (a level-last (y, x, z)
+// field has y * x slabs, a daily record over 179 years 65535 time steps) is launched in chunks of
+// kMaxSlabs, each with its pointers moved to its first slab.
+constexpr i64 kMaxSlabs = 65535;
+
+// fill_slabs of the kernels for the chunk [s0, s0 + n) of a call's slabs: fill_mode 0 = the surface level of
+// every slab (-1); k >= 1 = every level of the call's slabs [0, k), i.e. the chunk's first k - s0 slabs, and
+// none at all in a chunk past them
+inline int chunk_fill(int fill_mode, i64 s0, i64 n) {
+  if (fill_mode == 0) return -1;
+  const i64 k = (i64)fill_mode - s0;
+  return (int)(k <= 0 ? 0 : (k < n ? k : n));
+}
+
+inline int check_fill_mode(int fill_mode, int64_t nouter) {
+  if (fill_mode < 0 || fill_mode > nouter)
+    return fail(ML_ERR_MODE, "fill_mode must be 0 (surface level) or 1..nouter=%lld (leading slabs), got %d",
+                (long long)nouter, fill_mode);
+  return ML_OK;
 }
 
 template <int OUT>
 int launch_strat(int eos, int dtype, const void* T, const void* S, const double* z_l, const double* p_level,
                  double gravity, double patm, int fill_mode, i64 nouter, int nz, i64 ncol, double* out,
                  cudaStream_t st) {
-  const dim3 grid((unsigned)((ncol + kBlock - 1) / kBlock), (unsigned)nouter);
   const size_t smem = (size_t)4 * nz * sizeof(double) + (size_t)2 * kRing * kBlock * elem_size(dtype);
+  for (i64 s0 = 0; s0 < nouter; s0 += kMaxSlabs) {
+    const i64 n = nouter - s0 < kMaxSlabs ? nouter - s0 : kMaxSlabs;
+    const i64 off = s0 * nz * ncol;
+    const char* Tc = static_cast<const char*>(T) + off * elem_size(dtype);
+    const char* Sc = static_cast<const char*>(S) + off * elem_size(dtype);
+    const int fill = chunk_fill(fill_mode, s0, n);
+    const dim3 grid((unsigned)((ncol + kBlock - 1) / kBlock), (unsigned)n);
 #define ML_STRAT(TIN, E) \
-  k_strat<TIN, E, OUT><<<grid, kBlock, smem, st>>>((const TIN*)T, (const TIN*)S, z_l, p_level, gravity, patm, fill_mode, nz, ncol, out)
-  if (dtype == ML_F32) {
-    if (eos == ML_EOS_WRIGHT) ML_STRAT(float, 0); else ML_STRAT(float, 1);
-  } else {
-    if (eos == ML_EOS_WRIGHT) ML_STRAT(double, 0); else ML_STRAT(double, 1);
-  }
+  k_strat<TIN, E, OUT><<<grid, kBlock, smem, st>>>((const TIN*)Tc, (const TIN*)Sc, z_l, p_level, gravity, patm, fill, nz, ncol, out + off)
+    if (dtype == ML_F32) {
+      if (eos == ML_EOS_WRIGHT) ML_STRAT(float, 0); else ML_STRAT(float, 1);
+    } else {
+      if (eos == ML_EOS_WRIGHT) ML_STRAT(double, 0); else ML_STRAT(double, 1);
+    }
 #undef ML_STRAT
-  return launched("k_strat");
+    const int rc = launched("k_strat");
+    if (rc) return rc;
+  }
+  return ML_OK;
 }
 
 int check_strat(int eos, int dtype, const void* T, const void* S, const double* z_l, const double* out, int64_t nouter,
@@ -249,8 +281,8 @@ int check_strat(int eos, int dtype, const void* T, const void* S, const double* 
   ML_REQUIRE_PTR(z_l);
   ML_REQUIRE_PTR(out);
   // numpy.gradient(edge_order=2) needs three points; the coefficient table lives in shared memory
-  if (nouter <= 0 || ncol <= 0 || nz < 3 || nz > kMaxLevels || nouter > 65535)
-    return fail(ML_ERR_SHAPE, "bad extents nouter=%lld nz=%lld ncol=%lld (3 <= nz <= %d, nouter <= 65535)",
+  if (nouter <= 0 || ncol <= 0 || nz < 3 || nz > kMaxLevels)
+    return fail(ML_ERR_SHAPE, "bad extents nouter=%lld nz=%lld ncol=%lld (3 <= nz <= %d)",
                 (long long)nouter, (long long)nz, (long long)ncol, kMaxLevels);
   ML_REQUIRE_ALIGNED(T, elem_size(dtype));
   ML_REQUIRE_ALIGNED(S, elem_size(dtype));
@@ -269,7 +301,7 @@ int ml_calc_n2(int eos, int dtype, const void* T, const void* S, const double* z
                void* stream) {
   int rc = check_strat(eos, dtype, T, S, z_l, out, nouter, nz, ncol);
   if (rc) return rc;
-  if (fill_mode != 0 && fill_mode != 1) return fail(ML_ERR_MODE, "fill_mode must be 0 or 1, got %d", fill_mode);
+  if ((rc = check_fill_mode(fill_mode, nouter))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   if (adjust_negative)
     return launch_strat<kN2Adjusted>(eos, dtype, T, S, z_l, nullptr, gravity, patm, fill_mode, nouter, (int)nz, ncol, out, st);
@@ -289,12 +321,18 @@ int ml_adjust_negative_n2(const double* n2, int fill_mode, int64_t nouter, int64
                           void* stream) {
   ML_REQUIRE_PTR(n2);
   ML_REQUIRE_PTR(out);
-  if (fill_mode != 0 && fill_mode != 1) return fail(ML_ERR_MODE, "fill_mode must be 0 or 1, got %d", fill_mode);
-  if (nouter <= 0 || nz <= 0 || ncol <= 0 || nouter > 65535 || nz > INT32_MAX)
+  if (nouter <= 0 || nz <= 0 || ncol <= 0 || nz > INT32_MAX)
     return fail(ML_ERR_SHAPE, "bad extents nouter=%lld nz=%lld ncol=%lld", (long long)nouter, (long long)nz, (long long)ncol);
-  const dim3 grid((unsigned)((ncol + kBlock - 1) / kBlock), (unsigned)nouter);
-  k_adjust_n2<<<grid, kBlock, 0, (cudaStream_t)stream>>>(n2, fill_mode, (int)nz, ncol, out);
-  return launched("k_adjust_n2");
+  int rc = check_fill_mode(fill_mode, nouter);
+  if (rc) return rc;
+  for (i64 s0 = 0; s0 < nouter; s0 += kMaxSlabs) {
+    const i64 n = nouter - s0 < kMaxSlabs ? nouter - s0 : kMaxSlabs;
+    const i64 off = s0 * nz * ncol;
+    const dim3 grid((unsigned)((ncol + kBlock - 1) / kBlock), (unsigned)n);
+    k_adjust_n2<<<grid, kBlock, 0, (cudaStream_t)stream>>>(n2 + off, chunk_fill(fill_mode, s0, n), (int)nz, ncol, out + off);
+    if ((rc = launched("k_adjust_n2"))) return rc;
+  }
+  return ML_OK;
 }
 
 int ml_wave_speed(const double* n2, const double* dz, int fill_mode, int64_t nouter, int64_t nz, int64_t ncol,
@@ -302,12 +340,18 @@ int ml_wave_speed(const double* n2, const double* dz, int fill_mode, int64_t nou
   ML_REQUIRE_PTR(n2);
   ML_REQUIRE_PTR(dz);
   ML_REQUIRE_PTR(out);
-  if (fill_mode != 0 && fill_mode != 1) return fail(ML_ERR_MODE, "fill_mode must be 0 or 1, got %d", fill_mode);
-  if (nouter <= 0 || nz <= 0 || ncol <= 0 || nouter > 65535 || nz > INT32_MAX)
+  if (nouter <= 0 || nz <= 0 || ncol <= 0 || nz > INT32_MAX)
     return fail(ML_ERR_SHAPE, "bad extents nouter=%lld nz=%lld ncol=%lld", (long long)nouter, (long long)nz, (long long)ncol);
-  const dim3 grid((unsigned)((ncol + kBlock - 1) / kBlock), (unsigned)nouter);
-  k_wave_speed<<<grid, kBlock, 0, (cudaStream_t)stream>>>(n2, dz, fill_mode, (int)nz, ncol, out);
-  return launched("k_wave_speed");
+  int rc = check_fill_mode(fill_mode, nouter);
+  if (rc) return rc;
+  for (i64 s0 = 0; s0 < nouter; s0 += kMaxSlabs) {
+    const i64 n = nouter - s0 < kMaxSlabs ? nouter - s0 : kMaxSlabs;
+    const dim3 grid((unsigned)((ncol + kBlock - 1) / kBlock), (unsigned)n);
+    k_wave_speed<<<grid, kBlock, 0, (cudaStream_t)stream>>>(n2 + s0 * nz * ncol, dz, chunk_fill(fill_mode, s0, n), (int)nz,
+                                                            ncol, out + s0 * ncol);
+    if ((rc = launched("k_wave_speed"))) return rc;
+  }
+  return ML_OK;
 }
 
 }  // extern "C"

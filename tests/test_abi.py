@@ -77,6 +77,22 @@ def test_argument_errors_are_reported_without_a_device():
         _lib.check(-6)
 
 
+def test_fill_mode_is_checked_before_any_launch():
+    """fill_mode is 0 (surface level of every slab) or k in [1, nouter] (every level of slabs [0, k))."""
+    from momlevel_b200 import _lib
+
+    L = _lib.lib()
+    buf = (ctypes.c_double * 64)()
+    p = ctypes.cast(buf, ctypes.c_void_p)
+    before = L.ml_launch_count()
+    for fill in (-1, 4):  # nouter = 3
+        assert L.ml_adjust_negative_n2(p, fill, 3, 4, 5, p, None) == -5
+        assert b"fill_mode" in L.ml_last_error()
+        assert L.ml_wave_speed(p, p, fill, 3, 4, 5, p, None) == -5
+        assert L.ml_calc_n2(0, 1, p, p, p, -9.8, 101325.0, 1, fill, 3, 4, 5, p, None) == -5
+    assert L.ml_launch_count() == before
+
+
 def test_no_product_import_of_the_oracle():
     """The product must never route through the oracle (test infrastructure only)."""
     for path in (ROOT / "momlevel_b200").rglob("*.py"):
