@@ -273,6 +273,38 @@ int ml_steric_local_layers_variants(int eos, int dtype, const void* T, const voi
                                     double* eta_thermosteric, double* eta_halosteric, void* stream);
 
 /* ---------------------------------------------------------------------------------------
+ * ml_steric_local_profile -- the area-weighted steric, thermosteric and halosteric height change by
+ * model level, from one pass over T and S:
+ *   prof_v[t][z] = neg_inv_rhozero * nansum_col( m * w * dz * delta_rho_v[t][z][col] )
+ * with delta_rho_v the anomaly of ml_delta_rho for variant v (steric.py:115-121, :151-153), dz the
+ * thickness of derived.calc_dz (derived.py:295-318, top=0, bottom=None), m = v_ref[0][col] present (the
+ * surface mask of steric.py:166) and w = weights[col] (a NaN weight counts as 0).  A NaN term (a hole at
+ * a wet cell, a missing reference volume) is skipped.  Summed over z this is nansum_col(w * eta) of
+ * ml_steric_local's height eta: dividing by nansum(w) is left to the caller.
+ * fp32 fields with 16-byte aligned rows (ncol % 4 == 0) stream through a shared-memory ring
+ * (csrc/ml_stream.cu); fp64 storage, ragged rows, a column pressure (ml_set_column_pressure) or
+ * ml_set_force_direct(1) take the plain-load kernel, which gives the same bits.  All the heights asked
+ * for come from one pass; each is bit-identical to a call that asks for it alone, and
+ * ml_set_force_direct(2) runs one launch per height (A/B).  Sums run in a fixed order: reproducible.
+ *   T, S          [nt][nz][ncol] of `dtype`
+ *   T_ref, S_ref  [nz][ncol] of `dtype`: reference["thetao"], reference["so"]
+ *   rho_ref       [nz][ncol] fp64: reference["rho"]
+ *   weights       [ncol] fp64 (device), e.g. areacello or areacello * basin mask
+ *   prof_*        [nt][nz] fp64 out each (device); a NULL pointer skips that variant; at least one is
+ *                 required (ML_ERR_NULL)
+ *   workspace     ml_profile_workspace_bytes(number of prof_* given, nt, nz, ncol) bytes
+ * Other arguments as ml_steric_local.  Every argument error returns before any launch.
+ * ------------------------------------------------------------------------------------- */
+size_t ml_profile_workspace_bytes(int nvariants, int64_t nt, int64_t nz, int64_t ncol);
+int ml_steric_local_profile(int eos, int dtype, const void* T, const void* S, const void* T_ref,
+                            const void* S_ref, const double* rho_ref, const void* v_ref,
+                            int vref_dtype, const double* z_i, const double* deptho,
+                            const double* weights, const double* p_level, double neg_inv_rhozero,
+                            int64_t nt, int64_t nz, int64_t ncol, double* prof_steric,
+                            double* prof_thermosteric, double* prof_halosteric, void* workspace,
+                            size_t ws_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------
  * ml_steric_global -- fused EOS -> sum_{z,col} rho * v_ref per time step.
  * Replaces calc_masso(rho, reference["volcello"]) in the global branch
  * (src/momlevel/steric.py:135, derived.py:435-438); the ln() formula (steric.py:136-142)

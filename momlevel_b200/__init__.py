@@ -11,9 +11,9 @@ reached through a C ABI; there is no CPU implementation in this package.
 from . import core, derived, distributed, dynamic, eos, reference, spice, test_data, util
 from .dynamic import inverse_barometer
 from .labeled import DataArray, Dataset
-from .steric import halosteric, steric, steric_layers, steric_variants, thermosteric
+from .steric import halosteric, steric, steric_layers, steric_profile, steric_variants, thermosteric
 
 __version__ = "0.1.0"
 
 __all__ = ["core", "derived", "distributed", "dynamic", "inverse_barometer", "eos", "reference", "spice", "test_data", "util", "DataArray", "Dataset",
-           "halosteric", "steric", "steric_layers", "steric_variants", "thermosteric"]
+           "halosteric", "steric", "steric_layers", "steric_profile", "steric_variants", "thermosteric"]

@@ -42,6 +42,9 @@ EXPORTS = {
                                     _vp]),
     "ml_steric_local_layers_variants": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _d, _vp, _i, _i64,
                                              _i64, _i64, _vp, _vp, _vp, _vp]),
+    "ml_profile_workspace_bytes": (_sz, [_i, _i64, _i64, _i64]),
+    "ml_steric_local_profile": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i64, _i64, _i64,
+                                     _vp, _vp, _vp, _vp, _sz, _vp]),
     "ml_delta_rho": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_delta_rho_annual": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_steric_local_selfref": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _d, _i64, _i64, _i64, _vp, _vp, _vp,

@@ -24,6 +24,7 @@ __all__ = [
     "steric_local_selfref",
     "steric_local_layers",
     "steric_local_layers_variants",
+    "steric_local_profile",
     "layer_edges",
     "delta_rho",
     "steric_global",
@@ -519,6 +520,45 @@ def steric_local_layers_variants(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho
                                               ptr("thermosteric"), ptr("halosteric"), _stream())
         )
     return eta
+
+
+def steric_local_profile(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho, p_level, weights, rhozero=1035.0,
+                         eos="Wright", variants=VARIANTS):
+    """The area-weighted height change of each level, ``-1/rhozero * nansum_col(m * w * dz * delta_rho) /
+    nansum(w)`` (steric.py:115-121, :151-166, derived.py:295-318), for the variants asked for.
+
+    ``T_ref, S_ref, rho_ref`` are the reference state (``reference["thetao"]``, ``["so"]``, ``["rho"]``); ``weights``
+    is one weight per column (``areacello``, or ``areacello`` times a basin mask; NaN counts as 0).  Returns
+    ``{variant: [nt, nz]}`` fp64 on the device, from one pass over T and S (``ml_steric_local_profile``).
+    """
+    L = _lib.lib()
+    names = variant_names(variants)
+    p_level, _pcol = _pressure_parts(p_level)
+    T, S, nt, nz, ncol, _ = _steric_operands(T, S, False, False)
+    Tr, Sr = to_device(T_ref), to_device(S_ref)
+    dt = _field_dtype(T, S, Tr, Sr)
+    T, S, Tr, Sr = T.to(dt), S.to(dt), Tr.to(dt), Sr.to(dt)
+    rho_ref = _f64(rho_ref)
+    v_ref = to_device(v_ref)
+    z_i, depth, p, w = _f64(z_i), _f64(deptho), _f64(p_level), _f64(weights)
+    assert Tr.numel() == nz * ncol and Sr.numel() == nz * ncol and rho_ref.numel() == nz * ncol
+    assert v_ref.numel() == nz * ncol and depth.numel() == ncol and z_i.numel() == nz + 1 and p.numel() == nz
+    if w.numel() != ncol:
+        raise ValueError(f"one weight per column: got {w.numel()} weights for {ncol} columns")
+    prof = {v: torch.empty((nt, nz), dtype=torch.float64, device=T.device) for v in names}
+    nbytes = L.ml_profile_workspace_bytes(len(names), nt, nz, ncol)
+    ws = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=T.device)
+    ptr = lambda v: prof[v].data_ptr() if v in prof else None  # noqa: E731
+    with _pcol:
+        _lib.check(
+            L.ml_steric_local_profile(_eos_id(eos), _dt_id(T), T.data_ptr(), S.data_ptr(), Tr.data_ptr(), Sr.data_ptr(),
+                                      rho_ref.data_ptr(), v_ref.data_ptr(), _dt_id(v_ref), z_i.data_ptr(),
+                                      depth.data_ptr(), w.data_ptr(), p.data_ptr(), -1.0 / rhozero, nt, nz, ncol,
+                                      ptr("steric"), ptr("thermosteric"), ptr("halosteric"), ws.data_ptr(), nbytes,
+                                      _stream())
+        )
+    total = torch.nansum(w)
+    return {v: prof[v] / total for v in names}
 
 
 def delta_rho(T, S, rho_ref, v_ref, p_level, eos="Wright", t_bcast=False, s_bcast=False):

@@ -485,6 +485,74 @@ __global__ void __launch_bounds__(kBlock)
   }
 }
 
+// ----------------------------------------------------------- K8 direct: level profile
+// ml_steric_local_profile on plain loads, for what the ring of k_stream_profile (ml_stream.cu) does not take: fp64
+// storage, rows that are not 16-byte aligned, a column pressure, ml_set_force_direct(1).  A block owns one (level,
+// kProfSeg-column segment) pair and walks every time step.  Point -> thread mapping (two quads per thread, kBlock
+// apart), the order of a thread's sum and the per-warp partial slots are those of k_stream_profile, so the two
+// families give the same bits.
+constexpr int kProfSeg = 2048;
+template <typename TIn, int EOS, int VM>
+__global__ void __launch_bounds__(kBlock)
+    k_profile_direct(const TIn* __restrict__ T, const TIn* __restrict__ S, const TIn* __restrict__ T_ref,
+                     const TIn* __restrict__ S_ref, const double* __restrict__ rho_ref, const void* __restrict__ v_ref,
+                     int v_f32, const double* __restrict__ z_i, const double* __restrict__ deptho,
+                     const double* __restrict__ weights, const double* __restrict__ p_level,
+                     const double* __restrict__ p_col, double coef, int nt, int nz, i64 ncol, double* part0,
+                     double* part1, double* part2) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const i64 col0 = (i64)blockIdx.x * kProfSeg;
+  const i64 nblk = (i64)gridDim.x * kWarps;
+  const i64 lvl = (i64)nz * ncol;
+  double* const part[3] = {part0, part1, part2};
+  Eos<EOS> eos;
+  for (int z = blockIdx.y; z < nz; z += gridDim.y) {
+    const double plev = __ldg(p_level + z);
+    const double ztop = __ldg(z_i + z), zbot = __ldg(z_i + z + 1);
+    double ref[8], cw[8], pz[8];
+    TIn tref[8], sref[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      const i64 c = col0 + 4 * (tid + (k >> 2) * kBlock) + (k & 3);
+      ref[k] = nan("");
+      cw[k] = 0.0;
+      pz[k] = plev;
+      tref[k] = sref[k] = TIn(0);
+      if (c < ncol) {
+        const i64 i = (i64)z * ncol + c;
+        double depth = __ldg(deptho + c);
+        if (isnan(depth)) depth = 0.0;  // derived.py:295
+        ref[k] = vref_wet(v_ref, v_f32, i) ? __ldg(rho_ref + i) : nan("");
+        cw[k] = profile_weight(vref_wet(v_ref, v_f32, c), __ldg(weights + c), clipped_dz(depth, ztop, zbot), coef);
+        if (p_col != nullptr) pz[k] = plev + __ldg(p_col + c);  // a 2-D patm (steric.py:96)
+        if (VM & 4) tref[k] = __ldg(T_ref + i);
+        if (VM & 2) sref[k] = __ldg(S_ref + i);
+      }
+    }
+    for (int t = 0; t < nt; ++t) {
+      double acc[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        const i64 c = col0 + 4 * (tid + (k >> 2) * kBlock) + (k & 3);
+        if (c < ncol) {
+          const i64 i = (i64)t * lvl + (i64)z * ncol + c;
+          const double Tv = (VM & 3) ? ldf(T + i) : 0.0, Sv = (VM & 5) ? ldf(S + i) : 0.0;
+          if (VM & 1) acc[0] = profile_add(acc[0], cw[k], eos.rho_at(Tv, Sv, pz[k]), ref[k]);
+          if (VM & 2) acc[1] = profile_add(acc[1], cw[k], eos.rho_at(Tv, (double)sref[k], pz[k]), ref[k]);
+          if (VM & 4) acc[2] = profile_add(acc[2], cw[k], eos.rho_at((double)tref[k], Sv, pz[k]), ref[k]);
+        }
+      }
+      const i64 slot = ((i64)t * nz + z) * nblk + (i64)blockIdx.x * kWarps + warp;
+#pragma unroll
+      for (int v = 0; v < 3; ++v)
+        if (VM & (1 << v)) {
+          const double w = warp_sum(acc[v]);
+          if (lane == 0) part[v][slot] = w;
+        }
+    }
+  }
+}
+
 // --------------------------------------------------------------------------- dispatch
 inline i64 cdiv(i64 a, i64 b) { return (a + b - 1) / b; }
 
@@ -585,6 +653,33 @@ int launch_global_direct(const void* T, const void* S, i64 ts, i64 ss, const voi
   if (rc) return rc;
   k_reduce_rows<<<nt, kBlock, 0, st>>>(partials, nblk, masso);
   return launched("k_reduce_rows");
+}
+
+template <typename TIn, int EOS>
+int launch_profile_direct(int vm, const void* T, const void* S, const void* T_ref, const void* S_ref,
+                          const double* rho_ref, const void* v_ref, int v_f32, const double* z_i, const double* deptho,
+                          const double* weights, const double* p_level, double coef, int nt, int nz, i64 ncol,
+                          double* const part[3], cudaStream_t st) {
+  const dim3 grid((unsigned)cdiv(ncol, kProfSeg), (unsigned)(nz < 65535 ? nz : 65535));
+#define ML_PROF_DIRECT(VM)                                                                                              \
+  case VM:                                                                                                              \
+    k_profile_direct<TIn, EOS, VM><<<grid, kBlock, 0, st>>>((const TIn*)T, (const TIn*)S, (const TIn*)T_ref,           \
+                                                            (const TIn*)S_ref, rho_ref, v_ref, v_f32, z_i, deptho,      \
+                                                            weights, p_level, tls().p_col, coef, nt, nz, ncol, part[0], \
+                                                            part[1], part[2]);                                          \
+    break
+  switch (vm) {
+    ML_PROF_DIRECT(1);
+    ML_PROF_DIRECT(2);
+    ML_PROF_DIRECT(3);
+    ML_PROF_DIRECT(4);
+    ML_PROF_DIRECT(5);
+    ML_PROF_DIRECT(6);
+    ML_PROF_DIRECT(7);
+    default: return fail(ML_ERR_MODE, "variant mask %d", vm);
+  }
+#undef ML_PROF_DIRECT
+  return launched("k_profile_direct");
 }
 
 namespace tma {
@@ -988,6 +1083,91 @@ int ml_steric_local_layers_variants(int eos, int dtype, const void* T, const voi
     if ((rc = ml_steric_local_layers(eos, dtype, v.T, v.S, v.t_bcast, v.s_bcast, rho_ref, v_ref, vref_dtype, z_i, deptho,
                                      p_level, neg_inv_rhozero, edges, nlayers, nt, nz, ncol, v.eta, stream)))
       return rc;
+  }
+  return ML_OK;
+}
+
+size_t ml_profile_workspace_bytes(int nvariants, int64_t nt, int64_t nz, int64_t ncol) {
+  nvariants = nvariants < 1 ? 1 : (nvariants > 3 ? 3 : nvariants);
+  if (nt < 1) nt = 1;
+  if (nz < 1) nz = 1;
+  const int64_t slots = stream::profile_slots(ncol > 0 ? ncol : 1);  // per-warp partials of one (step, level) row
+  return (size_t)(nvariants * nt * nz * slots) * sizeof(double) + 256;
+}
+
+int ml_steric_local_profile(int eos, int dtype, const void* T, const void* S, const void* T_ref, const void* S_ref,
+                            const double* rho_ref, const void* v_ref, int vref_dtype, const double* z_i,
+                            const double* deptho, const double* weights, const double* p_level,
+                            double neg_inv_rhozero, int64_t nt, int64_t nz, int64_t ncol, double* prof_steric,
+                            double* prof_thermosteric, double* prof_halosteric, void* workspace, size_t ws_bytes,
+                            void* stream) {
+  int rc = check_common(eos, dtype);
+  if (rc) return rc;
+  if (vref_dtype != ML_F32 && vref_dtype != ML_F64) return fail(ML_ERR_DTYPE, "unknown vref dtype id %d", vref_dtype);
+  ML_REQUIRE_PTR(T);
+  ML_REQUIRE_PTR(S);
+  ML_REQUIRE_PTR(T_ref);
+  ML_REQUIRE_PTR(S_ref);
+  ML_REQUIRE_PTR(rho_ref);
+  ML_REQUIRE_PTR(v_ref);
+  ML_REQUIRE_PTR(z_i);
+  ML_REQUIRE_PTR(deptho);
+  ML_REQUIRE_PTR(weights);
+  ML_REQUIRE_PTR(p_level);
+  double* const outs[3] = {prof_steric, prof_thermosteric, prof_halosteric};
+  const int wanted = (prof_steric != nullptr) + (prof_thermosteric != nullptr) + (prof_halosteric != nullptr);
+  if (wanted == 0) return fail(ML_ERR_NULL, "prof_steric, prof_thermosteric and prof_halosteric are all NULL");
+  if (nt < 0 || nz <= 0 || ncol <= 0 || nt > INT32_MAX || nz > INT32_MAX || nt * nz > INT32_MAX)
+    return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ncol=%lld", (long long)nt, (long long)nz, (long long)ncol);
+  if (int rcp = check_column_pressure(ncol)) return rcp;
+  if (workspace == nullptr || ws_bytes < ml_profile_workspace_bytes(wanted, nt, nz, ncol))
+    return fail(ML_ERR_WORKSPACE, "workspace needs %zu bytes, got %zu", ml_profile_workspace_bytes(wanted, nt, nz, ncol),
+                ws_bytes);
+  ML_REQUIRE_ALIGNED(workspace, 8);
+  ML_REQUIRE_ALIGNED(T, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(S, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(T_ref, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(S_ref, elem_size(dtype));
+  ML_REQUIRE_ALIGNED(v_ref, elem_size(vref_dtype));
+  if (nt == 0) return ML_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int v_f32 = vref_dtype == ML_F32;
+  // one region of per-warp partials per wanted variant, in the order steric, thermosteric, halosteric
+  const i64 nblk = stream::profile_slots(ncol);
+  double* part[3] = {nullptr, nullptr, nullptr};
+  int vm = 0;
+  for (int v = 0, r = 0; v < 3; ++v)
+    if (outs[v]) {
+      part[v] = static_cast<double*>(workspace) + (i64)r++ * nt * nz * nblk;
+      vm |= 1 << v;
+    }
+  // ml_set_force_direct(2): one launch per variant (A/B against the one pass)
+  const bool split = tls().force_direct == 2;
+  const bool ring = dtype == ML_F32 && !direct_only() && stream::eligible(T, S, nullptr, workspace, ncol);
+  tls().last_path = ring ? ML_PATH_TMA : ML_PATH_DIRECT;
+  for (int v = 0; v < 3; ++v) {
+    const int m = split ? (vm & (1 << v)) : (v == 0 ? vm : 0);
+    if (m == 0) continue;
+    double* const p[3] = {(m & 1) ? part[0] : nullptr, (m & 2) ? part[1] : nullptr, (m & 4) ? part[2] : nullptr};
+    if (ring)
+      rc = stream::launch_profile(eos, m, (const float*)T, (const float*)S, (const float*)T_ref, (const float*)S_ref,
+                                  rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, nz,
+                                  ncol, p, st);
+    else if (dtype == ML_F32)
+      rc = eos == ML_EOS_WRIGHT
+               ? launch_profile_direct<float, 0>(m, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, p, st)
+               : launch_profile_direct<float, 1>(m, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, p, st);
+    else
+      rc = eos == ML_EOS_WRIGHT
+               ? launch_profile_direct<double, 0>(m, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, p, st)
+               : launch_profile_direct<double, 1>(m, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, p, st);
+    if (rc) return rc;
+  }
+  // fixed-order second stage: one block per (step, level) row
+  for (int v = 0; v < 3; ++v) {
+    if (outs[v] == nullptr) continue;
+    k_reduce_rows<<<(unsigned)(nt * nz), kBlock, 0, st>>>(part[v], nblk, outs[v]);
+    if ((rc = launched("k_reduce_rows"))) return rc;
   }
   return ML_OK;
 }

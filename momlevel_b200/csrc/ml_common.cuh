@@ -254,4 +254,17 @@ __device__ __forceinline__ double clipped_dz(double depth, double ztop, double z
   return fmin(fmax(depth - ztop, 0.0), zbot - ztop);
 }
 
+// --------------------------------------------------------------------- level profile (ml_steric_local_profile)
+// Weight of one point in the area-weighted profile: coef * w * dz where the surface cell holds water (steric.py:166)
+// and the column weight is a number; 0 elsewhere (a NaN weight counts as 0).  Both kernel families form it here.
+__device__ __forceinline__ double profile_weight(bool surface_wet, double w, double dz, double coef) {
+  return (surface_wet && !isnan(w)) ? __dmul_rn(__dmul_rn(w, dz), coef) : 0.0;
+}
+// One term of a profile sum, skipna: d = rho - rho_ref is rounded on its own (no contraction into an FMA), so a point
+// at its reference state contributes exactly 0 and a NaN term (a hole, a missing reference volume) is skipped.
+__device__ __forceinline__ double profile_add(double acc, double cw, double rho, double rref) {
+  const double d = __dsub_rn(rho, rref);
+  return is_nan_q(d) ? acc : fma(cw, d, acc);
+}
+
 }  // namespace ml

@@ -324,6 +324,132 @@ __global__ void __launch_bounds__(kThreads, 2)
   }
 }
 
+// ------------------------------------------------------------------------------ level profile
+// The area-weighted steric / thermosteric / halosteric height change of each level (ml_steric_local_profile):
+// partials[v][t * nz + z][seg * kWarps + warp] = sum over the warp's points of cw * (rho_v - rho_ref), skipna, with
+// cw = coef * m * w * dz (profile_weight).  The (level, segment) ownership and time-fastest sequence of
+// k_stream_delta_rho: per pair, rho_ref (NaN where the reference volume is missing), cw and the reference slabs the
+// variants hold fixed stay in registers.  Per streamed step a thread sums its 8 points in a fixed order, the warp
+// sums by shuffle and lane 0 stores the warp's partial: no CTA-wide barrier in the loop, and a partial's slot depends
+// on the point's position only, so the sums do not depend on the grid.  VM: bit 0 steric (T, S), bit 1 thermosteric
+// (T, S_ref), bit 2 halosteric (T_ref, S) (steric.py:115-121); only the operands the variants read are staged.
+constexpr size_t kProfileRing = ring_bytes<2>();  // the per-point state follows the ring
+struct ProfileOut {
+  double* part[3];  // per variant, [nt * nz][tiles_per_row * kWarps]; NULL for a variant not asked for
+};
+
+template <int EOS, int VM>
+__global__ void __launch_bounds__(kThreads, 2)
+    k_stream_profile(const float* __restrict__ T, const float* __restrict__ S, const float* __restrict__ T_ref,
+                     const float* __restrict__ S_ref, const double* __restrict__ rho_ref, const void* __restrict__ v_ref,
+                     int v_f32, const double* __restrict__ z_i, const double* __restrict__ deptho,
+                     const double* __restrict__ weights, const double* __restrict__ p_level, double coef, int nt, Geom g,
+                     ProfileOut out) {
+  constexpr bool kT = (VM & 3) != 0, kS = (VM & 5) != 0;  // which of T, S the ring carries
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  Ring<2> ring;
+  ring.init(smem_raw);
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  // per-pair state of a thread's 8 points, [point][thread]: only the owning thread reads its slots, so no barrier
+  double* const ref = reinterpret_cast<double*>(smem_raw + kProfileRing) + tid;
+  double* const cw = ref + 8 * kThreads;
+  // the reference slabs the variants hold fixed
+  float* const tref = reinterpret_cast<float*>(smem_raw + kProfileRing + 16 * kThreads * sizeof(double)) + tid;
+  float* const sref = tref + 8 * kThreads;
+  const i64 npairs = g.ntiles;
+  const i64 mine = npairs > (i64)blockIdx.x ? (npairs - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+  const i64 nseq = mine * nt;
+  const i64 lvl = (i64)g.nz * g.ncol;
+  const i64 nblk = (i64)g.tiles_per_row * kWarps;
+  auto issue = [&](i64 q, int s) {
+    const i64 pair = (i64)blockIdx.x + (q / nt) * gridDim.x;
+    const int t = (int)(q % nt);
+    const i64 row = pair / g.tiles_per_row;
+    const i64 col0 = (pair - row * g.tiles_per_row) * kTile;
+    const i64 len = g.ncol - col0 < kTile ? g.ncol - col0 : kTile;
+    const uint32_t bytes = (uint32_t)len * 4u;
+    const i64 off = (i64)t * lvl + row * g.ncol + col0;
+    tma::mbar_expect_tx(ring.full + s, (kT + kS) * bytes);
+    if (kT) bulk_load(ring.stage(s, 0), T + off, bytes, ring.full + s);
+    if (kS) bulk_load(ring.stage(s, 1), S + off, bytes, ring.full + s);
+  };
+  __syncthreads();
+  if (tid == 0)
+    for (int s = 0; s < kStages && s < nseq; ++s) issue(s, s);
+  Eos<EOS> eos;
+  i64 q = 0;
+  for (i64 i = 0; i < mine; ++i) {
+    const i64 pair = (i64)blockIdx.x + i * gridDim.x;
+    const i64 row = pair / g.tiles_per_row;
+    const i64 seg = pair - row * g.tiles_per_row;
+    const i64 col0 = seg * kTile;
+    const i64 len = g.ncol - col0 < kTile ? g.ncol - col0 : kTile;
+    const i64 off = row * g.ncol + col0;
+    eos.set_level(__ldg(p_level + row));
+    const double ztop = __ldg(z_i + row), zbot = __ldg(z_i + row + 1);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int qd = tid + h * kThreads;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        ref[(4 * h + j) * kThreads] = nan("");
+        cw[(4 * h + j) * kThreads] = 0.0;
+        tref[(4 * h + j) * kThreads] = sref[(4 * h + j) * kThreads] = 0.0f;
+      }
+      if (4 * qd < len) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const i64 c = col0 + 4 * qd + j;
+          const bool wet = v_f32 ? !isnan(__ldg(reinterpret_cast<const float*>(v_ref) + off + 4 * qd + j))
+                                 : !isnan(__ldg(reinterpret_cast<const double*>(v_ref) + off + 4 * qd + j));
+          const bool top = v_f32 ? !isnan(__ldg(reinterpret_cast<const float*>(v_ref) + c))
+                                 : !isnan(__ldg(reinterpret_cast<const double*>(v_ref) + c));
+          double depth = __ldg(deptho + c);
+          if (isnan(depth)) depth = 0.0;  // derived.py:295
+          ref[(4 * h + j) * kThreads] = wet ? __ldg(rho_ref + off + 4 * qd + j) : nan("");
+          cw[(4 * h + j) * kThreads] = profile_weight(top, __ldg(weights + c), clipped_dz(depth, ztop, zbot), coef);
+          if (VM & 4) tref[(4 * h + j) * kThreads] = __ldg(T_ref + off + 4 * qd + j);
+          if (VM & 2) sref[(4 * h + j) * kThreads] = __ldg(S_ref + off + 4 * qd + j);
+        }
+      }
+    }
+    for (int t = 0; t < nt; ++t, ++q) {
+      const int s = (int)(q % kStages);
+      tma::mbar_wait(ring.full + s, (uint32_t)(q / kStages) & 1u);
+      const float4* sT = reinterpret_cast<const float4*>(ring.stage(s, 0));
+      const float4* sS = reinterpret_cast<const float4*>(ring.stage(s, 1));
+      double acc[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int qd = tid + h * kThreads;
+        if (4 * qd < len) {
+          float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
+          if (kT) a = sT[qd];
+          if (kS) b = sS[qd];
+          const float ta[4] = {a.x, a.y, a.z, a.w}, sa[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            if (VM & 1) acc[0] = profile_add(acc[0], cw[(4 * h + j) * kThreads], eos.rho((double)ta[j], (double)sa[j]), ref[(4 * h + j) * kThreads]);
+            if (VM & 2) acc[1] = profile_add(acc[1], cw[(4 * h + j) * kThreads], eos.rho((double)ta[j], (double)sref[(4 * h + j) * kThreads]), ref[(4 * h + j) * kThreads]);
+            if (VM & 4) acc[2] = profile_add(acc[2], cw[(4 * h + j) * kThreads], eos.rho((double)tref[(4 * h + j) * kThreads], (double)sa[j]), ref[(4 * h + j) * kThreads]);
+          }
+        }
+      }
+      if (last_to_leave(ring.empty + s, ring.released + s, (uint32_t)(q / kStages) & 1u)) {
+        const i64 next = q + kStages;
+        if (next < nseq) issue(next, s);
+      }
+      const i64 slot = ((i64)t * g.nz + row) * nblk + seg * kWarps + warp;
+#pragma unroll
+      for (int v = 0; v < 3; ++v)
+        if (VM & (1 << v)) {
+          const double w = warp_sum(acc[v]);
+          if (lane == 0) out.part[v][slot] = w;
+        }
+    }
+  }
+}
+
 // ----------------------------------------------------------------------- host side
 static Geom geometry(i64 nrows, int nz, i64 ncol) {
   Geom g;
@@ -417,6 +543,53 @@ int launch_delta_rho(int eos, const float* T, const float* S, i64 t_stride, i64 
   }
 #undef ML_STREAM_DRHO
   return launched("k_stream_delta_rho");
+}
+
+constexpr size_t profile_smem_bytes() { return kProfileRing + 2 * kTile * (sizeof(double) + sizeof(float)); }
+
+int profile_slots(i64 ncol) { return (int)((ncol + kTile - 1) / kTile) * kWarps; }
+
+template <int EOS, int VM>
+static int launch_profile_vm(const float* T, const float* S, const float* T_ref, const float* S_ref,
+                             const double* rho_ref, const void* v_ref, int v_f32, const double* z_i,
+                             const double* deptho, const double* weights, const double* p_level, double coef, int nt,
+                             const Geom& g, const ProfileOut& out, cudaStream_t st) {
+  auto kern = k_stream_profile<EOS, VM>;
+  if (int rc = opt_in(kern, profile_smem_bytes())) return rc;
+  kern<<<persistent_grid(g.ntiles, 2), kThreads, profile_smem_bytes(), st>>>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i,
+                                                                         deptho, weights, p_level, coef, nt, g, out);
+  return launched("k_stream_profile");
+}
+
+template <int EOS>
+static int launch_profile_eos(int vm, const float* T, const float* S, const float* T_ref, const float* S_ref,
+                              const double* rho_ref, const void* v_ref, int v_f32, const double* z_i,
+                              const double* deptho, const double* weights, const double* p_level, double coef, int nt,
+                              const Geom& g, const ProfileOut& out, cudaStream_t st) {
+#define ML_STREAM_PROF(VM) \
+  case VM: return launch_profile_vm<EOS, VM>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, coef, nt, g, out, st)
+  switch (vm) {
+    ML_STREAM_PROF(1);
+    ML_STREAM_PROF(2);
+    ML_STREAM_PROF(3);
+    ML_STREAM_PROF(4);
+    ML_STREAM_PROF(5);
+    ML_STREAM_PROF(6);
+    ML_STREAM_PROF(7);
+  }
+#undef ML_STREAM_PROF
+  return fail(ML_ERR_MODE, "variant mask %d", vm);
+}
+
+int launch_profile(int eos, int vm, const float* T, const float* S, const float* T_ref, const float* S_ref,
+                   const double* rho_ref, const void* v_ref, int v_f32, const double* z_i, const double* deptho,
+                   const double* weights, const double* p_level, double coef, int nt, i64 nz, i64 ncol,
+                   double* const part[3], cudaStream_t st) {
+  const Geom g = geometry(nz, (int)nz, ncol);
+  const ProfileOut out = {{part[0], part[1], part[2]}};
+  if (eos == ML_EOS_WRIGHT)
+    return launch_profile_eos<0>(vm, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, coef, nt, g, out, st);
+  return launch_profile_eos<1>(vm, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, coef, nt, g, out, st);
 }
 
 }  // namespace stream

@@ -17,7 +17,7 @@ from .labeled import ChunkedArray, DataArray, Dataset
 from .reference import _pressure, setup_reference_state
 from .util import annual_average, calendar_axis, default_coords, validate_dataset, whole_years_in_order
 
-__all__ = ["halosteric", "steric", "steric_layers", "steric_variants", "thermosteric"]
+__all__ = ["halosteric", "steric", "steric_layers", "steric_profile", "steric_variants", "thermosteric"]
 
 
 def steric(
@@ -873,6 +873,98 @@ def steric_layers(dset, depth_edges=(0.0, 700.0, 2000.0, None), reference=None, 
         "long_name": "Top of depth layer", "units": "m"})
     result["layer_bottom"] = DataArray(edges[1:].copy(), ("depth_layer",), attrs={
         "long_name": "Bottom of depth layer (inf: the sea floor)", "units": "m"})
+    for var in set(result.dims):
+        if var in dset.variables:
+            coord = dset[var].copy(deep=False)
+            coord.attrs = dict(dset[var].attrs)
+            result[var] = coord
+    if annual:  # steric.py:181-182
+        result = annual_average(result, tcoord=tcoord, days_in_month=days_in_month)
+    if xarray_in:
+        return xarray_io.to_xarray(result, like=dset_x), xarray_io.to_xarray(reference, like=dset_x)
+    return (result, reference)
+
+
+def steric_profile(dset, variant="steric", reference=None, weights=None, coord_names=None, varname_map=None,
+                   rhozero=1035.0, patm=101325.0, equation_of_state="Wright", dtype="float32", strict=True, annual=False,
+                   days_in_month=None, verbose=False):
+    """How much each model level contributes to the area-weighted mean steric, thermosteric or halosteric sea level
+    change, per time step, from one pass over T and S (a depth-time Hovmoeller of the expansion; summed over the
+    levels below a depth, that depth's deep contribution).
+
+    ``profile[t, z] = -1/rhozero * nansum_col(m * w * dz * delta_rho[t, z]) / nansum_col(w)`` with ``delta_rho`` the
+    anomaly of :func:`steric` for the variant, ``dz`` from ``calc_dz`` (derived.py:249-325), ``m`` the surface mask of
+    the reference volume (steric.py:166) and ``w`` the column weights: ``weights`` (a ``(y, x)`` array, for example
+    ``areacello * atlantic_mask`` for a basin profile), ``areacello`` by default; a NaN weight counts as 0.  A NaN term
+    (a hole at a wet cell) is skipped.  Summed over the levels it is the ``w``-weighted mean of :func:`steric`'s local
+    height, ``nansum(w * eta) / nansum(w)``.  It is not the global series of ``steric(domain="global")``,
+    ``href * ln(rho0 / rho)``, which differs from that mean at second order.
+
+    ``variant`` is a name or a list or tuple of distinct names from ``("steric", "thermosteric", "halosteric")``: a list
+    moves T and S to the device once and one pass gives every profile asked for, each the one a call with that name
+    alone returns, bit for bit.  The remaining arguments are those of :func:`steric` with ``domain="local"``;
+    ``reference=None`` builds the reference state from the first step first.  Chunked (dask-backed) fields raise
+    ``NotImplementedError``.
+
+    Returns ``(result, reference)``: ``result[name]`` has dims ``(time, z_l)``.
+    """
+    names = core.variant_names(variant)
+    xarray_in = type(dset).__module__.startswith("xarray")
+    if xarray_in:
+        from . import xarray_io
+
+        dset_x = dset
+        t_, z_, zb_ = default_coords(coord_names)
+        needed = {"thetao", "so", "volcello", "areacello", "deptho", t_, z_, zb_}
+        needed |= {k for k, v in (varname_map or {}).items() if v in needed}
+        dset = xarray_io.from_xarray(dset, names=sorted(needed))
+        if reference is not None:
+            assert type(reference).__module__.startswith("xarray"), "`reference` must be an xarray Dataset"
+            reference = xarray_io.from_xarray(reference)
+
+    # steric.py:84-91
+    dset = dset.rename(varname_map)
+    tcoord, zcoord, zbounds = default_coords(coord_names)
+    if _chunked(dset):
+        raise NotImplementedError("steric_profile takes device-resident or in-memory fields; chunked (dask-backed) "
+                                  "fields are not supported yet")
+    validate_dataset(dset, strict=strict, additional_vars=[zbounds, "deptho"])
+    full = dset["thetao"]
+    if full.dims[0] != tcoord or full.dims[1] != zcoord or dset["so"].dims != full.dims:
+        raise ValueError(f"expecting fields laid out ({tcoord}, {zcoord}, y, x), got {full.dims}")
+    if weights is None:
+        w = dset["areacello"].data
+    else:
+        w = weights.data if isinstance(weights, DataArray) else weights
+        if type(w).__module__.startswith("xarray"):
+            w = w.values
+        if not isinstance(w, torch.Tensor):
+            w = np.asarray(w, dtype=np.float64)
+    if tuple(w.shape) != tuple(full.shape[2:]):
+        raise ValueError(f"weights of shape {tuple(w.shape)} do not match the horizontal grid {tuple(full.shape[2:])}")
+    pres = _pressure(dset, zcoord, patm)  # steric.py:96
+
+    # steric.py:98-112
+    if reference is not None:
+        assert isinstance(reference, Dataset), "`reference` must be an xarray Dataset"
+        if verbose:
+            print("Using supplied reference state")
+    else:
+        reference = setup_reference_state(dset, patm=patm, eos=equation_of_state, coord_names=coord_names)
+        if verbose:
+            print("Generating reference state from first timestep")
+    validate_dataset(reference, reference=True, strict=strict)
+
+    _check_depths(dset, zcoord, zbounds)
+    profs = core.steric_local_profile(full.data, dset["so"].data, reference["thetao"].data, reference["so"].data,
+                                      reference["rho"].data, reference["volcello"].data, dset[zbounds].data,
+                                      dset["deptho"].data, pres, w, rhozero=rhozero, eos=equation_of_state,
+                                      variants=names)
+    result = Dataset()
+    for name in names:
+        result[name] = DataArray(profs[name], (tcoord, zcoord), attrs={
+            "long_name": f"{name.capitalize()} height adjustment by level, area-weighted mean", "units": "m"})
+        result[name].encoding["dtype"] = dtype
     for var in set(result.dims):
         if var in dset.variables:
             coord = dset[var].copy(deep=False)
