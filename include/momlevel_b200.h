@@ -106,7 +106,8 @@ int ml_eos_eval(int eos, int func, int dtype, const void* T, const void* S, int 
 /* ---------------------------------------------------------------------------------------
  * ml_flament_spice -- Flament (2002) spiciness, elementwise, fp64 out.
  * Replaces spice.flament.spice (src/momlevel/spice/flament.py:43-95) as applied by
- * derived.calc_spice (src/momlevel/derived.py:669-711).
+ * derived.calc_spice (src/momlevel/derived.py:669-711).  A point with an infinite or NaN
+ * T or S, or whose powers overflow, is NaN, as in the reference (its power-table sum meets inf - inf).
  * ------------------------------------------------------------------------------------- */
 int ml_flament_spice(int dtype, const void* T, const void* S, int64_t n, double* out,
                      void* stream);
@@ -348,6 +349,8 @@ int ml_steric_global_variants(int eos, int dtype, const void* T, const void* S, 
  * `volcello.sum()`, the field passed as `rho` with nrows = 1).  Two fixed-order stages: bitwise reproducible.
  *   rho        device [nrows][n] of `dtype`;  volcello device [n] of `w_dtype` or NULL
  *   out        device fp64[nrows];  workspace: nrows * 1184 doubles are always enough
+ *   nrows      any count up to INT32_MAX: more than 65535 rows (a time axis of 3-hourly output over 23 years)
+ *              are launched in chunks of 65535; a row's result does not depend on nrows or on its chunk.
  * ------------------------------------------------------------------------------------- */
 int ml_calc_masso(int dtype, const void* rho, int w_dtype, const void* volcello, int64_t nrows, int64_t n,
                   double* out, void* workspace, size_t workspace_bytes, void* stream);

@@ -781,7 +781,9 @@ int ml_flament_spice(int dtype, const void* T, const void* S, int64_t n, double*
   const int es = elem_size(dtype);
   i64 done = 0;
   const bool aligned = ((reinterpret_cast<uintptr_t>(T) | reinterpret_cast<uintptr_t>(S) | reinterpret_cast<uintptr_t>(out)) & 15u) == 0;
-  if (aligned && dtype == ML_F32 && n >= 4 && n % 4 == 0 && tls().force_direct != 1)  // ring-staged streaming kernel (ml_stream.cu)
+  // ring-staged streaming kernel (ml_stream.cu); its 256-bit result stores need `out` on 32 bytes, which a caller's
+  // `out` tensor 16 bytes into its buffer is not -- that one takes k_spice_vec
+  if (dtype == ML_F32 && tls().force_direct != 1 && stream::eligible(T, S, nullptr, out, n))
     return stream::launch_spice((const float*)T, (const float*)S, n, out, st);
   if (aligned && n >= 4) {
     const i64 n4 = n / 4;
@@ -1451,7 +1453,7 @@ int ml_calc_masso(int dtype, const void* rho, int w_dtype, const void* volcello,
   if (volcello != nullptr && w_dtype != ML_F32 && w_dtype != ML_F64) return fail(ML_ERR_DTYPE, "unknown weight dtype id %d", w_dtype);
   ML_REQUIRE_PTR(rho);
   ML_REQUIRE_PTR(out);
-  if (nrows < 0 || n < 0 || nrows > 65535) return fail(ML_ERR_SHAPE, "bad extents nrows=%lld n=%lld", (long long)nrows, (long long)n);
+  if (nrows < 0 || n < 0 || nrows > INT32_MAX) return fail(ML_ERR_SHAPE, "bad extents nrows=%lld n=%lld", (long long)nrows, (long long)n);
   if (nrows == 0) return ML_OK;
   ML_REQUIRE_ALIGNED(rho, elem_size(dtype));
   const i64 want = cdiv(n > 0 ? n : 1, (i64)kBlock * 8);
@@ -1461,16 +1463,24 @@ int ml_calc_masso(int dtype, const void* rho, int w_dtype, const void* volcello,
   ML_REQUIRE_ALIGNED(workspace, 8);
   cudaStream_t st = (cudaStream_t)stream;
   double* partials = (double*)workspace;
-  dim3 grid((unsigned)nblk, (unsigned)nrows);
-#define ML_WNS(TA, TW) k_weighted_nansum<TA, TW><<<grid, kBlock, 0, st>>>((const TA*)rho, (const TW*)volcello, n, partials)
-  if (dtype == ML_F32) {
-    if (volcello == nullptr || w_dtype == ML_F32) ML_WNS(float, float); else ML_WNS(float, double);
-  } else {
-    if (volcello == nullptr || w_dtype == ML_F64) ML_WNS(double, double); else ML_WNS(double, float);
-  }
+  // rows run on grid.y, at most 65535 per launch: a longer series (3-hourly output over 23 years has 67160 steps) is
+  // launched in chunks with the pointers moved to each chunk's first row.  The partials keep their [row][nblk] layout,
+  // so a row's bits depend neither on its chunk nor on nrows.
+  const int es = elem_size(dtype);
+  for (i64 r0 = 0; r0 < nrows; r0 += 65535) {
+    const i64 rows = nrows - r0 < 65535 ? nrows - r0 : 65535;
+    const void* a = (const char*)rho + r0 * n * es;
+    double* part = partials + r0 * nblk;
+    dim3 grid((unsigned)nblk, (unsigned)rows);
+#define ML_WNS(TA, TW) k_weighted_nansum<TA, TW><<<grid, kBlock, 0, st>>>((const TA*)a, (const TW*)volcello, n, part)
+    if (dtype == ML_F32) {
+      if (volcello == nullptr || w_dtype == ML_F32) ML_WNS(float, float); else ML_WNS(float, double);
+    } else {
+      if (volcello == nullptr || w_dtype == ML_F64) ML_WNS(double, double); else ML_WNS(double, float);
+    }
 #undef ML_WNS
-  int rc = launched("k_weighted_nansum");
-  if (rc) return rc;
+    if (int rc = launched("k_weighted_nansum")) return rc;
+  }
   k_reduce_rows<<<(unsigned)nrows, kBlock, 0, st>>>(partials, nblk, out);
   return launched("k_reduce_rows");
 }

@@ -213,6 +213,10 @@ __device__ __forceinline__ double eos_func(double T, double S, double p) {
 // -------------------------------------------------------------------------------- spice
 // Flament (2002), flament.py:7-40: pi = sum_ij b_ij T^i s^j, s = S - 35.
 // Inner Horner in s for each power of T, outer Horner in T: 24 + 5 DFMA + 1 DADD.
+// A result that is not finite is NaN, as in the reference's sum of power-table terms (flament.py:82-90): an infinite
+// T or S, or a power that overflows, meets coefficients of both signs there (inf - inf), where the nested form alone
+// would return +-inf.  Finite inputs in range never give an infinite result, so the test is on the result: one
+// exponent-bit test on the integer pipe and a select, no branch and no extra fp64 work.
 __device__ __forceinline__ double flament_spice(double T, double S) {
   const double s = S - 35.0;
   const double r0 = s * fma(s, fma(s, fma(s, -2.06e-4, -9.84e-4), -5.85e-3), 7.7442e-1);
@@ -221,7 +225,8 @@ __device__ __forceinline__ double flament_spice(double T, double S) {
   const double r3 = fma(s, fma(s, fma(s, fma(s, -1.0853e-6, -3.0412e-6), 7.0036e-6), 7.326e-6), -5.4023e-5);
   const double r4 = fma(s, fma(s, fma(s, fma(s, 4.7133e-8, 1.0012e-7), -3.8209e-7), -3.029e-8), 3.949e-7);
   const double r5 = fma(s, fma(s, fma(s, fma(s, -6.676e-10, -1.1409e-9), 6.048e-9), -1.309e-9), -6.36e-10);
-  return fma(T, fma(T, fma(T, fma(T, fma(T, r5, r4), r3), r2), r1), r0);
+  const double r = fma(T, fma(T, fma(T, fma(T, fma(T, r5, r4), r3), r2), r1), r0);
+  return (__double2hiint(r) & 0x7ff00000) == 0x7ff00000 ? __longlong_as_double(0x7ff8000000000000ll) : r;
 }
 
 // --------------------------------------------------------------------------- reductions

@@ -93,6 +93,23 @@ def test_fill_mode_is_checked_before_any_launch():
     assert L.ml_launch_count() == before
 
 
+def test_calc_masso_takes_more_than_65535_rows():
+    """More rows than one grid.y are launched in chunks: 65536 rows now reach the workspace check (8 bytes are far
+    too few) instead of a shape error; a negative row count is still a shape error.  Neither launches anything."""
+    from momlevel_b200 import _lib
+
+    L = _lib.lib()
+    buf = (ctypes.c_double * 8)()
+    p = ctypes.cast(buf, ctypes.c_void_p)
+    before = L.ml_launch_count()
+    for dtype in (0, 1):
+        assert L.ml_calc_masso(dtype, p, 1, p, 65536, 4, p, p, 8, None) == -6
+        assert b"workspace" in L.ml_last_error()
+        assert L.ml_calc_masso(dtype, p, 0, None, 70001, 1, p, p, 70001 * 8 - 8, None) == -6
+        assert L.ml_calc_masso(dtype, p, 1, p, -1, 4, p, p, 8, None) == -2
+    assert L.ml_launch_count() == before
+
+
 def test_no_product_import_of_the_oracle():
     """The product must never route through the oracle (test infrastructure only)."""
     for path in (ROOT / "momlevel_b200").rglob("*.py"):
