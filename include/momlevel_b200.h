@@ -306,6 +306,35 @@ int ml_steric_local_profile(int eos, int dtype, const void* T, const void* S, co
                             size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------
+ * ml_steric_local_region_profile -- ml_steric_local_profile for every region of a region map at once
+ * (basins side by side), from one pass over T and S:
+ *   prof_v[r][t][z] = neg_inv_rhozero * nansum_{col: region[col] == r}( m * w * dz * delta_rho_v[t][z][col] )
+ * Region r is exactly what ml_steric_local_profile gives with weights where(region == r, w, 0), and a map that
+ * puts every column in region 0 gives exactly its one-region result.  Every density is evaluated once per step
+ * whatever the number of regions; a warp of 32 x 8 columns spread over many regions sums once per region it
+ * touches.  Routes and switches are those of ml_steric_local_profile (the ring for eligible fp32 fields, the
+ * plain-load kernel with the same bits otherwise, ml_set_force_direct(2) one launch per variant).
+ *   region        [ncol] int8 (device): the region index of each column, in [0, nregions); any other value
+ *                 (e.g. -1) puts the column in no region.  NULL returns ML_ERR_NULL.
+ *   nregions      1 <= nregions <= ML_MAX_REGIONS; anything else returns ML_ERR_SHAPE
+ *   prof_*        [nregions][nt][nz] fp64 out each (device): numerators only, the caller divides by each
+ *                 region's nansum(w); a NULL pointer skips that variant; at least one is required (ML_ERR_NULL)
+ *   workspace     at least one step: ml_region_profile_workspace_bytes(number of prof_* given, nregions, 1, nz,
+ *                 ncol) bytes (ML_ERR_WORKSPACE otherwise).  The time axis runs in chunks of as many steps as
+ *                 the workspace holds; the bits of a step do not depend on the chunks.
+ * Other arguments as ml_steric_local_profile.  Every argument error returns before any launch.
+ * ------------------------------------------------------------------------------------- */
+#define ML_MAX_REGIONS 15
+size_t ml_region_profile_workspace_bytes(int nvariants, int nregions, int64_t nt, int64_t nz, int64_t ncol);
+int ml_steric_local_region_profile(int eos, int dtype, const void* T, const void* S, const void* T_ref,
+                                   const void* S_ref, const double* rho_ref, const void* v_ref, int vref_dtype,
+                                   const double* z_i, const double* deptho, const double* weights,
+                                   const int8_t* region, int nregions, const double* p_level,
+                                   double neg_inv_rhozero, int64_t nt, int64_t nz, int64_t ncol,
+                                   double* prof_steric, double* prof_thermosteric, double* prof_halosteric,
+                                   void* workspace, size_t ws_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------
  * ml_steric_global -- fused EOS -> sum_{z,col} rho * v_ref per time step.
  * Replaces calc_masso(rho, reference["volcello"]) in the global branch
  * (src/momlevel/steric.py:135, derived.py:435-438); the ln() formula (steric.py:136-142)

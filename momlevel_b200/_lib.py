@@ -11,7 +11,8 @@ import pathlib
 from . import _build
 
 __all__ = ["lib", "check", "MLError", "F32", "F64", "EOS_IDS", "FUNC_IDS", "P_SCALAR", "P_PER_LEVEL", "P_FULL",
-           "PATH_DIRECT", "PATH_TMA", "MAX_LAYERS", "EXPORTS"]
+           "PATH_DIRECT", "PATH_TMA", "MAX_LAYERS", "MAX_REGIONS",
+           "EXPORTS"]
 
 F32, F64 = 0, 1
 EOS_IDS = {"wright": 0, "linear": 1}
@@ -20,6 +21,7 @@ P_SCALAR, P_PER_LEVEL, P_FULL = 0, 1, 2
 DOMAIN_LOCAL, DOMAIN_GLOBAL = 0, 1
 PATH_DIRECT, PATH_TMA = 1, 2
 MAX_LAYERS = 8  # ML_MAX_LAYERS
+MAX_REGIONS = 15  # ML_MAX_REGIONS
 
 _vp, _i, _i64, _d, _sz = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double, ctypes.c_size_t
 
@@ -45,6 +47,9 @@ EXPORTS = {
     "ml_profile_workspace_bytes": (_sz, [_i, _i64, _i64, _i64]),
     "ml_steric_local_profile": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i64, _i64, _i64,
                                      _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ml_region_profile_workspace_bytes": (_sz, [_i, _i, _i64, _i64, _i64]),
+    "ml_steric_local_region_profile": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _d, _i64,
+                                            _i64, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ml_delta_rho": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_delta_rho_annual": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_steric_local_selfref": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _d, _i64, _i64, _i64, _vp, _vp, _vp,

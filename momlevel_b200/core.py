@@ -25,6 +25,7 @@ __all__ = [
     "steric_local_layers",
     "steric_local_layers_variants",
     "steric_local_profile",
+    "steric_local_region_profile",
     "layer_edges",
     "delta_rho",
     "steric_global",
@@ -559,6 +560,60 @@ def steric_local_profile(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho, p_leve
         )
     total = torch.nansum(w)
     return {v: prof[v] / total for v in names}
+
+
+REGION_WORKSPACE_BYTES = 512 << 20  # the most steric_local_region_profile allocates for partials; the time axis is chunked
+
+
+def steric_local_region_profile(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho, p_level, weights, region_index,
+                                nregions, rhozero=1035.0, eos="Wright", variants=VARIANTS):
+    """:func:`steric_local_profile` for every region of a region map, from one pass over T and S
+    (``ml_steric_local_region_profile``).
+
+    ``region_index`` holds one integer per column: in ``[0, nregions)`` the column's region, any other value (e.g.
+    -1) no region; ``1 <= nregions <= 15``.  Region ``r`` is, bit for bit, :func:`steric_local_profile` with
+    ``weights=where(region_index == r, weights, 0)``.  Returns ``({variant: [nregions, nt, nz]}, totals[nregions])``
+    fp64 on the device: the profiles already divided by ``totals``, each region's ``nansum`` of the weights (0/0,
+    NaN, for a region without columns).
+    """
+    L = _lib.lib()
+    names = variant_names(variants)
+    p_level, _pcol = _pressure_parts(p_level)
+    T, S, nt, nz, ncol, _ = _steric_operands(T, S, False, False)
+    Tr, Sr = to_device(T_ref), to_device(S_ref)
+    dt = _field_dtype(T, S, Tr, Sr)
+    T, S, Tr, Sr = T.to(dt), S.to(dt), Tr.to(dt), Sr.to(dt)
+    rho_ref = _f64(rho_ref)
+    v_ref = to_device(v_ref)
+    z_i, depth, p, w = _f64(z_i), _f64(deptho), _f64(p_level), _f64(weights)
+    assert Tr.numel() == nz * ncol and Sr.numel() == nz * ncol and rho_ref.numel() == nz * ncol
+    assert v_ref.numel() == nz * ncol and depth.numel() == ncol and z_i.numel() == nz + 1 and p.numel() == nz
+    if w.numel() != ncol:
+        raise ValueError(f"one weight per column: got {w.numel()} weights for {ncol} columns")
+    nregions = int(nregions)
+    if not 1 <= nregions <= _lib.MAX_REGIONS:
+        raise ValueError(f"nregions={nregions}: between 1 and {_lib.MAX_REGIONS} regions")
+    ri = torch.as_tensor(region_index, device=T.device)
+    if ri.numel() != ncol:
+        raise ValueError(f"one region index per column: got {ri.numel()} for {ncol} columns")
+    ri = torch.where((ri >= 0) & (ri < nregions), ri, -1).to(torch.int8).reshape(w.shape).contiguous()
+    prof = {v: torch.empty((nregions, nt, nz), dtype=torch.float64, device=T.device) for v in names}
+    step = L.ml_region_profile_workspace_bytes(len(names), nregions, 1, nz, ncol) - 256
+    steps = max(1, min(nt, (REGION_WORKSPACE_BYTES - 256) // step))
+    nbytes = L.ml_region_profile_workspace_bytes(len(names), nregions, steps, nz, ncol)
+    ws = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=T.device)
+    ptr = lambda v: prof[v].data_ptr() if v in prof else None  # noqa: E731
+    with _pcol:
+        _lib.check(
+            L.ml_steric_local_region_profile(_eos_id(eos), _dt_id(T), T.data_ptr(), S.data_ptr(), Tr.data_ptr(),
+                                             Sr.data_ptr(), rho_ref.data_ptr(), v_ref.data_ptr(), _dt_id(v_ref),
+                                             z_i.data_ptr(), depth.data_ptr(), w.data_ptr(), ri.data_ptr(), nregions,
+                                             p.data_ptr(), -1.0 / rhozero, nt, nz, ncol, ptr("steric"),
+                                             ptr("thermosteric"), ptr("halosteric"), ws.data_ptr(), nbytes, _stream())
+        )
+    # each total as steric_local_profile forms it from the masked weights, so that the quotients match bit for bit
+    totals = torch.stack([torch.nansum(torch.where(ri == r, w, 0.0)) for r in range(nregions)])
+    return {v: prof[v] / totals[:, None, None] for v in names}, totals
 
 
 def delta_rho(T, S, rho_ref, v_ref, p_level, eos="Wright", t_bcast=False, s_bcast=False):

@@ -490,16 +490,17 @@ __global__ void __launch_bounds__(kBlock)
 // storage, rows that are not 16-byte aligned, a column pressure, ml_set_force_direct(1).  A block owns one (level,
 // kProfSeg-column segment) pair and walks every time step.  Point -> thread mapping (two quads per thread, kBlock
 // apart), the order of a thread's sum and the per-warp partial slots are those of k_stream_profile, so the two
-// families give the same bits.
+// families give the same bits; so does REG, the region mode of k_stream_profile (one partial per region,
+// [nregions][nt * nz][slot], the regions a warp touches walked in ascending order).
 constexpr int kProfSeg = 2048;
-template <typename TIn, int EOS, int VM>
+template <typename TIn, int EOS, int VM, bool REG>
 __global__ void __launch_bounds__(kBlock)
     k_profile_direct(const TIn* __restrict__ T, const TIn* __restrict__ S, const TIn* __restrict__ T_ref,
                      const TIn* __restrict__ S_ref, const double* __restrict__ rho_ref, const void* __restrict__ v_ref,
                      int v_f32, const double* __restrict__ z_i, const double* __restrict__ deptho,
                      const double* __restrict__ weights, const double* __restrict__ p_level,
                      const double* __restrict__ p_col, double coef, int nt, int nz, i64 ncol, double* part0,
-                     double* part1, double* part2) {
+                     double* part1, double* part2, const int8_t* __restrict__ region, int nregions) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const i64 col0 = (i64)blockIdx.x * kProfSeg;
   const i64 nblk = (i64)gridDim.x * kWarps;
@@ -529,26 +530,59 @@ __global__ void __launch_bounds__(kBlock)
         if (VM & 2) sref[k] = __ldg(S_ref + i);
       }
     }
-    for (int t = 0; t < nt; ++t) {
-      double acc[3] = {0.0, 0.0, 0.0};
+    uint32_t rbits = 0, wmask = 0;  // REG: the 4-bit region index of each point; the regions the warp touches
+    if constexpr (REG) {
 #pragma unroll
       for (int k = 0; k < 8; ++k) {
         const i64 c = col0 + 4 * (tid + (k >> 2) * kBlock) + (k & 3);
-        if (c < ncol) {
-          const i64 i = (i64)t * lvl + (i64)z * ncol + c;
-          const double Tv = (VM & 3) ? ldf(T + i) : 0.0, Sv = (VM & 5) ? ldf(S + i) : 0.0;
-          if (VM & 1) acc[0] = profile_add(acc[0], cw[k], eos.rho_at(Tv, Sv, pz[k]), ref[k]);
-          if (VM & 2) acc[1] = profile_add(acc[1], cw[k], eos.rho_at(Tv, (double)sref[k], pz[k]), ref[k]);
-          if (VM & 4) acc[2] = profile_add(acc[2], cw[k], eos.rho_at((double)tref[k], Sv, pz[k]), ref[k]);
+        const uint32_t r = c < ncol ? region_nibble(region, c, nregions) : 0xFu;
+        rbits |= r << (4 * k);
+        wmask |= r < 0xFu ? 1u << r : 0u;
+      }
+      wmask = __reduce_or_sync(0xffffffffu, wmask);
+    }
+    for (int t = 0; t < nt; ++t) {
+      const i64 slot = ((i64)t * nz + z) * nblk + (i64)blockIdx.x * kWarps + warp;
+      const i64 rstride = (i64)nt * nz * nblk;  // REG: from one region's partials to the next
+      double acc[3];
+      // without REG one iteration over every point; with REG one per region the warp touches
+      for (uint32_t todo = REG ? wmask : 1u; todo != 0; todo &= todo - 1) {
+        const uint32_t r = __ffs(todo) - 1;
+        acc[0] = acc[1] = acc[2] = 0.0;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+          const i64 c = col0 + 4 * (tid + (k >> 2) * kBlock) + (k & 3);
+          if (REG ? ((rbits >> (4 * k)) & 0xFu) == r : c < ncol) {  // REG: a point past ncol is in no region
+            const i64 i = (i64)t * lvl + (i64)z * ncol + c;
+            const double Tv = (VM & 3) ? ldf(T + i) : 0.0, Sv = (VM & 5) ? ldf(S + i) : 0.0;
+            if (VM & 1) acc[0] = profile_add(acc[0], cw[k], eos.rho_at(Tv, Sv, pz[k]), ref[k]);
+            if (VM & 2) acc[1] = profile_add(acc[1], cw[k], eos.rho_at(Tv, (double)sref[k], pz[k]), ref[k]);
+            if (VM & 4) acc[2] = profile_add(acc[2], cw[k], eos.rho_at((double)tref[k], Sv, pz[k]), ref[k]);
+          }
+        }
+        if constexpr (REG) {
+#pragma unroll
+          for (int v = 0; v < 3; ++v)
+            if (VM & (1 << v)) {
+              const double w = warp_sum(acc[v]);
+              if (lane == 0) part[v][r * rstride + slot] = w;
+            }
         }
       }
-      const i64 slot = ((i64)t * nz + z) * nblk + (i64)blockIdx.x * kWarps + warp;
+      if constexpr (REG) {
+        if (lane < nregions && ((wmask >> lane) & 1u) == 0) {
 #pragma unroll
-      for (int v = 0; v < 3; ++v)
-        if (VM & (1 << v)) {
-          const double w = warp_sum(acc[v]);
-          if (lane == 0) part[v][slot] = w;
+          for (int v = 0; v < 3; ++v)
+            if (VM & (1 << v)) part[v][lane * rstride + slot] = 0.0;
         }
+      } else {
+#pragma unroll
+        for (int v = 0; v < 3; ++v)
+          if (VM & (1 << v)) {
+            const double w = warp_sum(acc[v]);
+            if (lane == 0) part[v][slot] = w;
+          }
+      }
     }
   }
 }
@@ -659,14 +693,19 @@ template <typename TIn, int EOS>
 int launch_profile_direct(int vm, const void* T, const void* S, const void* T_ref, const void* S_ref,
                           const double* rho_ref, const void* v_ref, int v_f32, const double* z_i, const double* deptho,
                           const double* weights, const double* p_level, double coef, int nt, int nz, i64 ncol,
-                          double* const part[3], cudaStream_t st) {
+                          double* const part[3], const int8_t* region, int nregions, cudaStream_t st) {
   const dim3 grid((unsigned)cdiv(ncol, kProfSeg), (unsigned)(nz < 65535 ? nz : 65535));
-#define ML_PROF_DIRECT(VM)                                                                                              \
-  case VM:                                                                                                              \
-    k_profile_direct<TIn, EOS, VM><<<grid, kBlock, 0, st>>>((const TIn*)T, (const TIn*)S, (const TIn*)T_ref,           \
-                                                            (const TIn*)S_ref, rho_ref, v_ref, v_f32, z_i, deptho,      \
-                                                            weights, p_level, tls().p_col, coef, nt, nz, ncol, part[0], \
-                                                            part[1], part[2]);                                          \
+#define ML_PROF_DIRECT_REG(VM, REG)                                                                                      \
+  k_profile_direct<TIn, EOS, VM, REG><<<grid, kBlock, 0, st>>>((const TIn*)T, (const TIn*)S, (const TIn*)T_ref,         \
+                                                               (const TIn*)S_ref, rho_ref, v_ref, v_f32, z_i, deptho,    \
+                                                               weights, p_level, tls().p_col, coef, nt, nz, ncol,        \
+                                                               part[0], part[1], part[2], region, nregions)
+#define ML_PROF_DIRECT(VM)                  \
+  case VM:                                  \
+    if (region != nullptr)                  \
+      ML_PROF_DIRECT_REG(VM, true);         \
+    else                                    \
+      ML_PROF_DIRECT_REG(VM, false);        \
     break
   switch (vm) {
     ML_PROF_DIRECT(1);
@@ -679,6 +718,7 @@ int launch_profile_direct(int vm, const void* T, const void* S, const void* T_re
     default: return fail(ML_ERR_MODE, "variant mask %d", vm);
   }
 #undef ML_PROF_DIRECT
+#undef ML_PROF_DIRECT_REG
   return launched("k_profile_direct");
 }
 
@@ -1089,20 +1129,28 @@ int ml_steric_local_layers_variants(int eos, int dtype, const void* T, const voi
   return ML_OK;
 }
 
-size_t ml_profile_workspace_bytes(int nvariants, int64_t nt, int64_t nz, int64_t ncol) {
+size_t ml_region_profile_workspace_bytes(int nvariants, int nregions, int64_t nt, int64_t nz, int64_t ncol) {
   nvariants = nvariants < 1 ? 1 : (nvariants > 3 ? 3 : nvariants);
+  if (nregions < 1) nregions = 1;
   if (nt < 1) nt = 1;
   if (nz < 1) nz = 1;
   const int64_t slots = stream::profile_slots(ncol > 0 ? ncol : 1);  // per-warp partials of one (step, level) row
-  return (size_t)(nvariants * nt * nz * slots) * sizeof(double) + 256;
+  return (size_t)((int64_t)nvariants * nregions * nt * nz * slots) * sizeof(double) + 256;
 }
 
-int ml_steric_local_profile(int eos, int dtype, const void* T, const void* S, const void* T_ref, const void* S_ref,
-                            const double* rho_ref, const void* v_ref, int vref_dtype, const double* z_i,
-                            const double* deptho, const double* weights, const double* p_level,
-                            double neg_inv_rhozero, int64_t nt, int64_t nz, int64_t ncol, double* prof_steric,
-                            double* prof_thermosteric, double* prof_halosteric, void* workspace, size_t ws_bytes,
-                            void* stream) {
+size_t ml_profile_workspace_bytes(int nvariants, int64_t nt, int64_t nz, int64_t ncol) {
+  return ml_region_profile_workspace_bytes(nvariants, 1, nt, nz, ncol);
+}
+
+// ml_steric_local_profile (region == NULL: one region of every column, the workspace holds all nt steps) and
+// ml_steric_local_region_profile (the workspace holds at least one step).  The time axis runs in chunks of as many
+// steps as the workspace holds, with the field pointers moved for each; a step's partials and sums depend on its
+// points only, so its bits do not depend on the chunks.
+static int profile_impl(int eos, int dtype, const void* T, const void* S, const void* T_ref, const void* S_ref,
+                        const double* rho_ref, const void* v_ref, int vref_dtype, const double* z_i,
+                        const double* deptho, const double* weights, const int8_t* region, int nregions,
+                        const double* p_level, double neg_inv_rhozero, int64_t nt, int64_t nz, int64_t ncol,
+                        double* const outs[3], void* workspace, size_t ws_bytes, void* stream) {
   int rc = check_common(eos, dtype);
   if (rc) return rc;
   if (vref_dtype != ML_F32 && vref_dtype != ML_F64) return fail(ML_ERR_DTYPE, "unknown vref dtype id %d", vref_dtype);
@@ -1116,15 +1164,13 @@ int ml_steric_local_profile(int eos, int dtype, const void* T, const void* S, co
   ML_REQUIRE_PTR(deptho);
   ML_REQUIRE_PTR(weights);
   ML_REQUIRE_PTR(p_level);
-  double* const outs[3] = {prof_steric, prof_thermosteric, prof_halosteric};
-  const int wanted = (prof_steric != nullptr) + (prof_thermosteric != nullptr) + (prof_halosteric != nullptr);
+  const int wanted = (outs[0] != nullptr) + (outs[1] != nullptr) + (outs[2] != nullptr);
   if (wanted == 0) return fail(ML_ERR_NULL, "prof_steric, prof_thermosteric and prof_halosteric are all NULL");
   if (nt < 0 || nz <= 0 || ncol <= 0 || nt > INT32_MAX || nz > INT32_MAX || nt * nz > INT32_MAX)
     return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ncol=%lld", (long long)nt, (long long)nz, (long long)ncol);
   if (int rcp = check_column_pressure(ncol)) return rcp;
-  if (workspace == nullptr || ws_bytes < ml_profile_workspace_bytes(wanted, nt, nz, ncol))
-    return fail(ML_ERR_WORKSPACE, "workspace needs %zu bytes, got %zu", ml_profile_workspace_bytes(wanted, nt, nz, ncol),
-                ws_bytes);
+  const size_t need = ml_region_profile_workspace_bytes(wanted, nregions, region ? 1 : nt, nz, ncol);
+  if (workspace == nullptr || ws_bytes < need) return fail(ML_ERR_WORKSPACE, "workspace needs %zu bytes, got %zu", need, ws_bytes);
   ML_REQUIRE_ALIGNED(workspace, 8);
   ML_REQUIRE_ALIGNED(T, elem_size(dtype));
   ML_REQUIRE_ALIGNED(S, elem_size(dtype));
@@ -1134,44 +1180,88 @@ int ml_steric_local_profile(int eos, int dtype, const void* T, const void* S, co
   if (nt == 0) return ML_OK;
   cudaStream_t st = (cudaStream_t)stream;
   const int v_f32 = vref_dtype == ML_F32;
-  // one region of per-warp partials per wanted variant, in the order steric, thermosteric, halosteric
   const i64 nblk = stream::profile_slots(ncol);
-  double* part[3] = {nullptr, nullptr, nullptr};
+  // steps per chunk: as many as the workspace holds, and at most INT32_MAX rows for k_reduce_rows
+  const size_t step_bytes = ml_region_profile_workspace_bytes(wanted, nregions, 1, nz, ncol) - 256;
+  i64 tc = (i64)((ws_bytes - 256) / step_bytes);
+  if (tc > nt) tc = nt;
+  if (tc > INT32_MAX / ((i64)nregions * nz)) tc = INT32_MAX / ((i64)nregions * nz);
   int vm = 0;
-  for (int v = 0, r = 0; v < 3; ++v)
-    if (outs[v]) {
-      part[v] = static_cast<double*>(workspace) + (i64)r++ * nt * nz * nblk;
-      vm |= 1 << v;
-    }
+  for (int v = 0; v < 3; ++v)
+    if (outs[v]) vm |= 1 << v;
   // ml_set_force_direct(2): one launch per variant (A/B against the one pass)
   const bool split = tls().force_direct == 2;
   const bool ring = dtype == ML_F32 && !direct_only() && stream::eligible(T, S, nullptr, workspace, ncol);
   tls().last_path = ring ? ML_PATH_TMA : ML_PATH_DIRECT;
-  for (int v = 0; v < 3; ++v) {
-    const int m = split ? (vm & (1 << v)) : (v == 0 ? vm : 0);
-    if (m == 0) continue;
-    double* const p[3] = {(m & 1) ? part[0] : nullptr, (m & 2) ? part[1] : nullptr, (m & 4) ? part[2] : nullptr};
-    if (ring)
-      rc = stream::launch_profile(eos, m, (const float*)T, (const float*)S, (const float*)T_ref, (const float*)S_ref,
-                                  rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, nz,
-                                  ncol, p, st);
-    else if (dtype == ML_F32)
-      rc = eos == ML_EOS_WRIGHT
-               ? launch_profile_direct<float, 0>(m, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, p, st)
-               : launch_profile_direct<float, 1>(m, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, p, st);
-    else
-      rc = eos == ML_EOS_WRIGHT
-               ? launch_profile_direct<double, 0>(m, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, p, st)
-               : launch_profile_direct<double, 1>(m, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)nt, (int)nz, ncol, p, st);
-    if (rc) return rc;
-  }
-  // fixed-order second stage: one block per (step, level) row
-  for (int v = 0; v < 3; ++v) {
-    if (outs[v] == nullptr) continue;
-    k_reduce_rows<<<(unsigned)(nt * nz), kBlock, 0, st>>>(part[v], nblk, outs[v]);
-    if ((rc = launched("k_reduce_rows"))) return rc;
+  for (i64 t0 = 0; t0 < nt; t0 += tc) {
+    const i64 n = nt - t0 < tc ? nt - t0 : tc;
+    const size_t off = (size_t)(t0 * nz * ncol) * elem_size(dtype);
+    const void* Tc = static_cast<const char*>(T) + off;
+    const void* Sc = static_cast<const char*>(S) + off;
+    // per wanted variant, in the order steric, thermosteric, halosteric: [nregions][n * nz][nblk] per-warp partials
+    double* part[3] = {nullptr, nullptr, nullptr};
+    for (int v = 0, r = 0; v < 3; ++v)
+      if (outs[v]) part[v] = static_cast<double*>(workspace) + (i64)r++ * nregions * n * nz * nblk;
+    for (int v = 0; v < 3; ++v) {
+      const int m = split ? (vm & (1 << v)) : (v == 0 ? vm : 0);
+      if (m == 0) continue;
+      double* const p[3] = {(m & 1) ? part[0] : nullptr, (m & 2) ? part[1] : nullptr, (m & 4) ? part[2] : nullptr};
+      if (ring)
+        rc = stream::launch_profile(eos, m, (const float*)Tc, (const float*)Sc, (const float*)T_ref, (const float*)S_ref,
+                                    rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, nz,
+                                    ncol, p, region, nregions, st);
+      else if (dtype == ML_F32)
+        rc = eos == ML_EOS_WRIGHT
+                 ? launch_profile_direct<float, 0>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, st)
+                 : launch_profile_direct<float, 1>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, st);
+      else
+        rc = eos == ML_EOS_WRIGHT
+                 ? launch_profile_direct<double, 0>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, st)
+                 : launch_profile_direct<double, 1>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, st);
+      if (rc) return rc;
+    }
+    // fixed-order second stage: one block per (region, step, level) row; outputs are [nregions][nt][nz]
+    for (int v = 0; v < 3; ++v) {
+      if (outs[v] == nullptr) continue;
+      if (n == nt) {
+        k_reduce_rows<<<(unsigned)(nregions * nt * nz), kBlock, 0, st>>>(part[v], nblk, outs[v]);
+        if ((rc = launched("k_reduce_rows"))) return rc;
+        continue;
+      }
+      for (int r = 0; r < nregions; ++r) {
+        k_reduce_rows<<<(unsigned)(n * nz), kBlock, 0, st>>>(part[v] + (i64)r * n * nz * nblk, nblk,
+                                                             outs[v] + ((i64)r * nt + t0) * nz);
+        if ((rc = launched("k_reduce_rows"))) return rc;
+      }
+    }
   }
   return ML_OK;
+}
+
+int ml_steric_local_profile(int eos, int dtype, const void* T, const void* S, const void* T_ref, const void* S_ref,
+                            const double* rho_ref, const void* v_ref, int vref_dtype, const double* z_i,
+                            const double* deptho, const double* weights, const double* p_level,
+                            double neg_inv_rhozero, int64_t nt, int64_t nz, int64_t ncol, double* prof_steric,
+                            double* prof_thermosteric, double* prof_halosteric, void* workspace, size_t ws_bytes,
+                            void* stream) {
+  double* const outs[3] = {prof_steric, prof_thermosteric, prof_halosteric};
+  return profile_impl(eos, dtype, T, S, T_ref, S_ref, rho_ref, v_ref, vref_dtype, z_i, deptho, weights, nullptr, 1,
+                      p_level, neg_inv_rhozero, nt, nz, ncol, outs, workspace, ws_bytes, stream);
+}
+
+int ml_steric_local_region_profile(int eos, int dtype, const void* T, const void* S, const void* T_ref,
+                                   const void* S_ref, const double* rho_ref, const void* v_ref, int vref_dtype,
+                                   const double* z_i, const double* deptho, const double* weights,
+                                   const int8_t* region, int nregions, const double* p_level, double neg_inv_rhozero,
+                                   int64_t nt, int64_t nz, int64_t ncol, double* prof_steric,
+                                   double* prof_thermosteric, double* prof_halosteric, void* workspace,
+                                   size_t ws_bytes, void* stream) {
+  if (nregions < 1 || nregions > ML_MAX_REGIONS)
+    return fail(ML_ERR_SHAPE, "nregions=%d is outside [1, %d]", nregions, ML_MAX_REGIONS);
+  ML_REQUIRE_PTR(region);
+  double* const outs[3] = {prof_steric, prof_thermosteric, prof_halosteric};
+  return profile_impl(eos, dtype, T, S, T_ref, S_ref, rho_ref, v_ref, vref_dtype, z_i, deptho, weights, region,
+                      nregions, p_level, neg_inv_rhozero, nt, nz, ncol, outs, workspace, ws_bytes, stream);
 }
 
 static int delta_rho_impl(int eos, int dtype, const void* T, const void* S, int t_bcast, int s_bcast,

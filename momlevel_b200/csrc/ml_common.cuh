@@ -271,5 +271,11 @@ __device__ __forceinline__ double profile_add(double acc, double cw, double rho,
   const double d = __dsub_rn(rho, rref);
   return is_nan_q(d) ? acc : fma(cw, d, acc);
 }
+// Region of a column for ml_steric_local_region_profile as a 4-bit field: its index if in [0, nregions), else 0xF
+// (no region; nregions <= ML_MAX_REGIONS = 15).
+__device__ __forceinline__ uint32_t region_nibble(const int8_t* region, i64 c, int nregions) {
+  const int r = __ldg(region + c);
+  return (r >= 0 && r < nregions) ? (uint32_t)r : 0xFu;
+}
 
 }  // namespace ml

@@ -333,12 +333,21 @@ __global__ void __launch_bounds__(kThreads, 2)
 // sums by shuffle and lane 0 stores the warp's partial: no CTA-wide barrier in the loop, and a partial's slot depends
 // on the point's position only, so the sums do not depend on the grid.  VM: bit 0 steric (T, S), bit 1 thermosteric
 // (T, S_ref), bit 2 halosteric (T_ref, S) (steric.py:115-121); only the operands the variants read are staged.
+// REG (ml_steric_local_region_profile): one partial per region, partials[v][r][t * nz + z][seg * kWarps + warp].
+// At the setup of a pair a thread packs the region index of its 8 points into 4-bit fields of one register (0xF: no
+// region) and the warp ORs the regions its points touch into a mask fixed for the pair; the shared memory is full, so
+// the codes stay in registers.  Per step the warp walks the set bits of that mask in ascending order and in
+// iteration r each thread sums, in the order above, only its points of region r: every density is evaluated once,
+// and a warp whose points all lie in one region sums exactly as without regions.  Lane 0 stores region r's
+// partial; lane r stores 0 for a region the warp does not touch, so every slot is written on every step.
 constexpr size_t kProfileRing = ring_bytes<2>();  // the per-point state follows the ring
 struct ProfileOut {
-  double* part[3];  // per variant, [nt * nz][tiles_per_row * kWarps]; NULL for a variant not asked for
+  double* part[3];  // per variant, [nregions][nt * nz][tiles_per_row * kWarps]; NULL for a variant not asked for
+  const int8_t* region;  // REG: [ncol] region index of each column, one in [0, nregions) or none
+  int nregions;
 };
 
-template <int EOS, int VM>
+template <int EOS, int VM, bool REG>
 __global__ void __launch_bounds__(kThreads, 2)
     k_stream_profile(const float* __restrict__ T, const float* __restrict__ S, const float* __restrict__ T_ref,
                      const float* __restrict__ S_ref, const double* __restrict__ rho_ref, const void* __restrict__ v_ref,
@@ -387,6 +396,17 @@ __global__ void __launch_bounds__(kThreads, 2)
     const i64 off = row * g.ncol + col0;
     eos.set_level(__ldg(p_level + row));
     const double ztop = __ldg(z_i + row), zbot = __ldg(z_i + row + 1);
+    uint32_t rbits = 0, wmask = 0;  // REG: the 4-bit region index of each point; the regions the warp touches
+    if constexpr (REG) {
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        const i64 p = 4 * (tid + (k >> 2) * kThreads) + (k & 3);
+        const uint32_t r = p < len ? region_nibble(out.region, col0 + p, out.nregions) : 0xFu;
+        rbits |= r << (4 * k);
+        wmask |= r < 0xFu ? 1u << r : 0u;
+      }
+      wmask = __reduce_or_sync(0xffffffffu, wmask);
+    }
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
       const int qd = tid + h * kThreads;
@@ -418,34 +438,57 @@ __global__ void __launch_bounds__(kThreads, 2)
       tma::mbar_wait(ring.full + s, (uint32_t)(q / kStages) & 1u);
       const float4* sT = reinterpret_cast<const float4*>(ring.stage(s, 0));
       const float4* sS = reinterpret_cast<const float4*>(ring.stage(s, 1));
-      double acc[3] = {0.0, 0.0, 0.0};
+      const i64 slot = ((i64)t * g.nz + row) * nblk + seg * kWarps + warp;
+      const i64 rstride = (i64)nt * g.nz * nblk;  // REG: from one region's partials to the next
+      double acc[3];
+      // without REG one iteration over every point; with REG one per region the warp touches
+      for (uint32_t todo = REG ? wmask : 1u; todo != 0; todo &= todo - 1) {
+        const uint32_t r = __ffs(todo) - 1;
+        acc[0] = acc[1] = acc[2] = 0.0;
 #pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const int qd = tid + h * kThreads;
-        if (4 * qd < len) {
-          float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
-          if (kT) a = sT[qd];
-          if (kS) b = sS[qd];
-          const float ta[4] = {a.x, a.y, a.z, a.w}, sa[4] = {b.x, b.y, b.z, b.w};
+        for (int h = 0; h < 2; ++h) {
+          const int qd = tid + h * kThreads;
+          if (4 * qd < len) {
+            float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
+            if (kT) a = sT[qd];
+            if (kS) b = sS[qd];
+            const float ta[4] = {a.x, a.y, a.z, a.w}, sa[4] = {b.x, b.y, b.z, b.w};
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            if (VM & 1) acc[0] = profile_add(acc[0], cw[(4 * h + j) * kThreads], eos.rho((double)ta[j], (double)sa[j]), ref[(4 * h + j) * kThreads]);
-            if (VM & 2) acc[1] = profile_add(acc[1], cw[(4 * h + j) * kThreads], eos.rho((double)ta[j], (double)sref[(4 * h + j) * kThreads]), ref[(4 * h + j) * kThreads]);
-            if (VM & 4) acc[2] = profile_add(acc[2], cw[(4 * h + j) * kThreads], eos.rho((double)tref[(4 * h + j) * kThreads], (double)sa[j]), ref[(4 * h + j) * kThreads]);
+            for (int j = 0; j < 4; ++j) {
+              if (REG && ((rbits >> (4 * (4 * h + j))) & 0xFu) != r) continue;
+              if (VM & 1) acc[0] = profile_add(acc[0], cw[(4 * h + j) * kThreads], eos.rho((double)ta[j], (double)sa[j]), ref[(4 * h + j) * kThreads]);
+              if (VM & 2) acc[1] = profile_add(acc[1], cw[(4 * h + j) * kThreads], eos.rho((double)ta[j], (double)sref[(4 * h + j) * kThreads]), ref[(4 * h + j) * kThreads]);
+              if (VM & 4) acc[2] = profile_add(acc[2], cw[(4 * h + j) * kThreads], eos.rho((double)tref[(4 * h + j) * kThreads], (double)sa[j]), ref[(4 * h + j) * kThreads]);
+            }
           }
+        }
+        if constexpr (REG) {
+#pragma unroll
+          for (int v = 0; v < 3; ++v)
+            if (VM & (1 << v)) {
+              const double w = warp_sum(acc[v]);
+              if (lane == 0) out.part[v][r * rstride + slot] = w;
+            }
         }
       }
       if (last_to_leave(ring.empty + s, ring.released + s, (uint32_t)(q / kStages) & 1u)) {
         const i64 next = q + kStages;
         if (next < nseq) issue(next, s);
       }
-      const i64 slot = ((i64)t * g.nz + row) * nblk + seg * kWarps + warp;
+      if constexpr (REG) {
+        if (lane < out.nregions && ((wmask >> lane) & 1u) == 0) {
 #pragma unroll
-      for (int v = 0; v < 3; ++v)
-        if (VM & (1 << v)) {
-          const double w = warp_sum(acc[v]);
-          if (lane == 0) out.part[v][slot] = w;
+          for (int v = 0; v < 3; ++v)
+            if (VM & (1 << v)) out.part[v][lane * rstride + slot] = 0.0;
         }
+      } else {
+#pragma unroll
+        for (int v = 0; v < 3; ++v)
+          if (VM & (1 << v)) {
+            const double w = warp_sum(acc[v]);
+            if (lane == 0) out.part[v][slot] = w;
+          }
+      }
     }
   }
 }
@@ -549,12 +592,12 @@ constexpr size_t profile_smem_bytes() { return kProfileRing + 2 * kTile * (sizeo
 
 int profile_slots(i64 ncol) { return (int)((ncol + kTile - 1) / kTile) * kWarps; }
 
-template <int EOS, int VM>
+template <int EOS, int VM, bool REG>
 static int launch_profile_vm(const float* T, const float* S, const float* T_ref, const float* S_ref,
                              const double* rho_ref, const void* v_ref, int v_f32, const double* z_i,
                              const double* deptho, const double* weights, const double* p_level, double coef, int nt,
                              const Geom& g, const ProfileOut& out, cudaStream_t st) {
-  auto kern = k_stream_profile<EOS, VM>;
+  auto kern = k_stream_profile<EOS, VM, REG>;
   if (int rc = opt_in(kern, profile_smem_bytes())) return rc;
   kern<<<persistent_grid(g.ntiles, 2), kThreads, profile_smem_bytes(), st>>>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i,
                                                                          deptho, weights, p_level, coef, nt, g, out);
@@ -566,8 +609,12 @@ static int launch_profile_eos(int vm, const float* T, const float* S, const floa
                               const double* rho_ref, const void* v_ref, int v_f32, const double* z_i,
                               const double* deptho, const double* weights, const double* p_level, double coef, int nt,
                               const Geom& g, const ProfileOut& out, cudaStream_t st) {
-#define ML_STREAM_PROF(VM) \
-  case VM: return launch_profile_vm<EOS, VM>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, coef, nt, g, out, st)
+#define ML_STREAM_PROF(VM)                                                                                               \
+  case VM:                                                                                                               \
+    return out.region ? launch_profile_vm<EOS, VM, true>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho,        \
+                                                         weights, p_level, coef, nt, g, out, st)                        \
+                      : launch_profile_vm<EOS, VM, false>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho,       \
+                                                          weights, p_level, coef, nt, g, out, st)
   switch (vm) {
     ML_STREAM_PROF(1);
     ML_STREAM_PROF(2);
@@ -584,9 +631,9 @@ static int launch_profile_eos(int vm, const float* T, const float* S, const floa
 int launch_profile(int eos, int vm, const float* T, const float* S, const float* T_ref, const float* S_ref,
                    const double* rho_ref, const void* v_ref, int v_f32, const double* z_i, const double* deptho,
                    const double* weights, const double* p_level, double coef, int nt, i64 nz, i64 ncol,
-                   double* const part[3], cudaStream_t st) {
+                   double* const part[3], const int8_t* region, int nregions, cudaStream_t st) {
   const Geom g = geometry(nz, (int)nz, ncol);
-  const ProfileOut out = {{part[0], part[1], part[2]}};
+  const ProfileOut out = {{part[0], part[1], part[2]}, region, nregions};
   if (eos == ML_EOS_WRIGHT)
     return launch_profile_eos<0>(vm, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, coef, nt, g, out, st);
   return launch_profile_eos<1>(vm, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, coef, nt, g, out, st);

@@ -29,12 +29,13 @@ int launch_delta_rho(int eos, const float* T, const float* S, long long t_stride
 
 // level profile (ml_steric_local_profile): per-warp partials of coef * m * w * dz * (rho_v - rho_ref) into part[v]
 // ([nt * nz][profile_slots(ncol)], NULL for a variant not asked for), vm = the variants as bits (1 steric,
-// 2 thermosteric, 4 halosteric); the fixed-order second stage is k_reduce_rows
+// 2 thermosteric, 4 halosteric); the fixed-order second stage is k_reduce_rows.  With a region index ([ncol],
+// ml_steric_local_region_profile; NULL: none) part[v] is [nregions][nt * nz][profile_slots(ncol)].
 int profile_slots(long long ncol);
 int launch_profile(int eos, int vm, const float* T, const float* S, const float* T_ref, const float* S_ref,
                    const double* rho_ref, const void* v_ref, int v_f32, const double* z_i, const double* deptho,
                    const double* weights, const double* p_level, double coef, int nt, long long nz, long long ncol,
-                   double* const part[3], cudaStream_t st);
+                   double* const part[3], const int8_t* region, int nregions, cudaStream_t st);
 
 }  // namespace stream
 }  // namespace ml

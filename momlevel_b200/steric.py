@@ -12,7 +12,7 @@ import weakref
 import numpy as np
 import torch
 
-from . import core
+from . import _lib, core
 from .labeled import ChunkedArray, DataArray, Dataset
 from .reference import _pressure, setup_reference_state
 from .util import annual_average, calendar_axis, default_coords, validate_dataset, whole_years_in_order
@@ -885,9 +885,50 @@ def steric_layers(dset, depth_edges=(0.0, 700.0, 2000.0, None), reference=None, 
     return (result, reference)
 
 
+def _region_map(regions, region_codes):
+    """``(codes, index)`` of a region map: ``codes`` the selected codes in order (``region_codes``, or the sorted
+    distinct non-negative codes present), ``index`` an int8 ``(y, x)`` array, the position of each column's code in
+    ``codes`` or -1 (a NaN, negative or unselected code: no region)."""
+    if regions is None:
+        if region_codes is not None:
+            raise ValueError("region_codes selects codes of `regions`, which was not given")
+        return None, None
+    r = regions.data if isinstance(regions, DataArray) else regions
+    if type(r).__module__.startswith("xarray"):
+        r = r.values
+    r = r.detach().cpu().numpy() if isinstance(r, torch.Tensor) else np.asarray(r)
+    if r.dtype.kind not in "fiub":
+        raise ValueError(f"regions must hold numeric codes, got dtype {r.dtype}")
+    r = r.astype(np.float64)
+    coded = ~np.isnan(r) & (r >= 0)
+    if (coded & ((r != np.floor(r)) | np.isinf(r))).any():
+        raise ValueError("regions holds a code that is not an integer; NaN and negative values mean no region")
+    if region_codes is None:
+        codes = [int(c) for c in np.unique(r[coded])]
+        if not codes:
+            raise ValueError("regions holds no non-negative code; pass region_codes to select codes")
+    else:
+        codes = []
+        for c in np.atleast_1d(np.asarray(region_codes)).tolist():
+            if isinstance(c, bool) or not float(c).is_integer() or c < 0:
+                raise ValueError(f"region_codes must be non-negative integers, got {c!r}")
+            codes.append(int(c))
+        if not codes:
+            raise ValueError("region_codes is empty")
+        if len(set(codes)) != len(codes):
+            raise ValueError(f"region_codes holds a code twice: {codes}")
+    if len(codes) > _lib.MAX_REGIONS:
+        raise ValueError(f"{len(codes)} region codes: at most {_lib.MAX_REGIONS} regions in one call; select some "
+                         "with region_codes")
+    index = np.full(r.shape, -1, dtype=np.int8)
+    for i, c in enumerate(codes):
+        index[r == c] = i
+    return codes, index
+
+
 def steric_profile(dset, variant="steric", reference=None, weights=None, coord_names=None, varname_map=None,
                    rhozero=1035.0, patm=101325.0, equation_of_state="Wright", dtype="float32", strict=True, annual=False,
-                   days_in_month=None, verbose=False):
+                   days_in_month=None, verbose=False, regions=None, region_codes=None):
     """How much each model level contributes to the area-weighted mean steric, thermosteric or halosteric sea level
     change, per time step, from one pass over T and S (a depth-time Hovmoeller of the expansion; summed over the
     levels below a depth, that depth's deep contribution).
@@ -906,9 +947,18 @@ def steric_profile(dset, variant="steric", reference=None, weights=None, coord_n
     ``reference=None`` builds the reference state from the first step first.  Chunked (dask-backed) fields raise
     ``NotImplementedError``.
 
-    Returns ``(result, reference)``: ``result[name]`` has dims ``(time, z_l)``.
+    ``regions`` (a ``(y, x)`` array of codes, such as MOM6's ``basin`` or the CMIP ``basin`` variable) gives the
+    profile of every region from the same one pass: region ``c`` is, bit for bit, this call with
+    ``weights=where(regions == c, w, 0)``.  A NaN or negative code puts a column in no region.  ``region_codes``
+    selects and orders the codes (at most 15; for example ``[1, 2, 3, 5]`` leaves out CMIP code 0, land); by default
+    it is the sorted distinct non-negative codes present.  A selected code without columns gives NaN.
+
+    Returns ``(result, reference)``: ``result[name]`` has dims ``(time, z_l)``.  With ``regions`` it has dims ``(time,
+    region, z_l)``, the ``region`` coordinate holds the codes and ``result["region_weight"]`` is ``(region,)``, each
+    region's ``nansum(w)``, so that regions combine exactly: ``(p[a] * W[a] + p[b] * W[b]) / (W[a] + W[b])``.
     """
     names = core.variant_names(variant)
+    codes, region_index = _region_map(regions, region_codes)
     xarray_in = type(dset).__module__.startswith("xarray")
     if xarray_in:
         from . import xarray_io
@@ -928,6 +978,9 @@ def steric_profile(dset, variant="steric", reference=None, weights=None, coord_n
     if _chunked(dset):
         raise NotImplementedError("steric_profile takes device-resident or in-memory fields; chunked (dask-backed) "
                                   "fields are not supported yet")
+    if region_index is not None and region_index.shape != tuple(dset["thetao"].shape[2:]):
+        raise ValueError(f"regions of shape {region_index.shape} do not match the horizontal grid "
+                         f"{tuple(dset['thetao'].shape[2:])}")
     validate_dataset(dset, strict=strict, additional_vars=[zbounds, "deptho"])
     full = dset["thetao"]
     if full.dims[0] != tcoord or full.dims[1] != zcoord or dset["so"].dims != full.dims:
@@ -956,15 +1009,26 @@ def steric_profile(dset, variant="steric", reference=None, weights=None, coord_n
     validate_dataset(reference, reference=True, strict=strict)
 
     _check_depths(dset, zcoord, zbounds)
-    profs = core.steric_local_profile(full.data, dset["so"].data, reference["thetao"].data, reference["so"].data,
-                                      reference["rho"].data, reference["volcello"].data, dset[zbounds].data,
-                                      dset["deptho"].data, pres, w, rhozero=rhozero, eos=equation_of_state,
-                                      variants=names)
+    operands = (full.data, dset["so"].data, reference["thetao"].data, reference["so"].data, reference["rho"].data,
+                reference["volcello"].data, dset[zbounds].data, dset["deptho"].data, pres, w)
     result = Dataset()
-    for name in names:
-        result[name] = DataArray(profs[name], (tcoord, zcoord), attrs={
-            "long_name": f"{name.capitalize()} height adjustment by level, area-weighted mean", "units": "m"})
-        result[name].encoding["dtype"] = dtype
+    if region_index is None:
+        profs = core.steric_local_profile(*operands, rhozero=rhozero, eos=equation_of_state, variants=names)
+        for name in names:
+            result[name] = DataArray(profs[name], (tcoord, zcoord), attrs={
+                "long_name": f"{name.capitalize()} height adjustment by level, area-weighted mean", "units": "m"})
+            result[name].encoding["dtype"] = dtype
+    else:
+        profs, totals = core.steric_local_region_profile(*operands, region_index, len(codes), rhozero=rhozero,
+                                                         eos=equation_of_state, variants=names)
+        for name in names:
+            result[name] = DataArray(profs[name].permute(1, 0, 2).contiguous(), (tcoord, "region", zcoord), attrs={
+                "long_name": f"{name.capitalize()} height adjustment by level and region, area-weighted mean",
+                "units": "m"})
+            result[name].encoding["dtype"] = dtype
+        result["region"] = DataArray(np.asarray(codes, dtype=np.int64), ("region",), attrs={"long_name": "Region code"})
+        result["region_weight"] = DataArray(totals, ("region",), attrs={
+            "long_name": "Sum of the column weights of the region (nansum(w))"})
     for var in set(result.dims):
         if var in dset.variables:
             coord = dset[var].copy(deep=False)
