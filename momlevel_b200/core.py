@@ -713,7 +713,8 @@ def steric_local_variants(T, S, v_ref, z_i, deptho, p_level, T_ref=None, S_ref=N
     """Steric, thermosteric and halosteric height in one call (steric.py:115-121, :150-166).
 
     ``T_ref, S_ref`` default to step 0 of ``T, S`` (what ``steric()`` does without ``reference=``); with
-    ``rho_ref=None`` the reference density is evaluated on the way.  Returns
+    ``rho_ref=None`` the reference density is evaluated on the way.  The four operands are stored in one dtype:
+    fp32 only if all four are fp32, so an fp64 reference slab is never rounded to fp32 fields.  Returns
     ``({"steric": eta, "thermosteric": eta, "halosteric": eta}, rho_ref, sums or None)`` on the device.
     ``want_rho_ref=False`` (self-reference calls only) asks the library not to store the reference density when
     the one-pass kernel does not need the field; ``rho_ref`` is then ``None`` unless the layout needs it.
@@ -721,8 +722,10 @@ def steric_local_variants(T, S, v_ref, z_i, deptho, p_level, T_ref=None, S_ref=N
     L = _lib.lib()
     p_level, _pcol = _pressure_parts(p_level)
     T, S, nt, nz, ncol, hshape = _steric_operands(T, S, False, False)
-    Tr = T[0] if T_ref is None else to_device(T_ref).to(T.dtype)
-    Sr = S[0] if S_ref is None else to_device(S_ref).to(S.dtype)
+    Tr = T[0] if T_ref is None else to_device(T_ref)
+    Sr = S[0] if S_ref is None else to_device(S_ref)
+    dt = _field_dtype(T, S, Tr, Sr)
+    T, S, Tr, Sr = T.to(dt), S.to(dt), Tr.to(dt), Sr.to(dt)
     assert Tr.is_contiguous() and Sr.is_contiguous() and Tr.numel() == nz * ncol and Sr.numel() == nz * ncol
     v_ref = to_device(v_ref)
     z_i, depth, p = _f64(z_i), _f64(deptho), _f64(p_level)
@@ -784,6 +787,8 @@ def steric_global_variants(T, S, v_ref, p_level, T_ref=None, S_ref=None, eos="Wr
 
     ``T_ref, S_ref`` default to step 0 of ``T, S`` (what ``steric()`` does without ``reference=``); the sums
     ``{volo, masso}`` of that reference state are then produced on the way.  ``variants`` may name a subset.
+    The four operands are stored in one dtype: fp32 only if all four are fp32, so an fp64 reference slab is never
+    rounded to fp32 fields.
     Returns ``({variant: masso[nt]}, sums fp64[2] or None)`` on the device (``ml_steric_global_variants``).
     """
     L = _lib.lib()
@@ -791,8 +796,10 @@ def steric_global_variants(T, S, v_ref, p_level, T_ref=None, S_ref=None, eos="Wr
     T, S, nt, nz, ncol, _ = _steric_operands(T, S, False, False)
     if (T_ref is None) != (S_ref is None):
         raise ValueError("T_ref and S_ref are given together or not at all")
-    Tr = T if T_ref is None else to_device(T_ref).to(T.dtype).contiguous()
-    Sr = S if S_ref is None else to_device(S_ref).to(S.dtype).contiguous()
+    Tr = T if T_ref is None else to_device(T_ref)
+    Sr = S if S_ref is None else to_device(S_ref)
+    dt = _field_dtype(T, S, Tr, Sr)
+    T, S, Tr, Sr = T.to(dt), S.to(dt), Tr.to(dt).contiguous(), Sr.to(dt).contiguous()
     selfref = Tr.data_ptr() == T.data_ptr() and Sr.data_ptr() == S.data_ptr()  # step 0 of the fields themselves
     assert selfref or (Tr.numel() == nz * ncol and Sr.numel() == nz * ncol)
     v_ref = to_device(v_ref)
@@ -929,7 +936,10 @@ class HostStream:
     ``domain="local"``, ``[nt_block]`` masses for ``domain="global"`` -- which are complete once :meth:`finish`
     has returned.  With ``reference=None`` the reference state is step 0 of the first block; otherwise
     ``reference = {"thetao", "so", "rho"}`` (host arrays) is a supplied reference (steric.py:98-103).
-    The stream holds at most the current and the previous block alive.
+    ``dtype`` is how the blocks are stored on their way to the device.  An fp32 stream runs in fp64 when a supplied
+    ``thetao`` or ``so`` slab is fp64 and one of its values does not survive a round trip through fp32, so that the
+    slab is never rounded; an fp64 slab that is an upcast copy of fp32 data keeps the fp32 transfer.  ``self.dtype``
+    is the dtype the stream runs in.  The stream holds at most the current and the previous block alive.
     """
 
     def __init__(self, domain, v_ref, p_level, z_i=None, deptho=None, variants=("steric",), reference=None,
@@ -943,7 +953,6 @@ class HostStream:
         mask = 0
         for v in self.variants:
             mask |= VARIANT_BITS[v]
-        self.dtype = dtype
         host = _host_tensor
         self._v = host(v_ref)
         if self._v.dtype not in (torch.float32, torch.float64):
@@ -962,6 +971,8 @@ class HostStream:
         tref = sref = rref = None
         if reference is not None:
             self._ref = {k: host(reference[k]) for k in ("thetao", "so", "rho") if reference.get(k) is not None}
+            if dtype == torch.float32 and not all(_fp32_exact(self._ref[k]) for k in ("thetao", "so") if k in self._ref):
+                dtype = torch.float64
             if "thetao" in self._ref:
                 self._ref["thetao"] = self._ref["thetao"].to(dtype)
                 self._ref["so"] = self._ref["so"].to(dtype)
@@ -969,6 +980,7 @@ class HostStream:
             if "rho" in self._ref:
                 self._ref["rho"] = self._ref["rho"].to(torch.float64)
                 rref = self._ref["rho"].data_ptr()
+        self.dtype = dtype
         self.want_rho_ref = bool(want_rho_ref)
         self.max_block_steps = int(max_block_steps)
         handle = ctypes.c_void_p()
@@ -1030,6 +1042,14 @@ class HostStream:
 
 def _host_np(x):
     return x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else np.asarray(x)
+
+
+def _fp32_exact(t):
+    """Whether every value of the host tensor ``t`` survives a round trip through fp32 (NaN stays NaN)."""
+    if t.dtype == torch.float32:
+        return True
+    t = t.to(torch.float64)
+    return bool(((t.to(torch.float32).to(torch.float64) == t) | torch.isnan(t)).all())
 
 
 def host_release():
