@@ -335,6 +335,32 @@ int ml_steric_local_region_profile(int eos, int dtype, const void* T, const void
                                    void* workspace, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------
+ * ml_steric_local_zonal_profile -- ml_steric_local_profile for every grid row at once (a latitude-depth
+ * section), from one pass over T and S:
+ *   prof_v[t][z][j] = neg_inv_rhozero * nansum_i( m * w * dz * delta_rho_v[t][z][j][i] )
+ * Row j is bit for bit what ml_steric_local_profile gives on the fields, reference slabs, deptho, weights and
+ * column pressure of row j alone (sliced to [..., j:j+1, :], contiguous, ncol = nx): a (level, row) is split into
+ * the same 2048-column sub-tiles, summed in the same order into the same per-warp partials.  Routes and switches
+ * are those of ml_steric_local_profile (the ring for fp32 fields with nx % 4 == 0 and 16-byte aligned bases, the
+ * plain-load kernel with the same bits otherwise, ml_set_force_direct(2) one launch per variant).
+ *   T, S          [nt][nz][ny][nx] of `dtype`; T_ref, S_ref, rho_ref, v_ref [nz][ny][nx]
+ *   deptho, weights [ny][nx] fp64 (device); a column pressure (ml_set_column_pressure) has ny * nx values
+ *   prof_*        [nt][nz][ny] fp64 out each (device): numerators only, the caller divides row j by the row's
+ *                 nansum(w); a NULL pointer skips that variant; at least one is required (ML_ERR_NULL)
+ *   workspace     at least one step: ml_zonal_profile_workspace_bytes(number of prof_* given, 1, nz, ny, nx)
+ *                 bytes (ML_ERR_WORKSPACE otherwise).  The time axis runs in chunks of as many steps as the
+ *                 workspace holds; the bits of a step do not depend on the chunks.
+ * Other arguments as ml_steric_local_profile.  Every argument error returns before any launch.
+ * ------------------------------------------------------------------------------------- */
+size_t ml_zonal_profile_workspace_bytes(int nvariants, int64_t nt, int64_t nz, int64_t ny, int64_t nx);
+int ml_steric_local_zonal_profile(int eos, int dtype, const void* T, const void* S, const void* T_ref,
+                                  const void* S_ref, const double* rho_ref, const void* v_ref, int vref_dtype,
+                                  const double* z_i, const double* deptho, const double* weights,
+                                  const double* p_level, double neg_inv_rhozero, int64_t nt, int64_t nz,
+                                  int64_t ny, int64_t nx, double* prof_steric, double* prof_thermosteric,
+                                  double* prof_halosteric, void* workspace, size_t ws_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------
  * ml_steric_global -- fused EOS -> sum_{z,col} rho * v_ref per time step.
  * Replaces calc_masso(rho, reference["volcello"]) in the global branch
  * (src/momlevel/steric.py:135, derived.py:435-438); the ln() formula (steric.py:136-142)

@@ -50,6 +50,9 @@ EXPORTS = {
     "ml_region_profile_workspace_bytes": (_sz, [_i, _i, _i64, _i64, _i64]),
     "ml_steric_local_region_profile": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _d, _i64,
                                             _i64, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ml_zonal_profile_workspace_bytes": (_sz, [_i, _i64, _i64, _i64, _i64]),
+    "ml_steric_local_zonal_profile": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i64, _i64,
+                                           _i64, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ml_delta_rho": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_delta_rho_annual": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _i64, _i64, _i64, _vp, _vp]),
     "ml_steric_local_selfref": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _d, _i64, _i64, _i64, _vp, _vp, _vp,

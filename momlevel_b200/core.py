@@ -26,6 +26,7 @@ __all__ = [
     "steric_local_layers_variants",
     "steric_local_profile",
     "steric_local_region_profile",
+    "steric_local_zonal_profile",
     "layer_edges",
     "delta_rho",
     "steric_global",
@@ -614,6 +615,58 @@ def steric_local_region_profile(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho,
     # each total as steric_local_profile forms it from the masked weights, so that the quotients match bit for bit
     totals = torch.stack([torch.nansum(torch.where(ri == r, w, 0.0)) for r in range(nregions)])
     return {v: prof[v] / totals[:, None, None] for v in names}, totals
+
+
+def steric_local_zonal_profile(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho, p_level, weights, rhozero=1035.0,
+                               eos="Wright", variants=VARIANTS):
+    """:func:`steric_local_profile` for every grid row at once, from one pass over T and S
+    (``ml_steric_local_zonal_profile``).
+
+    ``T, S`` are ``[nt, nz, ny, nx]``, ``weights`` is ``[ny, nx]``.  Row ``j`` is, bit for bit,
+    :func:`steric_local_profile` on the operands of row ``j`` alone (sliced to ``[..., j:j+1, :]``).  Returns
+    ``({variant: [nt, nz, ny]}, totals[ny])`` fp64 on the device: the sections already divided by ``totals``, each
+    row's ``nansum`` of the weights (0/0, NaN, for a row whose weights sum to 0).
+    """
+    L = _lib.lib()
+    names = variant_names(variants)
+    p_level, _pcol = _pressure_parts(p_level)
+    T, S = to_device(T), to_device(S)
+    if T.dim() != 4 or tuple(S.shape) != tuple(T.shape):
+        raise ValueError(f"fields laid out (time, z, y, x): got {tuple(T.shape)} and {tuple(S.shape)}")
+    T, S, nt, nz, ncol, _ = _steric_operands(T, S, False, False)
+    ny, nx = T.shape[2], T.shape[3]
+    Tr, Sr = to_device(T_ref), to_device(S_ref)
+    dt = _field_dtype(T, S, Tr, Sr)
+    T, S, Tr, Sr = T.to(dt), S.to(dt), Tr.to(dt), Sr.to(dt)
+    rho_ref = _f64(rho_ref)
+    v_ref = to_device(v_ref)
+    z_i, depth, p, w = _f64(z_i), _f64(deptho), _f64(p_level), _f64(weights)
+    assert Tr.numel() == nz * ncol and Sr.numel() == nz * ncol and rho_ref.numel() == nz * ncol
+    assert v_ref.numel() == nz * ncol and depth.numel() == ncol and z_i.numel() == nz + 1 and p.numel() == nz
+    if tuple(w.shape) != (ny, nx):
+        raise ValueError(f"weights of shape {tuple(w.shape)} do not match the horizontal grid {(ny, nx)}")
+    prof = {v: torch.empty((nt, nz, ny), dtype=torch.float64, device=T.device) for v in names}
+    step = L.ml_zonal_profile_workspace_bytes(len(names), 1, nz, ny, nx) - 256
+    steps = max(1, min(nt, (REGION_WORKSPACE_BYTES - 256) // step))
+    nbytes = L.ml_zonal_profile_workspace_bytes(len(names), steps, nz, ny, nx)
+    ws = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=T.device)
+    ptr = lambda v: prof[v].data_ptr() if v in prof else None  # noqa: E731
+    with _pcol:
+        _lib.check(
+            L.ml_steric_local_zonal_profile(_eos_id(eos), _dt_id(T), T.data_ptr(), S.data_ptr(), Tr.data_ptr(),
+                                            Sr.data_ptr(), rho_ref.data_ptr(), v_ref.data_ptr(), _dt_id(v_ref),
+                                            z_i.data_ptr(), depth.data_ptr(), w.data_ptr(), p.data_ptr(),
+                                            -1.0 / rhozero, nt, nz, ny, nx, ptr("steric"), ptr("thermosteric"),
+                                            ptr("halosteric"), ws.data_ptr(), nbytes, _stream())
+        )
+    # each total as steric_local_profile forms it, torch.nansum of the row's weights in a buffer of their own, so that
+    # the quotients match bit for bit: torch's reduction order follows the alignment of its input, so every row is
+    # first given a start aligned as a fresh allocation is (one copy), then summed alone
+    pitch = -(-nx // 64) * 64  # 512 bytes
+    wp = w.new_zeros((ny, pitch))
+    wp[:, :nx] = w
+    totals = torch.stack([torch.nansum(wp[j, :nx]) for j in range(ny)])
+    return {v: prof[v] / totals for v in names}, totals
 
 
 def delta_rho(T, S, rho_ref, v_ref, p_level, eos="Wright", t_bcast=False, s_bcast=False):

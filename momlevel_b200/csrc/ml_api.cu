@@ -491,16 +491,20 @@ __global__ void __launch_bounds__(kBlock)
 // kProfSeg-column segment) pair and walks every time step.  Point -> thread mapping (two quads per thread, kBlock
 // apart), the order of a thread's sum and the per-warp partial slots are those of k_stream_profile, so the two
 // families give the same bits; so does REG, the region mode of k_stream_profile (one partial per region,
-// [nregions][nt * nz][slot], the regions a warp touches walked in ascending order).
+// [nregions][nt * nz][slot], the regions a warp touches walked in ascending order) and ZON, its zonal mode: nz is
+// then the nz * ny grid rows of ncol = nx columns (row = level * ny + j), each row with its own partials; the level and
+// the column j * nx + col of the (y, x) plane are read as k_stream_profile reads them.
 constexpr int kProfSeg = 2048;
-template <typename TIn, int EOS, int VM, bool REG>
-__global__ void __launch_bounds__(kBlock)
+// ZON asks for one CTA per SM at least: left unsaid, ptxas clamps some zonal instantiations to the 128 registers of two
+// CTAs and spills; 0 (unsaid) keeps the other instantiations as they were.
+template <typename TIn, int EOS, int VM, bool ZON, bool REG>
+__global__ void __launch_bounds__(kBlock, ZON ? 1 : 0)
     k_profile_direct(const TIn* __restrict__ T, const TIn* __restrict__ S, const TIn* __restrict__ T_ref,
                      const TIn* __restrict__ S_ref, const double* __restrict__ rho_ref, const void* __restrict__ v_ref,
                      int v_f32, const double* __restrict__ z_i, const double* __restrict__ deptho,
                      const double* __restrict__ weights, const double* __restrict__ p_level,
                      const double* __restrict__ p_col, double coef, int nt, int nz, i64 ncol, double* part0,
-                     double* part1, double* part2, const int8_t* __restrict__ region, int nregions) {
+                     double* part1, double* part2, const int8_t* __restrict__ region, int nregions, int ny) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const i64 col0 = (i64)blockIdx.x * kProfSeg;
   const i64 nblk = (i64)gridDim.x * kWarps;
@@ -508,8 +512,14 @@ __global__ void __launch_bounds__(kBlock)
   double* const part[3] = {part0, part1, part2};
   Eos<EOS> eos;
   for (int z = blockIdx.y; z < nz; z += gridDim.y) {
-    const double plev = __ldg(p_level + z);
-    const double ztop = __ldg(z_i + z), zbot = __ldg(z_i + z + 1);
+    int lev = z;
+    i64 cplane = 0;  // ZON: the level of row z, and the first column of its grid row in the (y, x) plane
+    if constexpr (ZON) {
+      lev = z / ny;
+      cplane = (i64)(z - lev * ny) * ncol;
+    }
+    const double plev = __ldg(p_level + lev);
+    const double ztop = __ldg(z_i + lev), zbot = __ldg(z_i + lev + 1);
     double ref[8], cw[8], pz[8];
     TIn tref[8], sref[8];
 #pragma unroll
@@ -520,12 +530,12 @@ __global__ void __launch_bounds__(kBlock)
       pz[k] = plev;
       tref[k] = sref[k] = TIn(0);
       if (c < ncol) {
-        const i64 i = (i64)z * ncol + c;
-        double depth = __ldg(deptho + c);
+        const i64 i = (i64)z * ncol + c, cp = cplane + c;
+        double depth = __ldg(deptho + cp);
         if (isnan(depth)) depth = 0.0;  // derived.py:295
         ref[k] = vref_wet(v_ref, v_f32, i) ? __ldg(rho_ref + i) : nan("");
-        cw[k] = profile_weight(vref_wet(v_ref, v_f32, c), __ldg(weights + c), clipped_dz(depth, ztop, zbot), coef);
-        if (p_col != nullptr) pz[k] = plev + __ldg(p_col + c);  // a 2-D patm (steric.py:96)
+        cw[k] = profile_weight(vref_wet(v_ref, v_f32, cp), __ldg(weights + cp), clipped_dz(depth, ztop, zbot), coef);
+        if (p_col != nullptr) pz[k] = plev + __ldg(p_col + cp);  // a 2-D patm (steric.py:96)
         if (VM & 4) tref[k] = __ldg(T_ref + i);
         if (VM & 2) sref[k] = __ldg(S_ref + i);
       }
@@ -693,19 +703,23 @@ template <typename TIn, int EOS>
 int launch_profile_direct(int vm, const void* T, const void* S, const void* T_ref, const void* S_ref,
                           const double* rho_ref, const void* v_ref, int v_f32, const double* z_i, const double* deptho,
                           const double* weights, const double* p_level, double coef, int nt, int nz, i64 ncol,
-                          double* const part[3], const int8_t* region, int nregions, cudaStream_t st) {
-  const dim3 grid((unsigned)cdiv(ncol, kProfSeg), (unsigned)(nz < 65535 ? nz : 65535));
-#define ML_PROF_DIRECT_REG(VM, REG)                                                                                      \
-  k_profile_direct<TIn, EOS, VM, REG><<<grid, kBlock, 0, st>>>((const TIn*)T, (const TIn*)S, (const TIn*)T_ref,         \
-                                                               (const TIn*)S_ref, rho_ref, v_ref, v_f32, z_i, deptho,    \
-                                                               weights, p_level, tls().p_col, coef, nt, nz, ncol,        \
-                                                               part[0], part[1], part[2], region, nregions)
+                          double* const part[3], const int8_t* region, int nregions, int ny, cudaStream_t st) {
+  const int rows = ny ? nz * ny : nz;  // ZON: nz * ny grid rows of ncol = nx columns
+  const dim3 grid((unsigned)cdiv(ncol, kProfSeg), (unsigned)(rows < 65535 ? rows : 65535));
+#define ML_PROF_DIRECT_REG(VM, ZON, REG)                                                                                 \
+  k_profile_direct<TIn, EOS, VM, ZON, REG><<<grid, kBlock, 0, st>>>((const TIn*)T, (const TIn*)S, (const TIn*)T_ref,    \
+                                                                    (const TIn*)S_ref, rho_ref, v_ref, v_f32, z_i,      \
+                                                                    deptho, weights, p_level, tls().p_col, coef, nt,    \
+                                                                    rows, ncol, part[0], part[1], part[2], region,      \
+                                                                    nregions, ny)
 #define ML_PROF_DIRECT(VM)                  \
   case VM:                                  \
     if (region != nullptr)                  \
-      ML_PROF_DIRECT_REG(VM, true);         \
+      ML_PROF_DIRECT_REG(VM, false, true);  \
+    else if (ny != 0)                       \
+      ML_PROF_DIRECT_REG(VM, true, false);  \
     else                                    \
-      ML_PROF_DIRECT_REG(VM, false);        \
+      ML_PROF_DIRECT_REG(VM, false, false); \
     break
   switch (vm) {
     ML_PROF_DIRECT(1);
@@ -1142,13 +1156,20 @@ size_t ml_profile_workspace_bytes(int nvariants, int64_t nt, int64_t nz, int64_t
   return ml_region_profile_workspace_bytes(nvariants, 1, nt, nz, ncol);
 }
 
-// ml_steric_local_profile (region == NULL: one region of every column, the workspace holds all nt steps) and
-// ml_steric_local_region_profile (the workspace holds at least one step).  The time axis runs in chunks of as many
-// steps as the workspace holds, with the field pointers moved for each; a step's partials and sums depend on its
-// points only, so its bits do not depend on the chunks.
+size_t ml_zonal_profile_workspace_bytes(int nvariants, int64_t nt, int64_t nz, int64_t ny, int64_t nx) {
+  if (nz < 1) nz = 1;
+  if (ny < 1) ny = 1;
+  return ml_region_profile_workspace_bytes(nvariants, 1, nt, nz * ny, nx);  // a (level, grid row) is a row of nx
+}
+
+// ml_steric_local_profile (region == NULL, ny == 0: one region of every column, the workspace holds all nt steps),
+// ml_steric_local_region_profile (the workspace holds at least one step) and ml_steric_local_zonal_profile (ny > 0:
+// a level is ny grid rows of ncol = nx columns, each row its own output; the workspace holds at least one step).  The
+// time axis runs in chunks of as many steps as the workspace holds, with the field pointers moved for each; a step's
+// partials and sums depend on its points only, so its bits do not depend on the chunks.
 static int profile_impl(int eos, int dtype, const void* T, const void* S, const void* T_ref, const void* S_ref,
                         const double* rho_ref, const void* v_ref, int vref_dtype, const double* z_i,
-                        const double* deptho, const double* weights, const int8_t* region, int nregions,
+                        const double* deptho, const double* weights, const int8_t* region, int nregions, int64_t ny,
                         const double* p_level, double neg_inv_rhozero, int64_t nt, int64_t nz, int64_t ncol,
                         double* const outs[3], void* workspace, size_t ws_bytes, void* stream) {
   int rc = check_common(eos, dtype);
@@ -1166,10 +1187,14 @@ static int profile_impl(int eos, int dtype, const void* T, const void* S, const 
   ML_REQUIRE_PTR(p_level);
   const int wanted = (outs[0] != nullptr) + (outs[1] != nullptr) + (outs[2] != nullptr);
   if (wanted == 0) return fail(ML_ERR_NULL, "prof_steric, prof_thermosteric and prof_halosteric are all NULL");
-  if (nt < 0 || nz <= 0 || ncol <= 0 || nt > INT32_MAX || nz > INT32_MAX || nt * nz > INT32_MAX)
-    return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ncol=%lld", (long long)nt, (long long)nz, (long long)ncol);
-  if (int rcp = check_column_pressure(ncol)) return rcp;
-  const size_t need = ml_region_profile_workspace_bytes(wanted, nregions, region ? 1 : nt, nz, ncol);
+  const int64_t nrow = ny ? ny : 1;  // grid rows per level, each with its own outputs
+  if (nt < 0 || nz <= 0 || ncol <= 0 || nrow <= 0 || nt > INT32_MAX || nz > INT32_MAX || nrow > INT32_MAX ||
+      nz * nrow > INT32_MAX || nt * nz * nrow > INT32_MAX)
+    return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ny=%lld ncol=%lld", (long long)nt, (long long)nz,
+                (long long)ny, (long long)ncol);
+  if (int rcp = check_column_pressure(nrow * ncol)) return rcp;
+  const i64 rows = nz * nrow;  // output rows of a step: (level, grid row)
+  const size_t need = ml_region_profile_workspace_bytes(wanted, nregions, (region || ny) ? 1 : nt, rows, ncol);
   if (workspace == nullptr || ws_bytes < need) return fail(ML_ERR_WORKSPACE, "workspace needs %zu bytes, got %zu", need, ws_bytes);
   ML_REQUIRE_ALIGNED(workspace, 8);
   ML_REQUIRE_ALIGNED(T, elem_size(dtype));
@@ -1182,10 +1207,10 @@ static int profile_impl(int eos, int dtype, const void* T, const void* S, const 
   const int v_f32 = vref_dtype == ML_F32;
   const i64 nblk = stream::profile_slots(ncol);
   // steps per chunk: as many as the workspace holds, and at most INT32_MAX rows for k_reduce_rows
-  const size_t step_bytes = ml_region_profile_workspace_bytes(wanted, nregions, 1, nz, ncol) - 256;
+  const size_t step_bytes = ml_region_profile_workspace_bytes(wanted, nregions, 1, rows, ncol) - 256;
   i64 tc = (i64)((ws_bytes - 256) / step_bytes);
   if (tc > nt) tc = nt;
-  if (tc > INT32_MAX / ((i64)nregions * nz)) tc = INT32_MAX / ((i64)nregions * nz);
+  if (tc > INT32_MAX / ((i64)nregions * rows)) tc = INT32_MAX / ((i64)nregions * rows);
   int vm = 0;
   for (int v = 0; v < 3; ++v)
     if (outs[v]) vm |= 1 << v;
@@ -1195,13 +1220,13 @@ static int profile_impl(int eos, int dtype, const void* T, const void* S, const 
   tls().last_path = ring ? ML_PATH_TMA : ML_PATH_DIRECT;
   for (i64 t0 = 0; t0 < nt; t0 += tc) {
     const i64 n = nt - t0 < tc ? nt - t0 : tc;
-    const size_t off = (size_t)(t0 * nz * ncol) * elem_size(dtype);
+    const size_t off = (size_t)(t0 * rows * ncol) * elem_size(dtype);
     const void* Tc = static_cast<const char*>(T) + off;
     const void* Sc = static_cast<const char*>(S) + off;
-    // per wanted variant, in the order steric, thermosteric, halosteric: [nregions][n * nz][nblk] per-warp partials
+    // per wanted variant, in the order steric, thermosteric, halosteric: [nregions][n * rows][nblk] per-warp partials
     double* part[3] = {nullptr, nullptr, nullptr};
     for (int v = 0, r = 0; v < 3; ++v)
-      if (outs[v]) part[v] = static_cast<double*>(workspace) + (i64)r++ * nregions * n * nz * nblk;
+      if (outs[v]) part[v] = static_cast<double*>(workspace) + (i64)r++ * nregions * n * rows * nblk;
     for (int v = 0; v < 3; ++v) {
       const int m = split ? (vm & (1 << v)) : (v == 0 ? vm : 0);
       if (m == 0) continue;
@@ -1209,28 +1234,28 @@ static int profile_impl(int eos, int dtype, const void* T, const void* S, const 
       if (ring)
         rc = stream::launch_profile(eos, m, (const float*)Tc, (const float*)Sc, (const float*)T_ref, (const float*)S_ref,
                                     rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, nz,
-                                    ncol, p, region, nregions, st);
+                                    ncol, p, region, nregions, (int)ny, st);
       else if (dtype == ML_F32)
         rc = eos == ML_EOS_WRIGHT
-                 ? launch_profile_direct<float, 0>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, st)
-                 : launch_profile_direct<float, 1>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, st);
+                 ? launch_profile_direct<float, 0>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, (int)ny, st)
+                 : launch_profile_direct<float, 1>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, (int)ny, st);
       else
         rc = eos == ML_EOS_WRIGHT
-                 ? launch_profile_direct<double, 0>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, st)
-                 : launch_profile_direct<double, 1>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, st);
+                 ? launch_profile_direct<double, 0>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, (int)ny, st)
+                 : launch_profile_direct<double, 1>(m, Tc, Sc, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, neg_inv_rhozero, (int)n, (int)nz, ncol, p, region, nregions, (int)ny, st);
       if (rc) return rc;
     }
-    // fixed-order second stage: one block per (region, step, level) row; outputs are [nregions][nt][nz]
+    // fixed-order second stage: one block per (region, step, level[, grid row]) row; outputs are [nregions][nt][rows]
     for (int v = 0; v < 3; ++v) {
       if (outs[v] == nullptr) continue;
       if (n == nt) {
-        k_reduce_rows<<<(unsigned)(nregions * nt * nz), kBlock, 0, st>>>(part[v], nblk, outs[v]);
+        k_reduce_rows<<<(unsigned)(nregions * nt * rows), kBlock, 0, st>>>(part[v], nblk, outs[v]);
         if ((rc = launched("k_reduce_rows"))) return rc;
         continue;
       }
       for (int r = 0; r < nregions; ++r) {
-        k_reduce_rows<<<(unsigned)(n * nz), kBlock, 0, st>>>(part[v] + (i64)r * n * nz * nblk, nblk,
-                                                             outs[v] + ((i64)r * nt + t0) * nz);
+        k_reduce_rows<<<(unsigned)(n * rows), kBlock, 0, st>>>(part[v] + (i64)r * n * rows * nblk, nblk,
+                                                               outs[v] + ((i64)r * nt + t0) * rows);
         if ((rc = launched("k_reduce_rows"))) return rc;
       }
     }
@@ -1245,7 +1270,7 @@ int ml_steric_local_profile(int eos, int dtype, const void* T, const void* S, co
                             double* prof_thermosteric, double* prof_halosteric, void* workspace, size_t ws_bytes,
                             void* stream) {
   double* const outs[3] = {prof_steric, prof_thermosteric, prof_halosteric};
-  return profile_impl(eos, dtype, T, S, T_ref, S_ref, rho_ref, v_ref, vref_dtype, z_i, deptho, weights, nullptr, 1,
+  return profile_impl(eos, dtype, T, S, T_ref, S_ref, rho_ref, v_ref, vref_dtype, z_i, deptho, weights, nullptr, 1, 0,
                       p_level, neg_inv_rhozero, nt, nz, ncol, outs, workspace, ws_bytes, stream);
 }
 
@@ -1261,7 +1286,20 @@ int ml_steric_local_region_profile(int eos, int dtype, const void* T, const void
   ML_REQUIRE_PTR(region);
   double* const outs[3] = {prof_steric, prof_thermosteric, prof_halosteric};
   return profile_impl(eos, dtype, T, S, T_ref, S_ref, rho_ref, v_ref, vref_dtype, z_i, deptho, weights, region,
-                      nregions, p_level, neg_inv_rhozero, nt, nz, ncol, outs, workspace, ws_bytes, stream);
+                      nregions, 0, p_level, neg_inv_rhozero, nt, nz, ncol, outs, workspace, ws_bytes, stream);
+}
+
+int ml_steric_local_zonal_profile(int eos, int dtype, const void* T, const void* S, const void* T_ref,
+                                  const void* S_ref, const double* rho_ref, const void* v_ref, int vref_dtype,
+                                  const double* z_i, const double* deptho, const double* weights,
+                                  const double* p_level, double neg_inv_rhozero, int64_t nt, int64_t nz, int64_t ny,
+                                  int64_t nx, double* prof_steric, double* prof_thermosteric,
+                                  double* prof_halosteric, void* workspace, size_t ws_bytes, void* stream) {
+  if (ny <= 0) return fail(ML_ERR_SHAPE, "bad extents nt=%lld nz=%lld ny=%lld nx=%lld", (long long)nt, (long long)nz,
+                           (long long)ny, (long long)nx);
+  double* const outs[3] = {prof_steric, prof_thermosteric, prof_halosteric};
+  return profile_impl(eos, dtype, T, S, T_ref, S_ref, rho_ref, v_ref, vref_dtype, z_i, deptho, weights, nullptr, 1, ny,
+                      p_level, neg_inv_rhozero, nt, nz, nx, outs, workspace, ws_bytes, stream);
 }
 
 static int delta_rho_impl(int eos, int dtype, const void* T, const void* S, int t_bcast, int s_bcast,

@@ -340,14 +340,22 @@ __global__ void __launch_bounds__(kThreads, 2)
 // iteration r each thread sums, in the order above, only its points of region r: every density is evaluated once,
 // and a warp whose points all lie in one region sums exactly as without regions.  Lane 0 stores region r's
 // partial; lane r stores 0 for a region the warp does not touch, so every slot is written on every step.
+// ZON (ml_steric_local_zonal_profile): one partial row per grid row.  A work item is a (level z, row j, kTile-column
+// sub-tile s) triple: the geometry above on a grid of nz * ny rows of nx columns (g.ncol = nx, g.nz = nz * ny,
+// row = z * ny + j), so the field offsets, the thread -> point map, the per-item state, the order of the sums and the
+// slot formula are those of a call on row j alone: partials[v][((t * nz + z) * ny + j) * nsub * kWarps + s * kWarps +
+// warp].  Only the level (pressure, interfaces) and the column of the (y, x) plane (deptho, weights, surface mask) are
+// read through z and j * nx + col.  So row j's partials are bit-identical to ml_steric_local_profile on row j sliced
+// out alone, and every slot is written on every step, a warp without points storing its 0.
 constexpr size_t kProfileRing = ring_bytes<2>();  // the per-point state follows the ring
 struct ProfileOut {
   double* part[3];  // per variant, [nregions][nt * nz][tiles_per_row * kWarps]; NULL for a variant not asked for
   const int8_t* region;  // REG: [ncol] region index of each column, one in [0, nregions) or none
   int nregions;
+  int ny;  // ZON: grid rows per level
 };
 
-template <int EOS, int VM, bool REG>
+template <int EOS, int VM, bool ZON, bool REG>
 __global__ void __launch_bounds__(kThreads, 2)
     k_stream_profile(const float* __restrict__ T, const float* __restrict__ S, const float* __restrict__ T_ref,
                      const float* __restrict__ S_ref, const double* __restrict__ rho_ref, const void* __restrict__ v_ref,
@@ -394,8 +402,13 @@ __global__ void __launch_bounds__(kThreads, 2)
     const i64 col0 = seg * kTile;
     const i64 len = g.ncol - col0 < kTile ? g.ncol - col0 : kTile;
     const i64 off = row * g.ncol + col0;
-    eos.set_level(__ldg(p_level + row));
-    const double ztop = __ldg(z_i + row), zbot = __ldg(z_i + row + 1);
+    i64 lev = row, cplane = col0;  // the level, and the first column of the item in the (y, x) plane
+    if constexpr (ZON) {
+      lev = row / out.ny;
+      cplane = (row - lev * out.ny) * g.ncol + col0;
+    }
+    eos.set_level(__ldg(p_level + lev));
+    const double ztop = __ldg(z_i + lev), zbot = __ldg(z_i + lev + 1);
     uint32_t rbits = 0, wmask = 0;  // REG: the 4-bit region index of each point; the regions the warp touches
     if constexpr (REG) {
 #pragma unroll
@@ -419,7 +432,7 @@ __global__ void __launch_bounds__(kThreads, 2)
       if (4 * qd < len) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-          const i64 c = col0 + 4 * qd + j;
+          const i64 c = cplane + 4 * qd + j;
           const bool wet = v_f32 ? !isnan(__ldg(reinterpret_cast<const float*>(v_ref) + off + 4 * qd + j))
                                  : !isnan(__ldg(reinterpret_cast<const double*>(v_ref) + off + 4 * qd + j));
           const bool top = v_f32 ? !isnan(__ldg(reinterpret_cast<const float*>(v_ref) + c))
@@ -592,12 +605,12 @@ constexpr size_t profile_smem_bytes() { return kProfileRing + 2 * kTile * (sizeo
 
 int profile_slots(i64 ncol) { return (int)((ncol + kTile - 1) / kTile) * kWarps; }
 
-template <int EOS, int VM, bool REG>
+template <int EOS, int VM, bool ZON, bool REG>
 static int launch_profile_vm(const float* T, const float* S, const float* T_ref, const float* S_ref,
                              const double* rho_ref, const void* v_ref, int v_f32, const double* z_i,
                              const double* deptho, const double* weights, const double* p_level, double coef, int nt,
                              const Geom& g, const ProfileOut& out, cudaStream_t st) {
-  auto kern = k_stream_profile<EOS, VM, REG>;
+  auto kern = k_stream_profile<EOS, VM, ZON, REG>;
   if (int rc = opt_in(kern, profile_smem_bytes())) return rc;
   kern<<<persistent_grid(g.ntiles, 2), kThreads, profile_smem_bytes(), st>>>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i,
                                                                          deptho, weights, p_level, coef, nt, g, out);
@@ -611,10 +624,12 @@ static int launch_profile_eos(int vm, const float* T, const float* S, const floa
                               const Geom& g, const ProfileOut& out, cudaStream_t st) {
 #define ML_STREAM_PROF(VM)                                                                                               \
   case VM:                                                                                                               \
-    return out.region ? launch_profile_vm<EOS, VM, true>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho,        \
-                                                         weights, p_level, coef, nt, g, out, st)                        \
-                      : launch_profile_vm<EOS, VM, false>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho,       \
-                                                          weights, p_level, coef, nt, g, out, st)
+    return out.region ? launch_profile_vm<EOS, VM, false, true>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i,         \
+                                                                deptho, weights, p_level, coef, nt, g, out, st)         \
+           : out.ny   ? launch_profile_vm<EOS, VM, true, false>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i,         \
+                                                                deptho, weights, p_level, coef, nt, g, out, st)         \
+                      : launch_profile_vm<EOS, VM, false, false>(T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i,        \
+                                                                 deptho, weights, p_level, coef, nt, g, out, st)
   switch (vm) {
     ML_STREAM_PROF(1);
     ML_STREAM_PROF(2);
@@ -631,9 +646,10 @@ static int launch_profile_eos(int vm, const float* T, const float* S, const floa
 int launch_profile(int eos, int vm, const float* T, const float* S, const float* T_ref, const float* S_ref,
                    const double* rho_ref, const void* v_ref, int v_f32, const double* z_i, const double* deptho,
                    const double* weights, const double* p_level, double coef, int nt, i64 nz, i64 ncol,
-                   double* const part[3], const int8_t* region, int nregions, cudaStream_t st) {
-  const Geom g = geometry(nz, (int)nz, ncol);
-  const ProfileOut out = {{part[0], part[1], part[2]}, region, nregions};
+                   double* const part[3], const int8_t* region, int nregions, int ny, cudaStream_t st) {
+  const i64 rows = ny ? nz * ny : nz;  // ZON: nz * ny rows of ncol = nx columns
+  const Geom g = geometry(rows, (int)rows, ncol);
+  const ProfileOut out = {{part[0], part[1], part[2]}, region, nregions, ny};
   if (eos == ML_EOS_WRIGHT)
     return launch_profile_eos<0>(vm, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, coef, nt, g, out, st);
   return launch_profile_eos<1>(vm, T, S, T_ref, S_ref, rho_ref, v_ref, v_f32, z_i, deptho, weights, p_level, coef, nt, g, out, st);

@@ -30,12 +30,14 @@ int launch_delta_rho(int eos, const float* T, const float* S, long long t_stride
 // level profile (ml_steric_local_profile): per-warp partials of coef * m * w * dz * (rho_v - rho_ref) into part[v]
 // ([nt * nz][profile_slots(ncol)], NULL for a variant not asked for), vm = the variants as bits (1 steric,
 // 2 thermosteric, 4 halosteric); the fixed-order second stage is k_reduce_rows.  With a region index ([ncol],
-// ml_steric_local_region_profile; NULL: none) part[v] is [nregions][nt * nz][profile_slots(ncol)].
+// ml_steric_local_region_profile; NULL: none) part[v] is [nregions][nt * nz][profile_slots(ncol)].  ny > 0
+// (ml_steric_local_zonal_profile): a level is ny grid rows of ncol = nx columns, T and S are [nt][nz][ny][nx] and
+// part[v] is [nt * nz * ny][profile_slots(nx)], one partial row per grid row; ny = 0: a level is one row of ncol.
 int profile_slots(long long ncol);
 int launch_profile(int eos, int vm, const float* T, const float* S, const float* T_ref, const float* S_ref,
                    const double* rho_ref, const void* v_ref, int v_f32, const double* z_i, const double* deptho,
                    const double* weights, const double* p_level, double coef, int nt, long long nz, long long ncol,
-                   double* const part[3], const int8_t* region, int nregions, cudaStream_t st);
+                   double* const part[3], const int8_t* region, int nregions, int ny, cudaStream_t st);
 
 }  // namespace stream
 }  // namespace ml

@@ -928,7 +928,7 @@ def _region_map(regions, region_codes):
 
 def steric_profile(dset, variant="steric", reference=None, weights=None, coord_names=None, varname_map=None,
                    rhozero=1035.0, patm=101325.0, equation_of_state="Wright", dtype="float32", strict=True, annual=False,
-                   days_in_month=None, verbose=False, regions=None, region_codes=None):
+                   days_in_month=None, verbose=False, regions=None, region_codes=None, zonal=False):
     """How much each model level contributes to the area-weighted mean steric, thermosteric or halosteric sea level
     change, per time step, from one pass over T and S (a depth-time Hovmoeller of the expansion; summed over the
     levels below a depth, that depth's deep contribution).
@@ -956,8 +956,20 @@ def steric_profile(dset, variant="steric", reference=None, weights=None, coord_n
     Returns ``(result, reference)``: ``result[name]`` has dims ``(time, z_l)``.  With ``regions`` it has dims ``(time,
     region, z_l)``, the ``region`` coordinate holds the codes and ``result["region_weight"]`` is ``(region,)``, each
     region's ``nansum(w)``, so that regions combine exactly: ``(p[a] * W[a] + p[b] * W[b]) / (W[a] + W[b])``.
+
+    ``zonal=True`` gives the section of every grid row from the same one pass, a latitude-depth section of the
+    change: ``section[t, z, j] = -1/rhozero * nansum_i(m * w * dz * delta_rho[t, z, j, i]) / nansum_i(w[j, i])``.
+    Row ``j`` is, bit for bit, this call on the dataset sliced to row ``j``.  Row ``j`` is a row of the model grid: on
+    a tripolar grid it is a circle of latitude only south of the fold, and a row of the Arctic patch north of it mixes
+    latitudes.  A row whose weights sum to 0 (all land, or outside the basin of ``weights=areacello * basin_mask``)
+    gives NaN.  The fields must be laid out ``(time, z, y, x)``, and ``zonal`` does not combine with ``regions``.
+    ``result[name]`` then has dims ``(time, z_l, y)`` (``y`` the field's third dim, its coordinate attached when
+    the dataset has one) and ``result["zonal_weight"]`` is ``(y,)``, each row's ``nansum(w)``, so that rows combine
+    exactly as regions do: ``sum_j section[..., j] * W[j] / sum_j W[j]`` is the profile of the whole grid.
     """
     names = core.variant_names(variant)
+    if zonal and regions is not None:
+        raise ValueError("zonal=True gives one section per grid row; it does not combine with regions")
     codes, region_index = _region_map(regions, region_codes)
     xarray_in = type(dset).__module__.startswith("xarray")
     if xarray_in:
@@ -1012,7 +1024,18 @@ def steric_profile(dset, variant="steric", reference=None, weights=None, coord_n
     operands = (full.data, dset["so"].data, reference["thetao"].data, reference["so"].data, reference["rho"].data,
                 reference["volcello"].data, dset[zbounds].data, dset["deptho"].data, pres, w)
     result = Dataset()
-    if region_index is None:
+    if zonal:
+        ydim = full.dims[2]
+        profs, totals = core.steric_local_zonal_profile(*operands, rhozero=rhozero, eos=equation_of_state,
+                                                        variants=names)
+        for name in names:
+            result[name] = DataArray(profs[name], (tcoord, zcoord, ydim), attrs={
+                "long_name": f"{name.capitalize()} height adjustment by level and grid row, area-weighted mean",
+                "units": "m"})
+            result[name].encoding["dtype"] = dtype
+        result["zonal_weight"] = DataArray(totals, (ydim,), attrs={
+            "long_name": "Sum of the column weights of the grid row (nansum(w))"})
+    elif region_index is None:
         profs = core.steric_local_profile(*operands, rhozero=rhozero, eos=equation_of_state, variants=names)
         for name in names:
             result[name] = DataArray(profs[name], (tcoord, zcoord), attrs={
