@@ -410,6 +410,30 @@ int ml_steric_global_variants(int eos, int dtype, const void* T, const void* S, 
 int ml_calc_masso(int dtype, const void* rho, int w_dtype, const void* volcello, int64_t nrows, int64_t n,
                   double* out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* bytes of the running sums of ml_mean_state_accumulate: 6 fp64 per cell (0 for a non-positive extent) */
+size_t ml_mean_state_bytes(int64_t nz, int64_t ncol);
+
+/* ---------------------------------------------------------------------------------------
+ * ml_mean_state_accumulate -- time mean of T, S and volcello over a baseline period, the fields of a
+ * climatological reference state (setup_reference_state(period=...)); ml_reference_state then runs on the means.
+ * For each cell and field on its own: mean = sum_t w_t x_t / sum_t w_t over the steps where x is not NaN (xarray's
+ * skipna weighted(...).mean); a cell with no value in the period is NaN.  Each step adds acc = acc + w*x and
+ * wsum = wsum + w, rounded separately, in ascending t; the mean is one IEEE division.  The bits do not depend on how
+ * the period is cut into calls or launches, nor on the kernel.
+ *   T, S        device [nt][nz][ncol] of `dtype`;  V device [nt][nz][ncol] of `vdtype` (volcello)
+ *   w           device fp64[nt], the weights of these steps, or NULL for ones
+ *   acc         device, ml_mean_state_bytes(nz, ncol) bytes: the running sums between calls.  Required
+ *               (ML_ERR_WORKSPACE) unless the call is flags = 3 with nt <= 1024; a longer call runs in launches of 1024
+ *               steps that carry the sums through it
+ *   flags       1 first: start the sums from zero (acc is not read); 2 last: write the means instead of the sums
+ *   T_mean, S_mean, V_mean  device [nz][ncol] fp64 out, required with flags & 2 (ML_ERR_NULL)
+ * Plain loads take ragged rows (ncol % 4 != 0), bases that are not 16-byte aligned and ml_set_force_direct(1);
+ * same bits.  Every argument error returns before any launch.
+ * ------------------------------------------------------------------------------------- */
+int ml_mean_state_accumulate(int dtype, const void* T, const void* S, const void* V, int vdtype, const double* w,
+                             int64_t nt, int64_t nz, int64_t ncol, void* acc, size_t acc_bytes, int flags,
+                             double* T_mean, double* S_mean, double* V_mean, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * ml_steric_local_host -- the same computation as reference_state + steric_local for
  * variant="steric" on HOST buffers: time steps are staged to the device through two

@@ -13,7 +13,8 @@ import sys
 PKG = pathlib.Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libmomlevel_b200.so"
-SOURCES = ["ml_api.cu", "ml_tma.cu", "ml_tma_flat.cu", "ml_tma3.cu", "ml_stream.cu", "ml_hostpath.cu", "ml_strat.cu", "ml_pack.cpp"]
+SOURCES = ["ml_api.cu", "ml_tma.cu", "ml_tma_flat.cu", "ml_tma3.cu", "ml_stream.cu", "ml_hostpath.cu", "ml_strat.cu", "ml_mean.cu",
+           "ml_pack.cpp"]
 NVCC_FLAGS = [
     "-gencode",
     "arch=compute_100a,code=sm_100a",

@@ -60,6 +60,8 @@ EXPORTS = {
     "ml_steric_local_variants": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _d, _i64, _i64, _i64, _vp, _vp,
                                       _vp, _vp, _vp, _vp, _sz, _vp]),
     "ml_calc_masso": (_i, [_i, _vp, _i, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),
+    "ml_mean_state_bytes": (_sz, [_i64, _i64]),
+    "ml_mean_state_accumulate": (_i, [_i, _vp, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _sz, _i, _vp, _vp, _vp, _vp]),
     "ml_steric_global": (_i, [_i, _i, _vp, _vp, _i, _i, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp, _sz, _vp]),
     "ml_steric_global_variants": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp,
                                        _sz, _vp]),

@@ -367,6 +367,128 @@ def weighted_nansum(a, w=None, nrows=1):
     return out
 
 
+MEAN_FIRST, MEAN_LAST = 1, 2
+
+
+def mean_state_bytes(nz, ncol):
+    """Bytes of the running sums of :func:`mean_state_accumulate` (``ml_mean_state_bytes``): 6 fp64 per cell."""
+    return int(_lib.lib().ml_mean_state_bytes(int(nz), int(ncol)))
+
+
+def mean_state_accumulate(T, S, V, weights=None, acc=None, first=True, last=True, out=None):
+    """One call of ``ml_mean_state_accumulate`` on device fields ``[nt, nz, ...]``: add their steps to the running
+    sums ``acc`` (``first``: start from zero) and, with ``last``, return the skipna weighted means
+    ``(T_mean, S_mean, V_mean)`` as fp64 ``[nz, ...]`` (``out`` may hand in the three tensors).  ``T`` and ``S``
+    share a storage dtype (fp32 only if both are); ``V`` keeps its own.  ``weights``: device fp64 ``[nt]`` or
+    ``None`` for ones."""
+    L = _lib.lib()
+    dt = _field_dtype(T, S)
+    T, S, V = T.to(dt).contiguous(), S.to(dt).contiguous(), V.contiguous()
+    if V.dtype not in (torch.float32, torch.float64):
+        V = V.to(torch.float64)
+    assert T.shape == S.shape == V.shape and T.dim() >= 2, "thetao, so and volcello must be [nt, nz, ...] alike"
+    nt, nz = int(T.shape[0]), int(T.shape[1])
+    ncol = int(np.prod(T.shape[2:], dtype=np.int64))
+    w = None
+    if weights is not None:
+        w = weights
+        assert w.dtype == torch.float64 and w.is_cuda and w.numel() == nt and w.is_contiguous(), "weights: fp64 [nt] on the device"
+    if last and out is None:
+        out = tuple(torch.empty(tuple(T.shape[1:]), dtype=torch.float64, device=T.device) for _ in range(3))
+    flags = (MEAN_FIRST if first else 0) | (MEAN_LAST if last else 0)
+    ptr = lambda x: x.data_ptr() if x is not None else None  # noqa: E731
+    _lib.check(L.ml_mean_state_accumulate(
+        _dt_id(T), T.data_ptr(), S.data_ptr(), V.data_ptr(), _dt_id(V), ptr(w), nt, nz, ncol, ptr(acc),
+        acc.numel() * acc.element_size() if acc is not None else 0, flags,
+        *(ptr(o) for o in (out if last else (None, None, None))), _stream()))
+    return out if last else None
+
+
+def mean_state(T, S, V, weights=None):
+    """The skipna weighted time means of device-resident fields ``[nt, nz, ...]``: one first-and-last call (the
+    running sums never leave registers).  Returns ``(T_mean, S_mean, V_mean)``, fp64 ``[nz, ...]``."""
+    acc = None
+    if int(T.shape[0]) > _MEAN_STEPS_PER_LAUNCH:  # launched in pieces that carry the sums through the accumulator
+        acc = torch.empty(mean_state_bytes(T.shape[1], int(np.prod(T.shape[2:], dtype=np.int64))) // 8,
+                          dtype=torch.float64, device=T.device)
+    return mean_state_accumulate(T, S, V, weights, acc)
+
+
+_MEAN_STEPS_PER_LAUNCH = 1024  # ml_mean_state_accumulate: longer calls need the accumulator
+
+
+def mean_state_blocks(pieces, shape, dtype, v_dtype, weights=None, max_steps=1):
+    """The skipna weighted time means of fields held in host memory, from consecutive step ranges.
+
+    ``pieces`` yields ``(T, S, V)`` host blocks (numpy or CPU tensors) ``[n, *shape]`` in period order, each of at most
+    ``max_steps`` steps; ``weights`` is ``None`` or the period's fp64 weights (host).  Each block is copied to one of
+    two device buffers on a copy stream -- through pinned staging unless it is already pinned -- while the block before
+    it is accumulated, so at most two blocks are in flight.  ``dtype`` / ``v_dtype``: how T, S and V travel.
+    Returns ``(T_mean, S_mean, V_mean)``, fp64 ``[*shape]`` on the device."""
+    dev = _device()
+    shape = tuple(int(s) for s in shape)
+    nz, ncol = shape[0], int(np.prod(shape[1:], dtype=np.int64))
+    acc = torch.empty(mean_state_bytes(nz, ncol) // 8, dtype=torch.float64, device=dev)
+    w = None
+    if weights is not None:
+        w = torch.as_tensor(np.ascontiguousarray(weights, dtype=np.float64)).to(dev)
+    compute = torch.cuda.current_stream()
+    copy = torch.cuda.Stream(device=dev)
+    dts = (dtype, dtype, v_dtype)
+    slots = [None, None]  # per slot: (device buffers, pinned buffers, host blocks in flight, copied event, used event)
+    t, k, out = 0, 0, None
+    pending = None  # (slot, n): the block waiting to be accumulated
+    it = iter(pieces)
+    nxt = next(it, None)
+    while nxt is not None:
+        blocks = [_host_tensor(b) for b in nxt]
+        n = int(blocks[0].shape[0])
+        assert all(tuple(b.shape) == (n,) + shape for b in blocks) and 0 < n <= max_steps
+        s = k % 2
+        if slots[s] is None:
+            slots[s] = ([torch.empty((max_steps,) + shape, dtype=d, device=dev) for d in dts], [None] * 3, None,
+                        torch.cuda.Event(), None)
+        devb, pinned, _, copied, used = slots[s]
+        if used is not None:
+            used.synchronize()  # the accumulation that read this slot, and so the copy into it, are done
+        src = []
+        for j, b in enumerate(blocks):
+            b = b.to(dts[j]) if b.dtype != dts[j] else b
+            if not b.is_pinned():
+                if pinned[j] is None:
+                    pinned[j] = torch.empty((max_steps,) + shape, dtype=dts[j], pin_memory=True)
+                pinned[j][:n].copy_(b)
+                b = pinned[j][:n]
+            src.append(b)
+        with torch.cuda.stream(copy):
+            for j in range(3):
+                devb[j][:n].copy_(src[j], non_blocking=True)
+            copied.record(copy)
+        slots[s] = (devb, pinned, src, copied, used)  # the host blocks stay referenced until their copy is done
+        if pending is not None:
+            out = _accumulate_slot(slots, pending, w, acc, compute, last=False)
+        pending = (s, n, t)
+        t += n
+        k += 1
+        nxt = next(it, None)
+    assert pending is not None, "an empty period"
+    out = _accumulate_slot(slots, pending, w, acc, compute, last=True)
+    compute.synchronize()
+    return out
+
+
+def _accumulate_slot(slots, pending, w, acc, compute, last):
+    s, n, t = pending
+    devb, pinned, src, copied, _ = slots[s]
+    compute.wait_event(copied)
+    out = mean_state_accumulate(devb[0][:n], devb[1][:n], devb[2][:n], w[t: t + n] if w is not None else None, acc,
+                                first=t == 0, last=last)
+    used = torch.cuda.Event()
+    used.record(compute)
+    slots[s] = (devb, pinned, src, copied, used)
+    return out
+
+
 def _steric_operands(T, S, t_bcast, s_bcast):
     T, S = to_device(T), to_device(S)
     dt = _field_dtype(T, S)
@@ -551,6 +673,10 @@ def steric_local_profile(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho, p_leve
     nbytes = L.ml_profile_workspace_bytes(len(names), nt, nz, ncol)
     ws = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=T.device)
     ptr = lambda v: prof[v].data_ptr() if v in prof else None  # noqa: E731
+    # The weight total is queued ahead of the profile kernel (same stream, same value).  A torch.profiler session in a
+    # long-running process can lose its first GPU activity; queued first, the library kernel is never that activity,
+    # so a trace of this call always shows which profile kernel ran.
+    total = torch.nansum(w)
     with _pcol:
         _lib.check(
             L.ml_steric_local_profile(_eos_id(eos), _dt_id(T), T.data_ptr(), S.data_ptr(), Tr.data_ptr(), Sr.data_ptr(),
@@ -559,7 +685,6 @@ def steric_local_profile(T, S, T_ref, S_ref, rho_ref, v_ref, z_i, deptho, p_leve
                                       ptr("steric"), ptr("thermosteric"), ptr("halosteric"), ws.data_ptr(), nbytes,
                                       _stream())
         )
-    total = torch.nansum(w)
     return {v: prof[v] / total for v in names}
 
 
